@@ -6,9 +6,11 @@ native food spawn, in-place reset of finished games, every live snake's fp32 NHW
 A "step" is one lockstep tic of all games = one launch of the fused tic+encode kernel.  N>1: one process per GPU
 (torchrun), every rank steps its own 65,536 games (weak scaling, no collective on the data path).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 Prints ONE JSON line (rank 0).  See DESIGN.md "Measurement" for the definitions of every field.
+--dump-outputs DIR writes what the last timed step computed as DIR/<name>.npy (see dump_outputs), so that two builds run
+with the same arguments can be compared output for output.
 """
 import argparse
 import ctypes as C
@@ -400,6 +402,32 @@ def run_reference(args, rank, world):
         "e2e": {"value": v, "unit": UNIT, "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}}))
 
 
+DUMP_PLANES = 4096     # planes in the dump: a fixed sample of the step's rows (one per live snake, ~1 GB of planes in all)
+
+
+def dump_outputs(eng, out_dir):
+    """What one eng.step of the timed loop hands its caller, as .npy files: the row count, every row id (game * 8 + snake),
+    the per-game ended flags and rewards (integers, stored as float64: exact), and a fixed, seeded sample of the fp32 planes
+    with the ids of the sampled rows.  Rows are put in row-id order first: the kernel hands rows out in whatever order its
+    warps finish, so the raw order differs from run to run while the set of rows does not."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    n = int(eng.row_count.item())
+    ids = eng.row_ids[:n]
+    order = torch.argsort(ids)
+    pick = np.sort(np.random.default_rng(0).choice(n, size=min(n, DUMP_PLANES), replace=False))
+    sel = order[torch.from_numpy(pick).to(order.device)]
+    out = {"row_count": np.array([n], np.float64),
+           "row_ids": ids[order].cpu().numpy().astype(np.float64),
+           "ended": eng.ended.cpu().numpy().astype(np.float64),
+           "rewards": eng.rewards.cpu().numpy().astype(np.float64),
+           "planes_sample_row_ids": ids[sel].cpu().numpy().astype(np.float64),
+           "planes_sample": eng.planes[:n][sel].cpu().numpy()}
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def run_ours(args, rank, world, local_rank):
     import numpy as np
     import torch
@@ -441,6 +469,8 @@ def run_ours(args, rank, world, local_rank):
     clocks = sampler.stop() if rank == 0 else None
     ms = ev0.elapsed_time(ev1)
     t_after = eng.totals()
+    if args.dump_outputs and rank == 0:     # before the untimed pass below steps the games on
+        dump_outputs(eng, args.dump_outputs)
     # per-launch percentiles from a second, untimed pass with an event after every launch (the events themselves cost ~1 us per
     # launch, which is why they are not in the timed region): a launch-time distribution with two modes would show here
     step_ev = [torch.cuda.Event(enable_timing=True) for _ in range(K + 1)]
@@ -729,7 +759,12 @@ def main():
     ap.add_argument("--no-selfplay", action="store_true", help="skip the self-play (MCTS + value net) leg")
     ap.add_argument("--sp-games", type=int, default=4096, help="root games of the self-play leg (configs[2]: 4096)")
     ap.add_argument("--sp-turns", type=int, default=2, help="timed root turns of the self-play leg")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step (rank 0) to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
