@@ -90,7 +90,6 @@ SYMBOLS = [
     ("asz_net_create", C.c_int, [C.POINTER(_vp), C.POINTER(NetWeights), _i32]),
     ("asz_net_destroy", C.c_int, [_vp]),
     ("asz_net_update_weights", C.c_int, [_vp, C.POINTER(NetWeights), _vp]),
-    ("asz_net_set_variant", C.c_int, [_vp, _i32]),
     ("asz_net_forward", C.c_int, [_vp, _vp, _i32, _vp, _vp]),
     ("asz_net_forward_pitched", C.c_int, [_vp, _vp, _i32, _i32, _vp, _vp]),
     ("asz_net_debug_layer", C.c_int, [_vp, _vp, _i32, _i32, _vp, _vp]),

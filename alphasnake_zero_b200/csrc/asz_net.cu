@@ -9,10 +9,10 @@
 //   A operand    one halo tile (256 + 2*24 rows, all 16 channel chunks) per CTA and super-tile, fetched with cp.async.bulk
 //                and reused by all 9 taps through the shared-memory descriptor's start address (no-swizzle K-major core
 //                matrices: 8 rows x 16 B contiguous, SBO = 128 B => rows are linear, any row offset is legal);
-//   B operand    weights [tap][kc][cout][8] bf16 streamed in half-tap chunks through an mbarrier ring (9 stages of 16 KB;
-//                16 stages of 8 KB per CTA of a pair, which holds only half of the output channels);
-//   D            two 128 x 128 fp32 accumulators per super-tile in TMEM (double buffered: 512 columns), 144 tcgen05.mma
-//                (M128 N128 K16, or M256 N128 K16 with cta_group::2 over a CTA pair) issued by one elected thread;
+//   B operand    weights [tap][kc][cout][8] bf16 in half-tap chunks of 8 KB per CTA of a pair, which holds only half of the
+//                output channels: resident for a whole launch where they fit (RESW), else streamed through an mbarrier ring;
+//   D            two 128 x 128 fp32 accumulators per CTA and super-tile in TMEM (double buffered: 512 columns), 144
+//                tcgen05.mma (M256 N128 K16, cta_group::2 over a CTA pair) issued by one elected thread;
 //   epilogue     8 warps read TMEM (tcgen05.ld 32x32b), apply the folded BatchNorm scale/bias, the residual add and
 //                the ReLU (alpha_nnet.py:22-47), zero the padding positions and store bf16 in the same layout; the
 //                last convolution instead applies the 1x1 head convolution + BN + ReLU (alpha_nnet.py:49-50).
@@ -20,7 +20,6 @@
 #include <cuda_bf16.h>
 
 #include <algorithm>
-#include <cstdlib>
 #include <cstring>
 #include <vector>
 
@@ -30,13 +29,13 @@ namespace asz {
 
 constexpr int kC = 128;          // channels of the tower
 constexpr int kKC = kC / 8;      // 16-byte channel chunks
-constexpr int kTileM = 128;      // output rows (positions) per CTA
+constexpr int kTileM = 128;      // output rows (positions) per accumulator
 constexpr int kHalo = 40;        // >= pitch + 1 = max |tap shift| (39 for the 38-pitch raster of 19x19 boards)
 constexpr int kGuard = 48;       // zero rows before and after the activation arrays
-constexpr int kStages = 3;
 
 __host__ __device__ constexpr int pitch_of(int side) { return 2 * side; }            // 2*side-1 real + 1 pad
 __host__ __device__ constexpr int img_rows_of(int side) { return 2 * side; }         // 2*side-1 real + 1 pad
+static_assert(pitch_of(19) + 1 <= kHalo, "conv_umma_kernel<kHalo, ..> must cover every tap shift of 19x19 boards");
 
 // ---- PTX wrappers -------------------------------------------------------------------------------------------------
 __device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
@@ -45,9 +44,6 @@ __device__ __forceinline__ void mbar_init(uint64_t* bar, uint32_t count) {
 }
 __device__ __forceinline__ void mbar_expect_tx(uint64_t* bar, uint32_t bytes) {
   asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_arrive(uint64_t* bar) {
-  asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
 }
 __device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
   asm volatile(
@@ -67,27 +63,8 @@ __device__ __forceinline__ void bulk_g2s(void* dst, const void* src, uint32_t by
                "l"(src), "r"(bytes), "r"(smem_u32(bar))
                : "memory");
 }
-__device__ __forceinline__ void tmem_alloc(uint32_t* slot, uint32_t cols) {
-  asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(slot)), "r"(cols) : "memory");
-  asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-}
-__device__ __forceinline__ void tmem_dealloc(uint32_t taddr, uint32_t cols) {
-  asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(cols) : "memory");
-}
 __device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
 __device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void umma_bf16(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
-  asm volatile(
-      "{\n"
-      ".reg .pred p;\n"
-      "setp.ne.b32 p, %4, 0;\n"
-      "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n"
-      "}\n" ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
-__device__ __forceinline__ void umma_commit(uint64_t* bar) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
 __device__ __forceinline__ void tmem_ld32(uint32_t taddr, uint32_t (&v)[32]) {
   asm volatile(
       "tcgen05.ld.sync.aligned.32x32b.x32.b32 "
@@ -149,22 +126,14 @@ __device__ __forceinline__ void umma_commit_pair(uint64_t* bar) {
                : "memory");
 }
 
-// shared-memory matrix descriptor, K-major, no swizzle: 8x(16 B) core matrices, LBO = byte distance between the two
-// 16-byte K chunks of one K=16 step, SBO = byte distance between 8-row groups (cute/arch/mma_sm100_desc.hpp layout:
-// start [0,14), LBO [16,30), SBO [32,46), version [46,48) = 1, layout type [61,64) = 0)
-__device__ __forceinline__ uint64_t smem_desc(uint32_t saddr, uint32_t lbo_bytes, uint32_t sbo_bytes) {
-  return (uint64_t)((saddr >> 4) & 0x3FFFu) | ((uint64_t)((lbo_bytes >> 4) & 0x3FFFu) << 16) |
-         ((uint64_t)((sbo_bytes >> 4) & 0x3FFFu) << 32) | (1ull << 46);
-}
 // instruction descriptor kind::f16: D fp32 (bits 4-5 = 1), A and B bf16 (bits 7-9, 10-12 = 1), both K-major,
 // N >> 3 at bits 17-22, M >> 4 at bits 24-28
-constexpr uint32_t kIdesc = (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(kC >> 3) << 17) | ((uint32_t)(kTileM >> 4) << 24);
 constexpr uint32_t kIdescPair = (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(kC >> 3) << 17) | ((uint32_t)((2 * kTileM) >> 4) << 24);
 
 // ---- convolution kernel -----------------------------------------------------------------------------------------
 struct ConvParams {
-  const __nv_bfloat16* in;     // [kc_in][P_tot][8]
-  const __nv_bfloat16* wt;     // [taps][kc_in][128][8]
+  const __nv_bfloat16* in;     // [16][P_tot][8], or [1][P_tot][8] for the first layer's raster
+  const __nv_bfloat16* wt;     // pair layouts of pair_weight_layout_kernel / first_weight_layout_kernel
   const float* scale;          // [128] folded BN
   const float* bias;           // [128]
   const __nv_bfloat16* res;    // [16][P_tot][8] or null
@@ -172,8 +141,6 @@ struct ConvParams {
   const float* head_w;         // [128] or null
   float head_scale, head_bias;
   float* head_out;             // [P_tot] (head mode)
-  int kc_in;                   // 16, or 4 for the first layer's im2col input
-  int taps;                    // 9 or 1
   int pitch;                   // raster pitch (22 at 11x11)
   int img_stride;              // positions per image (pitch * rows)
   int real;                    // real rows / cols per image (21)
@@ -181,176 +148,41 @@ struct ConvParams {
   int P_real;                  // positions that belong to images of this launch
 };
 
-constexpr int kRowsA = kTileM + 2 * kHalo;   // 208
-
-struct ConvSmem {
-  // A: [kc][208][16 B], B stages: [kc][128][16 B]
-  static constexpr size_t a_bytes = (size_t)kKC * kRowsA * 16;           // 53,248
-  static constexpr size_t b_bytes = (size_t)kKC * kC * 16;               // 32,768
-  static constexpr size_t total = a_bytes + kStages * b_bytes + 2 * kC * sizeof(float) * 2 + 256;
-};
-
-__global__ void __launch_bounds__(192, 1) conv_tile_kernel(const ConvParams p) {
-  extern __shared__ __align__(128) unsigned char smem[];
-  unsigned char* sA = smem;
-  unsigned char* sB = smem + ConvSmem::a_bytes;
-  float* s_scale = reinterpret_cast<float*>(sB + kStages * ConvSmem::b_bytes);
-  float* s_bias = s_scale + kC;
-  float* s_head = s_bias + kC;
-  uint64_t* bars = reinterpret_cast<uint64_t*>(s_head + kC);   // [0] A full, [1..3] B full, [4..6] B empty, [7] acc full
-  uint32_t* s_tmem = reinterpret_cast<uint32_t*>(bars + 8);
-  const int warp = (int)(threadIdx.x >> 5), lane = (int)(threadIdx.x & 31);
-  const int m0 = (int)blockIdx.x * kTileM;                     // first output position of this tile (image space)
-  const int kc_in = p.kc_in, taps = p.taps;
-
-  for (int i = (int)threadIdx.x; i < kC; i += (int)blockDim.x) {
-    s_scale[i] = p.scale[i]; s_bias[i] = p.bias[i];
-    s_head[i] = p.head_w ? p.head_w[i] : 0.0f;
-  }
-  if (threadIdx.x == 0) {
-    mbar_init(&bars[0], 1);
-    for (int s = 0; s < kStages; ++s) { mbar_init(&bars[1 + s], 1); mbar_init(&bars[4 + s], 1); }
-    mbar_init(&bars[7], 1);
-    fence_barrier_init();
-  }
-  if (warp == 1) tmem_alloc(s_tmem, kC);   // 128 fp32 columns
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem_d = *s_tmem;
-
-  if (warp == 0) {
-    if (lane == 0) {
-      // ---- producer: A halo tile once, then the weights tap by tap ----
-      const size_t row0 = (size_t)kGuard + (size_t)m0 - kHalo;   // first halo row in the global arrays
-      mbar_expect_tx(&bars[0], (uint32_t)(kc_in * kRowsA * 16));
-      for (int kc = 0; kc < kc_in; ++kc)
-        bulk_g2s(sA + (size_t)kc * kRowsA * 16, p.in + ((size_t)kc * p.P_tot + row0) * 8, kRowsA * 16, &bars[0]);
-      const uint32_t tap_bytes = (uint32_t)(kc_in * kC * 16);
-      for (int t = 0; t < taps; ++t) {
-        const int s = t % kStages;
-        if (t >= kStages) mbar_wait(&bars[4 + s], (uint32_t)(((t / kStages) - 1) & 1));
-        mbar_expect_tx(&bars[1 + s], tap_bytes);
-        bulk_g2s(sB + (size_t)s * ConvSmem::b_bytes, p.wt + (size_t)t * kc_in * kC * 8, tap_bytes, &bars[1 + s]);
-      }
-    }
-  } else if (warp == 1) {
-    if (lane == 0) {
-      // ---- MMA issuer ----
-      mbar_wait(&bars[0], 0);
-      tc_fence_after();
-      const uint32_t a_base = smem_u32(sA), b_base = smem_u32(sB);
-      uint32_t acc = 0;
-      for (int t = 0; t < taps; ++t) {
-        const int s = t % kStages;
-        mbar_wait(&bars[1 + s], (uint32_t)((t / kStages) & 1));
-        tc_fence_after();
-        const int shift = (taps == 1) ? 0 : ((t / 3) - 1) * p.pitch + ((t % 3) - 1);
-        for (int ks = 0; ks < kc_in / 2; ++ks) {
-          const uint32_t a_addr = a_base + (uint32_t)(((2 * ks) * kRowsA + kHalo + shift) * 16);
-          const uint32_t b_addr = b_base + (uint32_t)(s * ConvSmem::b_bytes) + (uint32_t)((2 * ks) * kC * 16);
-          umma_bf16(tmem_d, smem_desc(a_addr, kRowsA * 16, 128), smem_desc(b_addr, kC * 16, 128), kIdesc, acc);
-          acc = 1;
-        }
-        umma_commit(&bars[4 + s]);   // frees this weight stage when the MMAs above have read it
-      }
-      umma_commit(&bars[7]);         // accumulator complete
-    }
-  } else {
-    // ---- epilogue: warps 2..5, TMEM lane quarter = warp % 4 ----
-    const int q = warp & 3;
-    const int r = q * 32 + lane;                 // row of the tile == TMEM lane
-    const int pos = m0 + r;                      // image-space position
-    const int rem = pos % p.img_stride;
-    const int y = rem / p.pitch, x = rem - y * p.pitch;
-    const bool valid = pos < p.P_real && y < p.real && x < p.real;
-    const size_t grow = (size_t)kGuard + (size_t)pos;
-    mbar_wait(&bars[7], 0);
-    tc_fence_after();
-    float head_acc = 0.0f;
-#pragma unroll 1
-    for (int cb = 0; cb < kC / 32; ++cb) {
-      uint32_t v[32];
-      tmem_ld32(tmem_d + ((uint32_t)(q * 32) << 16) + (uint32_t)(cb * 32), v);
-#pragma unroll
-      for (int j8 = 0; j8 < 4; ++j8) {
-        const int kc = cb * 4 + j8;
-        float f[8];
-#pragma unroll
-        for (int j = 0; j < 8; ++j) {
-          const int c = kc * 8 + j;
-          f[j] = __uint_as_float(v[j8 * 8 + j]) * s_scale[c] + s_bias[c];
-        }
-        if (p.res != nullptr) {
-          const uint4 rv = *reinterpret_cast<const uint4*>(p.res + ((size_t)kc * p.P_tot + grow) * 8);
-          const __nv_bfloat162* rb = reinterpret_cast<const __nv_bfloat162*>(&rv);
-#pragma unroll
-          for (int j = 0; j < 4; ++j) { const float2 t2 = __bfloat1622float2(rb[j]); f[2 * j] += t2.x; f[2 * j + 1] += t2.y; }
-        }
-#pragma unroll
-        for (int j = 0; j < 8; ++j) f[j] = valid ? fmaxf(f[j], 0.0f) : 0.0f;
-        if (p.out != nullptr) {
-          uint4 ov;
-          __nv_bfloat162* ob = reinterpret_cast<__nv_bfloat162*>(&ov);
-#pragma unroll
-          for (int j = 0; j < 4; ++j) ob[j] = __floats2bfloat162_rn(f[2 * j], f[2 * j + 1]);
-          *reinterpret_cast<uint4*>(p.out + ((size_t)kc * p.P_tot + grow) * 8) = ov;
-        }
-        if (p.head_out != nullptr) {
-#pragma unroll
-          for (int j = 0; j < 8; ++j) {
-            // the head convolution reads the bf16-rounded activation, like every other consumer of this layer would
-            const float a = __bfloat162float(__float2bfloat16_rn(f[j]));
-            head_acc = fmaf(a, s_head[kc * 8 + j], head_acc);
-          }
-        }
-      }
-    }
-    if (p.head_out != nullptr)
-      p.head_out[grow] = valid ? fmaxf(head_acc * p.head_scale + p.head_bias, 0.0f) : 0.0f;   // alpha_nnet.py:49-50
-    tc_fence_before();
-  }
-  __syncthreads();
-  if (warp == 1) { tc_fence_after(); tmem_dealloc(tmem_d, kC); }
-}
-
-// ---- persistent convolution kernel (single CTA or CTA pair) -------------------------------------------------------------
-// One CTA per SM loops over super-tiles of 256 positions.  Per super-tile the weights stream through shared memory once
-// (half a tap per stage) and feed two M=128 accumulators; TMEM holds two accumulator pairs (4 x 128 columns) so that the
-// epilogue of super-tile i overlaps the MMAs of super-tile i+1.
+// ---- persistent convolution kernel over CTA pairs -----------------------------------------------------------------------
+// The two CTAs of a cluster (the two SMs of a TPC) issue ONE tcgen05.mma.cta_group::2 of M = 256: every CTA supplies its own
+// 128 rows of A (its own halo tile) but only HALF of the weights (64 of the 128 output channels).  One pair per TPC loops over
+// pair super-tiles of 512 positions; CTA r owns positions [512 st + 256 r, +256).  Per super-tile the weights stream through
+// shared memory once (half a tap per stage; or stay resident, RESW) and feed two M=128 accumulators per CTA; TMEM holds two
+// accumulator pairs (4 x 128 columns) so that the epilogue of super-tile i overlaps the MMAs of super-tile i+1.
 //   warp 0      producer  : cp.async.bulk of the A halo tile and of the weight chunks, mbarrier complete_tx
-//   warp 1      MMA issuer: one elected thread, tcgen05.mma M128 N128 K16, tcgen05.commit releases stages / publishes accumulators
+//   warp 1      rank 0: MMA issuer, one elected thread, tcgen05.commit releases stages / publishes accumulators;
+//               rank 1: relays "my operands have landed" to rank 0's full barriers
 //   warps 2..9  epilogue  : tcgen05.ld, BN scale/bias, residual, ReLU, padding mask, bf16 store (or the fused head conv)
 // Loop order inside a super-tile: channel half c (8 of the 16 chunks) outermost, then the 9 taps.  The A half c is
 // released as soon as its 9 taps are issued, so the next super-tile's half 0 streams in while half 1 is being consumed:
 // the halo tile is effectively double buffered at 1x its size, which leaves room for 9+ weight stages.
+//   barriers    full barriers of rank 0 count 2 arrivals (own producer + the relay); empty / accumulator-full barriers are
+//               signalled in both CTAs by a multicast tcgen05.commit; accumulator-empty lives in rank 0 and counts the 16
+//               epilogue warps of the pair.
+//   weights     pair layout [tap][half][rank][8 kc][64 cout][8] (pair_weight_layout_kernel): a chunk is one bulk copy and
+//               is fetched from L2 once per CTA pair.
 //
 // The MMA issue loop is written for issue rate: an M128 N128 K16 MMA lasts 64 tensor cycles, and ONE thread has to issue
 // them back to back.  (tools/umma_probe.cu: the tensor pipe sustains 64.1 clk per MMA for every operand layout and shape
 // tried, with bulk-copy fills running; the first version of this loop spent 196 SASS instructions per 8 MMAs rebuilding
 // descriptors and walking divergence waterfalls and reached 46 % of that.)  So: the whole warp runs the loop in uniform
 // control flow, one elected lane issues; loops have compile-time trip counts; a descriptor's low word is base + constant.
-//
-// PAIR = true: the two CTAs of a cluster (the two SMs of a TPC) issue ONE tcgen05.mma.cta_group::2 of M = 256: every CTA
-// supplies its own 128 rows of A (its own halo tile) but only HALF of the weights (64 of the 128 output channels).
-//   work unit   a pair super-tile of 512 positions: CTA r owns positions [512 st + 256 r, +256)
-//   rank 0      issues the MMAs of the pair; rank 1's warp 1 relays "my operands have landed" to rank 0's full barriers
-//   barriers    full barriers of rank 0 count 2 arrivals (own producer + the relay); empty / accumulator-full barriers are
-//               signalled in both CTAs by a multicast tcgen05.commit; accumulator-empty lives in rank 0 and counts the 16
-//               epilogue warps of the pair.
-//   weights     pair layout [tap][half][rank][8 kc][64 cout][8] (pair_weight_layout_kernel): a chunk is one bulk copy and
-//               is fetched from L2 once per CTA pair.
-template <int HALO, bool PAIR>
+template <int HALO>
 struct UmmaSmem {
   static constexpr int kSuper = 256;                               // positions per CTA and weight pass
   static constexpr int rows = kSuper + 2 * HALO;
   static constexpr size_t a_bytes = (size_t)kKC * rows * 16;       // one halo tile, managed as two channel halves
-  static constexpr int b_rows = PAIR ? kC / 2 : kC;                // output channels whose weights this CTA holds
-  static constexpr size_t b_chunk = (size_t)8 * b_rows * 16;       // half a tap: 16 KB (8 KB per CTA of a pair)
+  static constexpr int b_rows = kC / 2;                            // output channels whose weights this CTA holds
+  static constexpr size_t b_chunk = (size_t)8 * b_rows * 16;       // half a tap: 8 KB per CTA
   static constexpr int max_stages = 18;                            // 18 = every weight chunk of a 3x3 layer (9 taps x 2 channel halves)
   static constexpr size_t tail = 3 * kC * sizeof(float) + (8 + 2 * max_stages) * sizeof(uint64_t) + 64;
   static constexpr int raw_stages = (int)((232448 - a_bytes - tail) / b_chunk);
-  static constexpr int b_stages = raw_stages > max_stages ? max_stages : raw_stages;   // 9 / 8 single; pair: 18 (HALO 24) / 17 (HALO 40)
+  static constexpr int b_stages = raw_stages > max_stages ? max_stages : raw_stages;   // 18 (HALO 24) / 17 (HALO 40)
   static constexpr size_t total = a_bytes + b_stages * b_chunk + tail;
 };
 
@@ -365,6 +197,9 @@ __device__ __forceinline__ bool elect_one() {
       : "=r"(pred));
   return pred != 0;
 }
+// shared-memory matrix descriptor, K-major, no swizzle: 8x(16 B) core matrices, LBO = byte distance between the two
+// 16-byte K chunks of one K=16 step, SBO = byte distance between 8-row groups (cute/arch/mma_sm100_desc.hpp layout:
+// start [0,14), LBO [16,30), SBO [32,46), version [46,48) = 1, layout type [61,64) = 0); lo = bits 0-31, hi = bits 32-63
 __device__ __forceinline__ uint64_t desc64(uint32_t lo, uint32_t hi) { return ((uint64_t)hi << 32) | (uint64_t)lo; }
 
 // FIRST = the first convolution (alpha_nnet.py:21-22, 3 input channels).  Its input is the same raster as every other layer's,
@@ -374,20 +209,20 @@ __device__ __forceinline__ uint64_t desc64(uint32_t lo, uint32_t hi) { return ((
 // (8 channels of tap 2j | 8 channels of tap 2j+1) of every row with the matching weight rows.  Five MMAs (the fifth pairs tap 8
 // with zero weights) instead of an im2col buffer: the layer reads 16 B per position where the im2col rows were 64 B, and the
 // separate im2col pass (write 64 B + read 64 B per position) is gone.  Weights: two chunks per tile, K steps 0..3 and K step 4.
-template <int HALO, bool PAIR, bool FIRST>
+template <int HALO, bool FIRST>
 __global__ void __launch_bounds__(320, 1) conv_umma_kernel(const ConvParams p, int n_tiles) {
-  using SM = UmmaSmem<HALO, PAIR>;
+  using SM = UmmaSmem<HALO>;
   constexpr int NS = SM::b_stages;
   constexpr int KC_HALF = FIRST ? 1 : 8;                           // channel chunks of A per half
   constexpr int HALVES = FIRST ? 1 : 2;
   constexpr int TAPS = FIRST ? 2 : 9;                              // weight chunks per half (FIRST: K steps 0..3, K step 4)
-  constexpr int TILE = PAIR ? 2 * SM::kSuper : SM::kSuper;         // positions per work unit
+  constexpr int TILE = 2 * SM::kSuper;                             // positions per work unit (pair super-tile)
   constexpr uint32_t chunk_bytes = (uint32_t)(8 * SM::b_rows * 16);          // a full weight chunk: 8 K chunks
   constexpr uint32_t last_chunk_bytes = FIRST ? (uint32_t)(2 * SM::b_rows * 16) : chunk_bytes;   // FIRST: K step 4 alone
-  // RESW: the CTA's half of the layer's weights (9 taps x 2 halves x 8 KB = 144 KB) fits next to the halo tile (11x11 boards, CTA
-  // pairs): it is loaded ONCE per launch and stays resident, instead of streaming through the stage ring once per super-tile
+  // RESW: the CTA's half of the layer's weights (9 taps x 2 halves x 8 KB = 144 KB) fits next to the halo tile (HALO 24: 7x7 and
+  // 11x11 boards): it is loaded ONCE per launch and stays resident, instead of streaming through the stage ring once per super-tile
   // (52 times per CTA and layer at 4,096 images).  Stage index = chunk index t * HALVES + c; b_full[0] is the only weight barrier.
-  constexpr bool RESW = PAIR && !FIRST && NS >= TAPS * HALVES;
+  constexpr bool RESW = !FIRST && NS >= TAPS * HALVES;
   extern __shared__ __align__(128) unsigned char smem[];
   unsigned char* sA = smem;
   unsigned char* sB = smem + SM::a_bytes;
@@ -398,33 +233,33 @@ __global__ void __launch_bounds__(320, 1) conv_umma_kernel(const ConvParams p, i
   uint64_t* a_full = bars;             // [2] channel halves
   uint64_t* a_empty = bars + 2;        // [2]
   uint64_t* acc_full = bars + 4;       // [2] accumulator pairs
-  uint64_t* acc_empty = bars + 6;      // [2] (of rank 0 in a pair)
+  uint64_t* acc_empty = bars + 6;      // [2] (of rank 0)
   uint64_t* b_full = bars + 8;         // [NS]
   uint64_t* b_empty = bars + 8 + SM::max_stages;   // [NS]
   uint32_t* s_tmem = reinterpret_cast<uint32_t*>(bars + 8 + 2 * SM::max_stages);
   const int warp = __shfl_sync(0xffffffffu, (int)(threadIdx.x >> 5), 0);   // provably warp-uniform
   const int lane = (int)(threadIdx.x & 31);
-  const uint32_t rank = PAIR ? cluster_ctarank() : 0u;
-  const int first_tile = PAIR ? (int)(blockIdx.x >> 1) : (int)blockIdx.x;
-  const int tile_step = PAIR ? (int)(gridDim.x >> 1) : (int)gridDim.x;
+  const uint32_t rank = cluster_ctarank();
+  const int first_tile = (int)(blockIdx.x >> 1);
+  const int tile_step = (int)(gridDim.x >> 1);
 
   for (int i = (int)threadIdx.x; i < kC; i += (int)blockDim.x) {
     s_scale[i] = p.scale[i]; s_bias[i] = p.bias[i];
     s_head[i] = p.head_w ? p.head_w[i] : 0.0f;
   }
   if (threadIdx.x == 0) {
-    const uint32_t full_count = (PAIR && rank == 0) ? 2u : 1u;
+    const uint32_t full_count = rank == 0 ? 2u : 1u;
     for (int i = 0; i < 2; ++i) {
       mbar_init(&a_full[i], full_count); mbar_init(&a_empty[i], 1);
-      mbar_init(&acc_full[i], 1); mbar_init(&acc_empty[i], PAIR ? 16 : 8);
+      mbar_init(&acc_full[i], 1); mbar_init(&acc_empty[i], 16);
     }
     for (int i = 0; i < NS; ++i) { mbar_init(&b_full[i], full_count); mbar_init(&b_empty[i], 1); }
     fence_barrier_init();
   }
-  if (warp == 1) { if (PAIR) tmem_alloc_pair(s_tmem, 512); else tmem_alloc(s_tmem, 512); }
+  if (warp == 1) tmem_alloc_pair(s_tmem, 512);
   tc_fence_before();
   __syncthreads();
-  if (PAIR) cluster_sync_all();   // the peer's barriers are initialised before anything is signalled across the pair
+  cluster_sync_all();   // the peer's barriers are initialised before anything is signalled across the pair
   tc_fence_after();
   const uint32_t tmem_base = *s_tmem;
 
@@ -432,7 +267,7 @@ __global__ void __launch_bounds__(320, 1) conv_umma_kernel(const ConvParams p, i
     if (lane == 0) {
       // ---- producer ----
       uint32_t stage = 0, phase = 0, it = 0;
-      constexpr size_t chunk_stride = (size_t)(PAIR ? 2 : 1) * (chunk_bytes / 2);        // bf16 elements between chunks
+      constexpr size_t chunk_stride = (size_t)2 * (chunk_bytes / 2);                     // bf16 elements between chunks
       if constexpr (RESW) {
         if (first_tile < n_tiles) {
           mbar_expect_tx(&b_full[0], (uint32_t)(TAPS * HALVES) * chunk_bytes);
@@ -458,11 +293,10 @@ __global__ void __launch_bounds__(320, 1) conv_umma_kernel(const ConvParams p, i
             const uint32_t bytes = (t == TAPS - 1) ? last_chunk_bytes : chunk_bytes;
             mbar_wait(&b_empty[stage], phase ^ 1u);
             mbar_expect_tx(&b_full[stage], bytes);
-            // single layout [tap][kc][128][8]: chunk (t, c) starts at (t * HALVES + c) * 8 * 128 * 8
-            // pair layout   [tap][half][rank][8][64][8]: chunk (t, c, rank) = ((t * HALVES + c) * 2 + rank) * chunk
-            // (FIRST: chunk 1 is short, and in the pair layout its two rank parts follow the two full parts of chunk 0)
-            const size_t off = (FIRST && PAIR && t == 1) ? (size_t)2 * (chunk_bytes / 2) + (size_t)rank * (last_chunk_bytes / 2)
-                                                         : (PAIR ? (size_t)rank * (chunk_bytes / 2) : 0) + (size_t)(t * HALVES + c) * chunk_stride;
+            // pair layout [tap][half][rank][8][64][8]: chunk (t, c, rank) = ((t * HALVES + c) * 2 + rank) * chunk
+            // (FIRST: chunk 1 is short, and its two rank parts follow the two full parts of chunk 0)
+            const size_t off = (FIRST && t == 1) ? (size_t)2 * (chunk_bytes / 2) + (size_t)rank * (last_chunk_bytes / 2)
+                                                 : (size_t)rank * (chunk_bytes / 2) + (size_t)(t * HALVES + c) * chunk_stride;
             bulk_g2s(sB + (size_t)stage * SM::b_chunk, p.wt + off, bytes, &b_full[stage]);
             if (++stage == NS) { stage = 0; phase ^= 1u; }
           }
@@ -471,13 +305,12 @@ __global__ void __launch_bounds__(320, 1) conv_umma_kernel(const ConvParams p, i
       }
     }
   } else if (warp == 1) {
-    if (!PAIR || rank == 0) {
+    if (rank == 0) {
       // ---- MMA issuer: the whole warp runs the loop (uniform control flow), one elected lane issues ----
       const bool issuer = elect_one();
       const uint32_t a_lo0 = ((smem_u32(sA) >> 4) & 0x3FFFu) | ((uint32_t)SM::rows << 16);      // LBO = rows * 16 B
       const uint32_t b_lo0 = ((smem_u32(sB) >> 4) & 0x3FFFu) | ((uint32_t)SM::b_rows << 16);    // LBO = b_rows * 16 B
       constexpr uint32_t desc_hi = (128u >> 4) | (1u << 14);                                     // SBO = 128 B, version 1
-      constexpr uint32_t idesc = PAIR ? kIdescPair : kIdesc;
       const int pitch = p.pitch;
       uint32_t stage = 0, phase = 0, it = 0;
       if constexpr (RESW) {
@@ -515,8 +348,7 @@ __global__ void __launch_bounds__(320, 1) conv_umma_kernel(const ConvParams p, i
                     const uint64_t ad = desc64((a_rows + (uint32_t)(sa + sub * kTileM)) | (lbo << 16), desc_hi);
                     const uint64_t bd = desc64(b_s + (uint32_t)(2 * ks * SM::b_rows), desc_hi);
                     const uint32_t acc = (j == 0) ? 0u : 1u;
-                    if (PAIR) umma_bf16_pair(tmem_d + (uint32_t)(sub * kC), ad, bd, idesc, acc);
-                    else umma_bf16(tmem_d + (uint32_t)(sub * kC), ad, bd, idesc, acc);
+                    umma_bf16_pair(tmem_d + (uint32_t)(sub * kC), ad, bd, kIdescPair, acc);
                   }
                 }
               } else {
@@ -528,19 +360,18 @@ __global__ void __launch_bounds__(320, 1) conv_umma_kernel(const ConvParams p, i
                     const uint64_t ad = desc64(a_t + (uint32_t)(sub * kTileM + 2 * ks * SM::rows), desc_hi);
                     const uint64_t bd = desc64(b_s + (uint32_t)(2 * ks * SM::b_rows), desc_hi);
                     const uint32_t acc = (t == 0 && ks == 0) ? (uint32_t)c : 1u;
-                    if (PAIR) umma_bf16_pair(tmem_d + (uint32_t)(sub * kC), ad, bd, idesc, acc);
-                    else umma_bf16(tmem_d + (uint32_t)(sub * kC), ad, bd, idesc, acc);
+                    umma_bf16_pair(tmem_d + (uint32_t)(sub * kC), ad, bd, kIdescPair, acc);
                   }
                 }
               }
-              if constexpr (!RESW) { if (PAIR) umma_commit_pair(&b_empty[stage]); else umma_commit(&b_empty[stage]); }
+              if constexpr (!RESW) umma_commit_pair(&b_empty[stage]);
             }
             __syncwarp();
             if constexpr (!RESW) { if (++stage == NS) { stage = 0; phase ^= 1u; } }
           }
-          if (issuer) { if (PAIR) umma_commit_pair(&a_empty[c]); else umma_commit(&a_empty[c]); }
+          if (issuer) umma_commit_pair(&a_empty[c]);
         }
-        if (issuer) { if (PAIR) umma_commit_pair(&acc_full[buf]); else umma_commit(&acc_full[buf]); }
+        if (issuer) umma_commit_pair(&acc_full[buf]);
         __syncwarp();
       }
     } else if (lane == 0) {
@@ -620,18 +451,15 @@ __global__ void __launch_bounds__(320, 1) conv_umma_kernel(const ConvParams p, i
       if (p.head_out != nullptr) p.head_out[grow] = valid ? fmaxf(head_acc * p.head_scale + p.head_bias, 0.0f) : 0.0f;
       tc_fence_before();
       __syncwarp();
-      if (lane == 0) {
-        if (PAIR) mbar_arrive_cluster(mapa_u32(smem_u32(&acc_empty[buf]), 0));
-        else mbar_arrive(&acc_empty[buf]);
-      }
+      if (lane == 0) mbar_arrive_cluster(mapa_u32(smem_u32(&acc_empty[buf]), 0));
     }
   }
   tc_fence_before();
   __syncthreads();
-  if (PAIR) cluster_sync_all();   // nobody leaves (or frees tensor memory) while the peer can still signal or accumulate
+  cluster_sync_all();   // nobody leaves (or frees tensor memory) while the peer can still signal or accumulate
   if (warp == 1) {
     tc_fence_after();
-    if (PAIR) tmem_dealloc_pair(tmem_base, 512); else tmem_dealloc(tmem_base, 512);
+    tmem_dealloc_pair(tmem_base, 512);
   }
 }
 
@@ -645,40 +473,6 @@ __global__ void pair_weight_layout_kernel(const __nv_bfloat16* __restrict__ src,
   const int c = kc / kc_half, k = kc % kc_half, r = cout / (kC / 2), co = cout % (kC / 2);
   const size_t o = ((((size_t)t * halves + c) * 2 + r) * kc_half + k) * (kC / 2) + co;
   reinterpret_cast<uint4*>(dst)[o] = reinterpret_cast<const uint4*>(src)[i];
-}
-
-// ---- input preparation: fp32 NHWC planes -> bf16 im2col rows of the first convolution (K = 27 padded to 32) --------
-__global__ void im2col_kernel(const float* __restrict__ planes, size_t plane_stride, int n_img, int real, int pitch, int img_stride, int P_tot,
-                              __nv_bfloat16* __restrict__ out /* [4][P_tot][8] */) {
-  const int pos = (int)(blockIdx.x * blockDim.x + threadIdx.x);
-  if (pos >= n_img * img_stride) return;
-  const int n = pos / img_stride, rem = pos - n * img_stride;
-  const int y = rem / pitch, x = rem - y * pitch;
-  float k[32];
-#pragma unroll
-  for (int i = 0; i < 32; ++i) k[i] = 0.0f;
-  if (y < real && x < real) {
-    const float* pl = planes + (size_t)n * plane_stride;
-#pragma unroll
-    for (int dy = 0; dy < 3; ++dy)
-#pragma unroll
-      for (int dx = 0; dx < 3; ++dx) {
-        const int yy = y + dy - 1, xx = x + dx - 1;
-        if (yy >= 0 && yy < real && xx >= 0 && xx < real) {
-          const float* s = pl + ((size_t)yy * real + xx) * 3;
-          k[(dy * 3 + dx) * 3 + 0] = s[0]; k[(dy * 3 + dx) * 3 + 1] = s[1]; k[(dy * 3 + dx) * 3 + 2] = s[2];
-        }
-      }
-  }
-  const size_t grow = (size_t)kGuard + (size_t)pos;
-#pragma unroll
-  for (int kc = 0; kc < 4; ++kc) {
-    uint4 ov;
-    __nv_bfloat162* ob = reinterpret_cast<__nv_bfloat162*>(&ov);
-#pragma unroll
-    for (int j = 0; j < 4; ++j) ob[j] = __floats2bfloat162_rn(k[kc * 8 + 2 * j], k[kc * 8 + 2 * j + 1]);
-    *reinterpret_cast<uint4*>(out + ((size_t)kc * P_tot + grow) * 8) = ov;
-  }
 }
 
 // ---- input of the persistent first convolution: fp32 NHWC planes -> the raster with one 16-byte chunk per position (3 channels
@@ -700,10 +494,9 @@ __global__ void planes_to_raster_kernel(const float* __restrict__ planes, size_t
 }
 
 // first-layer weights for the tap-paired contraction: the caller's im2col layout [4 kc][128][8] (k = tap * 3 + channel, 27 of 32
-// used) -> K chunk t = the 8 channel slots of tap t (3 real), 10 chunks (tap 9 = zeros):
-//   single [10][128][8];   pair [chunk 0: rank][8][64][8] then [chunk 1: rank][2][64][8]
-__global__ void first_weight_layout_kernel(const __nv_bfloat16* __restrict__ src, __nv_bfloat16* __restrict__ dst_single,
-                                           __nv_bfloat16* __restrict__ dst_pair) {
+// used) -> K chunk t = the 8 channel slots of tap t (3 real), 10 chunks (tap 9 = zeros), split for CTA pairs:
+//   [chunk 0: rank][8][64][8] then [chunk 1: rank][2][64][8]
+__global__ void first_weight_layout_kernel(const __nv_bfloat16* __restrict__ src, __nv_bfloat16* __restrict__ dst) {
   const int i = (int)(blockIdx.x * blockDim.x + threadIdx.x);      // (tap chunk, cout)
   if (i >= 10 * kC) return;
   const int t = i / kC, cout = i - t * kC;
@@ -713,11 +506,9 @@ __global__ void first_weight_layout_kernel(const __nv_bfloat16* __restrict__ src
     const int k = t * 3 + c;
     v[c] = (t < 9 && c < 3) ? src[((size_t)(k >> 3) * kC + cout) * 8 + (k & 7)] : __float2bfloat16_rn(0.0f);
   }
-  const uint4 pk = *reinterpret_cast<const uint4*>(v);
-  reinterpret_cast<uint4*>(dst_single)[(size_t)t * kC + cout] = pk;
   const int r = cout / (kC / 2), co = cout % (kC / 2);
   const size_t o = t < 8 ? ((size_t)r * 8 + t) * (kC / 2) + co : (size_t)2 * 8 * (kC / 2) + ((size_t)r * 2 + (t - 8)) * (kC / 2) + co;
-  reinterpret_cast<uint4*>(dst_pair)[o] = pk;
+  reinterpret_cast<uint4*>(dst)[o] = *reinterpret_cast<const uint4*>(v);
 }
 
 // ---- dense head: Flatten + Dense(128) + ReLU + Dense(3) + tanh (alpha_nnet.py:52-54), 8 images per CTA ------------------
@@ -793,40 +584,32 @@ __global__ void dense1_raster_kernel(const float* __restrict__ w1, int real, int
 
 
 
-template <int HALO, bool PAIR, bool FIRST>
+template <int HALO, bool FIRST>
 static int configure_one() {
-  return cuda_ok(cudaFuncSetAttribute(conv_umma_kernel<HALO, PAIR, FIRST>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                      (int)UmmaSmem<HALO, PAIR>::total), "cudaFuncSetAttribute(conv_umma_kernel)") ? ASZ_OK : ASZ_ERR_CUDA;
+  return cuda_ok(cudaFuncSetAttribute(conv_umma_kernel<HALO, FIRST>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                      (int)UmmaSmem<HALO>::total), "cudaFuncSetAttribute(conv_umma_kernel)") ? ASZ_OK : ASZ_ERR_CUDA;
 }
 static int configure_umma_kernels() {
   int rc = ASZ_OK;
-  if ((rc = configure_one<24, false, false>()) != ASZ_OK) return rc;
-  if ((rc = configure_one<24, false, true>()) != ASZ_OK) return rc;
-  if ((rc = configure_one<40, false, false>()) != ASZ_OK) return rc;
-  if ((rc = configure_one<40, false, true>()) != ASZ_OK) return rc;
-  if ((rc = configure_one<24, true, false>()) != ASZ_OK) return rc;
-  if ((rc = configure_one<24, true, true>()) != ASZ_OK) return rc;
-  if ((rc = configure_one<40, true, false>()) != ASZ_OK) return rc;
-  if ((rc = configure_one<40, true, true>()) != ASZ_OK) return rc;
+  if ((rc = configure_one<24, false>()) != ASZ_OK) return rc;
+  if ((rc = configure_one<24, true>()) != ASZ_OK) return rc;
+  if ((rc = configure_one<kHalo, false>()) != ASZ_OK) return rc;
+  if ((rc = configure_one<kHalo, true>()) != ASZ_OK) return rc;
   return rc;
 }
-template <int HALO, bool PAIR, bool FIRST>
+template <int HALO, bool FIRST>
 static int launch_one(int grid, const ConvParams& p, int n_tiles, cudaStream_t st) {
   cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3((unsigned)grid); cfg.blockDim = dim3(320); cfg.dynamicSmemBytes = UmmaSmem<HALO, PAIR>::total; cfg.stream = st;
+  cfg.gridDim = dim3((unsigned)grid); cfg.blockDim = dim3(320); cfg.dynamicSmemBytes = UmmaSmem<HALO>::total; cfg.stream = st;
   cudaLaunchAttribute at[1];
   at[0].id = cudaLaunchAttributeClusterDimension;
-  at[0].val.clusterDim.x = PAIR ? 2 : 1; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
+  at[0].val.clusterDim.x = 2; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
   cfg.attrs = at; cfg.numAttrs = 1;
-  return cuda_ok(cudaLaunchKernelEx(&cfg, conv_umma_kernel<HALO, PAIR, FIRST>, p, n_tiles), "conv_umma_kernel") ? ASZ_OK : ASZ_ERR_CUDA;
+  return cuda_ok(cudaLaunchKernelEx(&cfg, conv_umma_kernel<HALO, FIRST>, p, n_tiles), "conv_umma_kernel") ? ASZ_OK : ASZ_ERR_CUDA;
 }
-static int launch_umma(bool pair, bool big, bool first, int grid, const ConvParams& p, int n_tiles, cudaStream_t st) {
-  if (!big) {
-    if (!pair) return first ? launch_one<24, false, true>(grid, p, n_tiles, st) : launch_one<24, false, false>(grid, p, n_tiles, st);
-    return first ? launch_one<24, true, true>(grid, p, n_tiles, st) : launch_one<24, true, false>(grid, p, n_tiles, st);
-  }
-  if (!pair) return first ? launch_one<40, false, true>(grid, p, n_tiles, st) : launch_one<40, false, false>(grid, p, n_tiles, st);
-  return first ? launch_one<40, true, true>(grid, p, n_tiles, st) : launch_one<40, true, false>(grid, p, n_tiles, st);
+static int launch_umma(bool big, bool first, int grid, const ConvParams& p, int n_tiles, cudaStream_t st) {
+  if (!big) return first ? launch_one<24, true>(grid, p, n_tiles, st) : launch_one<24, false>(grid, p, n_tiles, st);
+  return first ? launch_one<kHalo, true>(grid, p, n_tiles, st) : launch_one<kHalo, false>(grid, p, n_tiles, st);
 }
 
 }  // namespace asz
@@ -839,16 +622,13 @@ struct asz_net {
   int chunk = 0;           // images per pass
   int P_tot = 0;           // rows of the activation arrays (guards + padded positions)
   __nv_bfloat16* act[3] = {nullptr, nullptr, nullptr};
-  __nv_bfloat16* col = nullptr;   // im2col input of the first layer [4][P_tot][8]
+  __nv_bfloat16* col = nullptr;   // input raster of the first layer [P_tot][8] (planes_to_raster_kernel)
   float* head = nullptr;          // [P_tot]
   float* w1r = nullptr;           // dense1 weights on the padded raster [img_stride][128]
   int n_sm = 148;
   int device = 0;                 // the device this network lives on (asz_net_create's current device)
-  int variant = 3;                // 1 = one tile per CTA (conv_tile_kernel), 2 = persistent (conv_umma_kernel, one CTA per SM),
-                                  // 3 = persistent over CTA pairs (conv_umma_kernel PAIR, cta_group::2)
   __nv_bfloat16* w_pair[9] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
-  __nv_bfloat16* w_first = nullptr;        // first-layer weights, tap-paired layout [10][128][8] (first_weight_layout_kernel)
-  __nv_bfloat16* w_first_pair = nullptr;   // ... split for CTA pairs
+  __nv_bfloat16* w_first_pair = nullptr;   // first-layer weights, tap-paired and split for CTA pairs (first_weight_layout_kernel)
 };
 
 static int net_forward_impl(asz_net* n, const float* d_planes, int32_t count, float* d_values, int stop_layer, float* d_act, cudaStream_t st,
@@ -860,7 +640,7 @@ extern "C" {
 static int net_derive(asz_net* n, cudaStream_t st) {
   dense1_raster_kernel<<<(n->img_stride * 128 + 255) / 256, 256, 0, st>>>(n->w.dense1_w, n->real, n->pitch, n->img_stride, n->w1r);
   if (!cuda_ok(cudaGetLastError(), "dense1_raster_kernel")) return ASZ_ERR_CUDA;
-  first_weight_layout_kernel<<<(10 * kC + 255) / 256, 256, 0, st>>>(reinterpret_cast<const __nv_bfloat16*>(n->w.w_conv[0]), n->w_first, n->w_first_pair);
+  first_weight_layout_kernel<<<(10 * kC + 255) / 256, 256, 0, st>>>(reinterpret_cast<const __nv_bfloat16*>(n->w.w_conv[0]), n->w_first_pair);
   if (!cuda_ok(cudaGetLastError(), "first_weight_layout_kernel")) return ASZ_ERR_CUDA;
   for (int l = 1; l < 9; ++l) {
     const int total = 9 * kKC * kC;
@@ -874,7 +654,6 @@ static int net_derive(asz_net* n, cudaStream_t st) {
 static int net_alloc(asz_net* n, const asz_net_weights* w, int32_t chunk_images) {
   n->w = *w;
   n->side = w->side; n->real = 2 * w->side - 1; n->pitch = pitch_of(w->side); n->img_stride = n->pitch * img_rows_of(w->side);
-  if (n->pitch + 1 > kHalo) { set_error("board too large for the halo of conv_tile_kernel"); return ASZ_ERR_ARG; }
   n->chunk = chunk_images;
   const size_t P = (size_t)chunk_images * n->img_stride;
   const size_t P_pad = (P + 511) / 512 * 512;                 // whole pair super-tiles
@@ -884,25 +663,21 @@ static int net_alloc(asz_net* n, const asz_net_weights* w, int32_t chunk_images)
     ASZ_CUDA(cudaMalloc(&n->act[i], act_bytes));
     ASZ_CUDA(cudaMemset(n->act[i], 0, act_bytes));
   }
-  ASZ_CUDA(cudaMalloc(&n->col, (size_t)4 * n->P_tot * 8 * sizeof(__nv_bfloat16)));
-  ASZ_CUDA(cudaMemset(n->col, 0, (size_t)4 * n->P_tot * 8 * sizeof(__nv_bfloat16)));
+  ASZ_CUDA(cudaMalloc(&n->col, (size_t)n->P_tot * 8 * sizeof(__nv_bfloat16)));
+  ASZ_CUDA(cudaMemset(n->col, 0, (size_t)n->P_tot * 8 * sizeof(__nv_bfloat16)));
   ASZ_CUDA(cudaMalloc(&n->head, (size_t)n->P_tot * sizeof(float)));
   ASZ_CUDA(cudaMemset(n->head, 0, (size_t)n->P_tot * sizeof(float)));
-  ASZ_CUDA(cudaFuncSetAttribute(conv_tile_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ConvSmem::total));
   {
     int dev = 0; cudaDeviceProp prop;
     ASZ_CUDA(cudaGetDevice(&dev));
     ASZ_CUDA(cudaGetDeviceProperties(&prop, dev));
     n->n_sm = prop.multiProcessorCount;
     n->device = dev;
-    const char* v = getenv("ASZ_NET_VARIANT");
-    if (v && v[0] >= '1' && v[0] <= '3') n->variant = v[0] - '0';
   }
   { int rc = configure_umma_kernels(); if (rc != ASZ_OK) return rc; }
   ASZ_CUDA(cudaFuncSetAttribute(dense_head_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024));
   ASZ_CUDA(cudaMalloc(&n->w1r, (size_t)n->img_stride * 128 * sizeof(float)));
   for (int l = 1; l < 9; ++l) ASZ_CUDA(cudaMalloc(&n->w_pair[l], (size_t)9 * kKC * kC * 16));
-  ASZ_CUDA(cudaMalloc(&n->w_first, (size_t)10 * kC * 16));
   ASZ_CUDA(cudaMalloc(&n->w_first_pair, (size_t)10 * kC * 16));
   { int rc = net_derive(n, nullptr); if (rc != ASZ_OK) return rc; }
   ASZ_CUDA(cudaDeviceSynchronize());
@@ -938,7 +713,7 @@ int asz_net_destroy(asz_net* n) {
   for (int i = 0; i < 3; ++i) cudaFree(n->act[i]);
   cudaFree(n->col); cudaFree(n->head); cudaFree(n->w1r);
   for (int l = 0; l < 9; ++l) cudaFree(n->w_pair[l]);
-  cudaFree(n->w_first); cudaFree(n->w_first_pair);
+  cudaFree(n->w_first_pair);
   delete n;
   return ASZ_OK;
 }
@@ -947,32 +722,16 @@ static int launch_conv(asz_net* n, int layer, const __nv_bfloat16* in, const __n
                        int n_img, cudaStream_t st) {
   ConvParams p;
   memset(&p, 0, sizeof p);
-  p.in = in; p.wt = reinterpret_cast<const __nv_bfloat16*>(n->w.w_conv[layer]);
+  p.in = in; p.wt = layer == 0 ? n->w_first_pair : n->w_pair[layer];
   p.scale = n->w.scale[layer]; p.bias = n->w.bias[layer];
   p.res = res; p.out = outp;
   if (head) { p.head_w = n->w.head_w; p.head_scale = n->w.head_scale; p.head_bias = n->w.head_bias; p.head_out = n->head; }
-  p.kc_in = layer == 0 ? 4 : kKC; p.taps = layer == 0 ? 1 : 9;
   p.pitch = n->pitch; p.img_stride = n->img_stride; p.real = n->real; p.P_tot = n->P_tot;
   p.P_real = n_img * n->img_stride;
-  if (n->variant == 1) {
-    const int tiles = (p.P_real + kTileM - 1) / kTileM;
-    conv_tile_kernel<<<tiles, 192, ConvSmem::total, st>>>(p);
-    return cuda_ok(cudaGetLastError(), "conv_tile_kernel") ? ASZ_OK : ASZ_ERR_CUDA;
-  }
-  const bool pair = n->variant == 3;
-  if (layer == 0) p.wt = pair ? n->w_first_pair : n->w_first;
-  else if (pair) p.wt = n->w_pair[layer];
   const bool big = n->pitch + 1 > 24;
-  const int n_tiles = pair ? (p.P_real + 511) / 512 : (p.P_real + 255) / 256;
-  const int grid = pair ? 2 * std::min(n_tiles, n->n_sm / 2) : std::min(n_tiles, n->n_sm);
-  return launch_umma(pair, big, layer == 0, grid, p, n_tiles, st);
-}
-
-int asz_net_set_variant(asz_net* n, int32_t variant) {
-  if (!n) { set_error("null argument"); return ASZ_ERR_ARG; }
-  if (variant < 1 || variant > 3) { set_error("variant must be 1 (tile), 2 (persistent) or 3 (CTA pair)"); return ASZ_ERR_ARG; }
-  n->variant = variant;
-  return ASZ_OK;
+  const int n_tiles = (p.P_real + 511) / 512;                   // pair super-tiles
+  const int grid = 2 * std::min(n_tiles, n->n_sm / 2);
+  return launch_umma(big, layer == 0, grid, p, n_tiles, st);
 }
 
 int asz_net_forward(asz_net* n, const float* d_planes, int32_t count, float* d_values, void* stream) {
@@ -1031,13 +790,8 @@ static int net_forward_impl(asz_net* n, const float* d_planes, int32_t count, fl
   for (int i0 = 0; i0 < count; i0 += per_pass) {
     const int m = std::min(per_pass, count - i0);
     const int P = m * n->img_stride;
-    if (n->variant == 1) {     // one tile per CTA: im2col rows, one tap over K = 32
-      im2col_kernel<<<(P + 127) / 128, 128, 0, st>>>(d_planes + (size_t)i0 * plane, plane, m, n->real, n->pitch, n->img_stride, n->P_tot, n->col);
-      if (!cuda_ok(cudaGetLastError(), "im2col_kernel")) return ASZ_ERR_CUDA;
-    } else {                   // persistent kernels: the 8-channel raster, taps contracted two per MMA
-      planes_to_raster_kernel<<<(P + 255) / 256, 256, 0, st>>>(d_planes + (size_t)i0 * plane, plane, m, n->real, n->pitch, n->img_stride, n->col);
-      if (!cuda_ok(cudaGetLastError(), "planes_to_raster_kernel")) return ASZ_ERR_CUDA;
-    }
+    planes_to_raster_kernel<<<(P + 255) / 256, 256, 0, st>>>(d_planes + (size_t)i0 * plane, plane, m, n->real, n->pitch, n->img_stride, n->col);
+    if (!cuda_ok(cudaGetLastError(), "planes_to_raster_kernel")) return ASZ_ERR_CUDA;
     int rc = launch_conv(n, 0, n->col, nullptr, n->act[0], false, m, st);          // alpha_nnet.py:21-22
     if (rc != ASZ_OK) return rc;
     if (stop_layer == 0) return dump(n->act[0], nullptr, m);

@@ -34,7 +34,7 @@ def _conv0_layout(k):
 
 class NativeNet:
 
-    def __init__(self, weights, device, chunk_images=16384, variant=None):
+    def __init__(self, weights, device, chunk_images=16384):
         if not torch.cuda.is_available():
             raise _lib.AszError("no CUDA device: the native network has no CPU fallback")
         self.device = torch.device(device)
@@ -47,8 +47,6 @@ class NativeNet:
         with torch.cuda.device(self.device):
             check(self.L.asz_net_create(C.byref(h), C.byref(nw), chunk_images))
         self.h = h
-        if variant is not None:
-            check(self.L.asz_net_set_variant(self.h, int(variant)))
 
     def _upload(self, weights):
         """device copies of the weights in the layouts the kernels consume -> (tensors kept alive, asz_net_weights)"""

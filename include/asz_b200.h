@@ -280,10 +280,6 @@ int asz_net_destroy(asz_net* net);
 /* the per-generation weight push (alpha_snake_zero_trainer.py:52-57, 79-83): *w replaces the network's weight pointers
  * (same side; arrays stay owned by the caller) and the operands derived from them are rebuilt on `stream` */
 int asz_net_update_weights(asz_net* net, const asz_net_weights* w, void* stream);
-/* convolution kernel variant: 1 = one tile per CTA, 2 = persistent single-CTA, 3 = persistent CTA pairs (cta_group::2).
- * 2 and 3 compute the same bits (same accumulation order), 1 agrees to bf16 rounding; the default is 3, the fastest
- * (environment override: ASZ_NET_VARIANT). */
-int asz_net_set_variant(asz_net* net, int32_t variant);
 /* d_planes [count][2*side-1][2*side-1][3] float32 NHWC -> d_values [count][3] float32 tanh outputs (no obstacle mask;
  * asz_obstacle_mask applies AlphaNNet.v's mask).  bf16 operands, fp32 accumulation. */
 int asz_net_forward(asz_net* net, const float* d_planes, int32_t count, float* d_values, void* stream);

@@ -83,26 +83,18 @@ def test_native_net_layer_by_layer(side, S):
 
 
 @pytest.mark.parametrize("side,S,n,chunk", [(11, 4, 700, 256), (7, 4, 90, 32), (19, 8, 40, 16)])
-def test_conv_variants_agree(side, S, n, chunk):
-    """the persistent single-CTA and CTA-pair (cta_group::2) convolutions accumulate in the same order: identical bits on
-    every layer and on the outputs; the one-tile-per-CTA kernel accumulates tap-major instead of channel-half-major and
-    agrees to bf16 rounding (chunk sizes chosen so that several chunks and a ragged last pair tile occur)"""
+def test_chunked_forward_bit_identical(side, S, n, chunk):
+    """a forward split into several passes of chunk_images gives the same bits as one pass over the whole batch (chunk sizes
+    chosen so that several passes and a ragged last pair tile occur)"""
     import torch
     from alphasnake_zero_b200.net import NativeNet
     from oracle import net_oracle as no
     w = no.init_weights(side, seed=11, randomize_bn=True)
     X = torch.from_numpy(game_planes(side, S, n, seed=7)).cuda()
-    nets = {v: NativeNet(w, "cuda", chunk_images=chunk, variant=v) for v in (1, 2, 3)}
-    outs = {v: net.forward(X).cpu().numpy() for v, net in nets.items()}
-    assert np.isfinite(outs[2]).all() and np.abs(outs[2]).max() > 0.01
-    assert np.array_equal(outs[3].view(np.uint32), outs[2].view(np.uint32))
-    assert np.abs(outs[1] - outs[2]).max() < 1e-2
-    m = min(n, chunk)
-    for layer in (0, 1, 4, 8):
-        acts = {v: net.debug_layer(X[:m], layer).cpu().numpy() for v, net in nets.items()}
-        assert np.array_equal(acts[3].view(np.uint32), acts[2].view(np.uint32)), layer
-        # different accumulation order => different bf16 roundings, which compound over the layers
-        assert np.abs(acts[1] - acts[2]).max() <= 0.03 * np.abs(acts[2]).max() + 1e-3, layer
+    chunked = NativeNet(w, "cuda", chunk_images=chunk).forward(X).cpu().numpy()
+    whole = NativeNet(w, "cuda", chunk_images=n).forward(X).cpu().numpy()
+    assert np.isfinite(whole).all() and np.abs(whole).max() > 0.01
+    assert np.array_equal(chunked.view(np.uint32), whole.view(np.uint32))
 
 
 def test_weight_update_equals_a_fresh_network():

@@ -35,13 +35,12 @@ def main():
         e1.record()
         torch.cuda.synchronize()
         return e0.elapsed_time(e1) / reps * 1e-3
-    for v in (2, 3):
-        for ch in sorted({chunk, 4 * chunk} if "--chunks" in sys.argv else {chunk}):
-            nat = NativeNet(w, "cuda", chunk_images=ch, variant=v)
-            t = timeit(lambda: nat.forward(x))
-            out["native_bf16_v%d_chunk%d" % (v, ch)] = {"evals_per_s": n / t, "tflops": n / t * FLOPS[side] / 1e12 if FLOPS[side] else None,
-                                                         "ms": t * 1e3}
-            del nat
+    for ch in sorted({chunk, 4 * chunk} if "--chunks" in sys.argv else {chunk}):
+        nat = NativeNet(w, "cuda", chunk_images=ch)
+        t = timeit(lambda: nat.forward(x))
+        out["native_bf16_chunk%d" % ch] = {"evals_per_s": n / t, "tflops": n / t * FLOPS[side] / 1e12 if FLOPS[side] else None,
+                                           "ms": t * 1e3}
+        del nat
     if "--no-torch" in sys.argv:
         print(json.dumps({"n": n, "side": side, "chunk": chunk, **out}))
         return

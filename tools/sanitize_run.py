@@ -23,11 +23,9 @@ def main():
             eng.step(spawn_mode=_lib.SPAWN_NATIVE, tic=True, encode=True, auto_reset=True, random_actions=True, keys=True)
         net = AlphaNNet(input_shape=(2 * side - 1, 2 * side - 1, 3), seed=0, backend="native")
         net._native = NativeNet(net.weights, "cuda", chunk_images=64)
-        for variant in (3, 2, 1):
-            _lib.check(_lib.lib().asz_net_set_variant(net._native.h, variant))
-            q, mv = eng.search(net=net._native)
-            act = torch.where(mv < 3, mv, torch.ones_like(mv))
-            eng.step(actions=act, spawn_mode=_lib.SPAWN_NATIVE, tic=True, encode=False, auto_reset=True)
+        q, mv = eng.search(net=net._native)
+        act = torch.where(mv < 3, mv, torch.ones_like(mv))
+        eng.step(actions=act, spawn_mode=_lib.SPAWN_NATIVE, tic=True, encode=False, auto_reset=True)
         q, mv = eng.search(value_fn=None)
         torch.cuda.synchronize()
         st = eng.search_stats()
