@@ -9,6 +9,7 @@ LIB_PATH = os.environ.get("ASZ_LIB") or os.path.join(HERE, "libasz_b200.so")   #
 ASZ_MAX_SNAKES = 8
 STEP_TIC, STEP_ENCODE, STEP_AUTO_RESET, STEP_RANDOM_ACT, STEP_KEYS = 1, 2, 4, 8, 16
 SPAWN_NONE, SPAWN_REPLAY, SPAWN_NATIVE = 0, 1, 2
+ASZ_ERR_ARG, ASZ_ERR_CUDA, ASZ_ERR_STATE, ASZ_ERR_CAPACITY = -1, -2, -3, -4
 
 
 class AszError(RuntimeError):
@@ -33,6 +34,10 @@ class NetWeights(C.Structure):
     _fields_ = [("side", C.c_int32), ("w_conv", C.c_void_p * 9), ("scale", C.c_void_p * 9), ("bias", C.c_void_p * 9),
                 ("head_w", C.c_void_p), ("head_scale", C.c_float), ("head_bias", C.c_float), ("dense1_w", C.c_void_p),
                 ("dense1_b", C.c_void_p), ("dense2_w", C.c_void_p), ("dense2_b", C.c_void_p)]
+
+
+class PitPlayer(C.Structure):
+    _fields_ = [("net", C.c_void_p), ("stub_word", C.c_int32)]
 
 
 _lib = None
@@ -93,6 +98,11 @@ SYMBOLS = [
     ("asz_net_forward", C.c_int, [_vp, _vp, _i32, _vp, _vp]),
     ("asz_net_forward_pitched", C.c_int, [_vp, _vp, _i32, _i32, _vp, _vp]),
     ("asz_net_debug_layer", C.c_int, [_vp, _vp, _i32, _i32, _vp, _vp]),
+    ("asz_pit_begin", C.c_int, [_vp, C.POINTER(PitPlayer), C.POINTER(PitPlayer), _i32, _vp, _vp]),
+    ("asz_pit_turn", C.c_int, [_vp, _i32, _vp, _vp, _vp, _vp]),
+    ("asz_pit_finish", C.c_int, [_vp, _vp, _vp, _vp, _vp]),
+    ("asz_pit_run", C.c_int, [_vp, C.POINTER(PitPlayer), C.POINTER(PitPlayer), _i32, _i32, _vp, _vp, _vp, _vp]),
+    ("asz_pit_stats", C.c_int, [_vp, _vp]),
 ]
 
 

@@ -7,7 +7,7 @@ from concurrent.futures import ThreadPoolExecutor
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libasz_b200.so")
-SOURCES = ["asz_env.cu", "asz_mcts.cu", "asz_net.cu", "asz_records.cu"]
+SOURCES = ["asz_env.cu", "asz_mcts.cu", "asz_net.cu", "asz_records.cu", "asz_pit.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17", "-Xcompiler", "-fPIC",
               "--expt-relaxed-constexpr"]
 

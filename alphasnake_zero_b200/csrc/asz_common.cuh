@@ -66,6 +66,13 @@ __host__ __device__ __forceinline__ void key_accumulate(uint32_t pix, uint32_t a
   k1 += fmix64(fmix64(x ^ 0xC2B2AE3D27D4EB4FULL) + y);
 }
 
+// ---- policy -----------------------------------------------------------------------------------------------------
+// Agent.argmaxs (agent.py:124-137, pit_agent.py:16-23) with its tie rule: a tie between 0 and 1 goes to 1 or 2, ties with 2 go to 2
+__device__ __forceinline__ int argmax3(const float z[3]) {
+  if (z[0] > z[1]) return (z[0] > z[2]) ? 0 : 2;
+  return (z[1] > z[2]) ? 1 : 2;
+}
+
 // ---- warp helpers -----------------------------------------------------------------------------------------------
 __device__ __forceinline__ int lane_id() { return (int)(threadIdx.x & 31u); }
 __device__ __forceinline__ uint64_t warp_sum_u64(uint64_t v) {

@@ -20,6 +20,7 @@ bool cuda_ok(cudaError_t err, const char* what);
 
 struct SearchState;   // asz_mcts.cu
 struct RecordStore;   // asz_records.cu
+struct PitState;      // asz_pit.cu
 
 // Every entry point that takes an engine (or a network) runs on THAT object's device, whatever device is current in the
 // calling thread ("one engine per GPU": several engines on different GPUs may live in one process).
@@ -94,6 +95,7 @@ struct asz_engine {
   } hostpipe;
   asz::SearchState* search = nullptr;
   asz::RecordStore* records = nullptr;   // device-resident training records (asz_records_*)
+  asz::PitState* pit = nullptr;          // two-network match (asz_pit_*), allocated by the first asz_pit_begin
 };
 
 namespace asz {
@@ -102,5 +104,9 @@ void gameset_free(GameSet& gs);
 int search_create(asz_engine* e);
 void search_destroy(asz_engine* e);
 void records_destroy(asz_engine* e);
+void pit_destroy(asz_engine* e);
 void host_pipe_destroy(asz_engine* e);
+// board side and device of a value network (asz_net.cu)
+int net_side(const asz_net* n);
+int net_device(const asz_net* n);
 }  // namespace asz

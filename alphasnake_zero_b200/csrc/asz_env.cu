@@ -581,6 +581,7 @@ int asz_engine_destroy(asz_engine* e) {
   cudaDeviceSynchronize();   // launches and copies still in flight (asz_env_submit_host never waited for) use the buffers freed below
   search_destroy(e);
   records_destroy(e);
+  pit_destroy(e);
   host_pipe_destroy(e);
   gameset_free(e->root);
   cudaFree(e->planes); cudaFree(e->row_ids); cudaFree(e->row_count); cudaFree(e->totals);

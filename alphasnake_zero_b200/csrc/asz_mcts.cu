@@ -334,12 +334,6 @@ __device__ __forceinline__ int choice3(const float pmf[3], double u) {
   if (c1 / c2 <= u) idx = 2;
   return idx;
 }
-// agent.py:124-137
-__device__ __forceinline__ int argmax3(const float z[3]) {
-  if (z[0] > z[1]) return (z[0] > z[2]) ? 0 : 2;
-  return (z[1] > z[2]) ? 1 : 2;
-}
-
 __device__ __forceinline__ void read_q(const Table& t, uint32_t slot, float q[3]) {
   const float4 w = t.w[slot], n = t.n[slot];
   q[0] = __fdiv_rn(w.x, n.x); q[1] = __fdiv_rn(w.y, n.y); q[2] = __fdiv_rn(w.z, n.z);

@@ -634,6 +634,11 @@ struct asz_net {
 static int net_forward_impl(asz_net* n, const float* d_planes, int32_t count, float* d_values, int stop_layer, float* d_act, cudaStream_t st,
                             size_t plane_stride = 0);
 
+namespace asz {
+int net_side(const asz_net* n) { return n->side; }
+int net_device(const asz_net* n) { return n->device; }
+}  // namespace asz
+
 extern "C" {
 
 // operands derived from the caller's weight arrays: dense1 on the padded raster, convolution weights split for CTA pairs

@@ -49,6 +49,7 @@ class Engine:
         self.ended = torch.zeros(games, dtype=torch.uint8, device=dev)
         self.rewards = torch.zeros(games, 8, dtype=torch.int8, device=dev)
         self.keys = None
+        self._pit_open = False
 
     def close(self):
         if getattr(self, "h", None):
@@ -285,6 +286,65 @@ class Engine:
         tu = self._wrap(self.L.asz_records_turns(self.h), (n,), torch.int32)
         n = self.records_count()
         return pl[:n], va[:n], ids[:n], tu[:n]
+
+    # ---- pit: pit_mp_game_runner.MPGameRunner.run with pit_agent.Agent on both sides, on the device ----------------
+    # A player is a NativeNet, or 0 / 1: the stand-in player valued from that word of the plane key (tests).
+    @staticmethod
+    def _pit_player(p):
+        if isinstance(p, int):
+            return _lib.PitPlayer(None, p)
+        return _lib.PitPlayer(p.h.value, 0)
+
+    def pit_begin(self, alice, bob, alice_snakes):
+        """asz_pit_begin: a match of `alice` (snake ids < alice_snakes) against `bob` on the current root games.  Returns the
+        number of games running."""
+        a, b = self._pit_player(alice), self._pit_player(bob)
+        running = C.c_int32(0)
+        self._pit_open = False
+        check(self.L.asz_pit_begin(self.h, C.byref(a), C.byref(b), int(alice_snakes), C.byref(running), self.stream))
+        self._pit_open = True
+        return running.value
+
+    def pit_turn(self, spawn_cells=None, spawn_mode=SPAWN_NATIVE, moves=None):
+        """asz_pit_turn: one turn; spawn_cells int32 cuda [G] for SPAWN_REPLAY, moves uint8 cuda [G, 8] receives the moves played
+        (255 = none).  Returns the number of games still running."""
+        running = C.c_int32(0)
+        check(self.L.asz_pit_turn(self.h, spawn_mode, _ptr(spawn_cells), _ptr(moves), C.byref(running), self.stream))
+        return running.value
+
+    def _pit_results(self, rc_of, written_on_state):
+        """written_on_state: ASZ_ERR_STATE from this call means 'games still running, results so far written'"""
+        winners = torch.empty(self.G, dtype=torch.int32, device=self.device)
+        decided = torch.empty(self.G, dtype=torch.int32, device=self.device)
+        turns = C.c_int32(0)
+        rc = rc_of(_ptr(winners), _ptr(decided), C.byref(turns))
+        if rc != 0 and not (rc == _lib.ASZ_ERR_STATE and written_on_state):
+            check(rc)                     # nothing was written
+        res = (winners.cpu().numpy(), decided.cpu().numpy(), turns.value)
+        if rc != 0:
+            err = AszError("asz error %d: %s" % (rc, self.L.asz_last_error().decode()))
+            err.partial = res             # (winners, decided_turn, turns) of the games decided so far
+            raise err
+        return res
+
+    def pit_finish(self):
+        """asz_pit_finish -> (winners int32 [G] with -1 = draw, decided_turn int32 [G], turns).  Games still running raise
+        AszError with the results so far in `.partial` (winner -1 and decided_turn -1 for the running games)."""
+        open_match, self._pit_open = self._pit_open, False      # asz_pit_finish closes the match
+        return self._pit_results(lambda w, d, t: self.L.asz_pit_finish(self.h, w, d, t, self.stream), open_match)
+
+    def pit_run(self, alice, bob, alice_snakes, max_turns=0):
+        """asz_pit_run: the whole match with native food spawn, one call; results as pit_finish."""
+        a, b = self._pit_player(alice), self._pit_player(bob)
+        self._pit_open = False            # asz_pit_run abandons a match in progress and closes its own
+        # its ASZ_ERR_STATE comes only from the closing asz_pit_finish: results so far written (begin and turn fail otherwise)
+        return self._pit_results(lambda w, d, t: self.L.asz_pit_run(self.h, C.byref(a), C.byref(b), int(alice_snakes),
+                                                                    int(max_turns), w, d, t, self.stream), True)
+
+    def pit_stats(self):
+        s = np.zeros(4, np.float64)
+        check(self.L.asz_pit_stats(self.h, _np(s)))
+        return dict(turns=int(s[0]), net_rows=int(s[1]), stub_rows=int(s[2]), forward_ms=float(s[3]))
 
     # ---- helpers for the drop-in classes ---------------------------------------------------------------------------
     def alive_mask(self):

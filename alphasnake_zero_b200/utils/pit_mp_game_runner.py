@@ -1,10 +1,13 @@
 """pit MPGameRunner -- mirror of code/utils/pit_mp_game_runner.py:3-63 (two agents, argmax policy, early exit).
-Uses the same fused tic+encode kernel; the planes of all live snakes are produced by one launch per turn."""
+When both agents are pit_agent.Agent over a native AlphaNNet, the whole match runs on the device (asz_pit_*: the planes never
+leave HBM, one host wait per turn); any other agent is driven by the loop below, over the same fused tic+encode kernel."""
 import numpy as np
 import torch
 
 from ..engine import Engine
 from .. import _lib
+from .._lib import AszError
+from . import alpha_nnet, pit_agent
 
 
 class MPGameRunner:
@@ -15,13 +18,69 @@ class MPGameRunner:
         self.engine.reset()
 
     # Alice and Bob are agents using different nets
-    def run(self, Alice, Bob, Alice_snake_cnt=None, spawn_trace=None, move_log=None):
+    def run(self, Alice, Bob, Alice_snake_cnt=None, spawn_trace=None, move_log=None, native=None):
         """pit_mp_game_runner.py:14-63.  Extensions for trace replay (tests): spawn_trace[turn] = int32 [game_cnt] food cell
         spawned in that turn's tic (-1 none) instead of the engine's RNG; move_log (a list) receives per turn a uint8
-        [game_cnt, 8] array of the moves played (255 = no move)."""
-        eng = self.engine
+        [game_cnt, 8] array of the moves played (255 = no move).
+        native=None: the device arena when both agents are pit_agent.Agent over a native AlphaNNet of this board side on this
+        device, the loop otherwise; native=False: the loop; native=True: the arena, or AszError when it cannot be used.
+        Both give the same winners, moves and final game states.  A game that is already finished when the match begins is a
+        draw on the arena (the reference's loop fails on it)."""
         if Alice_snake_cnt is None:
             Alice_snake_cnt = self.snake_cnt // 2
+        if native is not False:
+            nets = self._arena_nets(Alice, Bob)
+            if nets is not None:
+                return self._run_arena(nets, Alice_snake_cnt, spawn_trace, move_log)
+            if native:
+                raise AszError("the device pit needs pit_agent.Agent over a native AlphaNNet for side %d on %s on both sides"
+                               % (self.height, self.engine.device))
+        return self._run_loop(Alice, Bob, Alice_snake_cnt, spawn_trace, move_log)
+
+    def _arena_nets(self, Alice, Bob):
+        """(Alice's NativeNet, Bob's NativeNet) when both agents are exactly pit_agent.Agent over an AlphaNNet whose `v` is
+        the native forward + float32 obstacle mask, for this runner's board side and device; else None"""
+        nets = []
+        for agent in (Alice, Bob):
+            if type(agent) is not pit_agent.Agent or type(agent.nnet) is not alpha_nnet.AlphaNNet:
+                return None
+            nnet = agent.nnet
+            if nnet.backend not in ("auto", "native") or nnet.weights is None or int(nnet.weights["side"]) != self.height:
+                return None
+            dev = nnet.device.index if nnet.device.index is not None else torch.cuda.current_device()
+            if nnet.device.type != "cuda" or dev != self.engine.device.index:
+                return None
+            nets.append(nnet._get_native())
+        return nets
+
+    def _run_arena(self, nets, Alice_snake_cnt, spawn_trace, move_log):
+        eng = self.engine
+        if spawn_trace is None and move_log is None:
+            winners, _, _ = eng.pit_run(nets[0], nets[1], Alice_snake_cnt)
+        else:
+            running = eng.pit_begin(nets[0], nets[1], Alice_snake_cnt)
+            trace = None
+            if spawn_trace is not None:
+                trace = torch.from_numpy(np.ascontiguousarray(np.asarray(spawn_trace, np.int32))).to(eng.device)
+            logs, turn = [], 0
+            while running:
+                if trace is not None and turn >= trace.shape[0]:
+                    eng.pit_finish()          # raises: games are still running, the results so far are attached
+                moves = torch.empty(self.game_cnt, 8, dtype=torch.uint8, device=eng.device) if move_log is not None else None
+                if trace is not None:
+                    running = eng.pit_turn(spawn_cells=trace[turn], spawn_mode=_lib.SPAWN_REPLAY, moves=moves)
+                else:
+                    running = eng.pit_turn(spawn_mode=_lib.SPAWN_NATIVE, moves=moves)
+                if moves is not None:
+                    logs.append(moves)
+                turn += 1
+            winners, _, _ = eng.pit_finish()
+            if move_log is not None:
+                move_log.extend(m.cpu().numpy() for m in logs)
+        return [None if w < 0 else int(w) for w in winners]
+
+    def _run_loop(self, Alice, Bob, Alice_snake_cnt, spawn_trace, move_log):
+        eng = self.engine
         winners = [None] * self.game_cnt
         running = np.ones(self.game_cnt, bool)
         eng.step(tic=False, encode=True)

@@ -289,6 +289,45 @@ int asz_net_forward_pitched(asz_net* net, const float* d_planes, int32_t plane_p
  * that layer's output as float32 [count][2*side-1][2*side-1][128] ([..][1] for layer 8: the fused 1x1 head conv) */
 int asz_net_debug_layer(asz_net* net, const float* d_planes, int32_t count, int32_t layer, float* d_act, void* stream);
 
+/* ---- pit: pit_mp_game_runner.MPGameRunner.run(Alice, Bob, Alice_snake_cnt) (pit_mp_game_runner.py:14-63) with
+ * pit_agent.Agent (pit_agent.py:10-28) on both sides, played on the engine's root games without planes through the host -----
+ * Snakes with id < alice_snakes are Alice's, the others Bob's.  One turn: the rows of the running games are gathered into one
+ * team buffer (Alice's, then Bob's, each in (game, snake) order), each side's network values its segment (one forward when
+ * both sides share a network), AlphaNNet.v's obstacle mask and Agent.argmaxs pick the moves (every other slot plays 1, as in
+ * the loop's np.ones((G, 8))), every unfinished game is stepped (a game decided early keeps being stepped with move 1 for its
+ * live snakes, exactly like the loop), and the referee decides: a game that ended in this tic is won by the lowest snake id
+ * with reward +1 (none = draw); otherwise, when one team has no live snake left, by the lowest live id.  The host waits once
+ * per turn, for (rows of Alice, rows of Bob, games running).
+ * Results: winners[g] = snake id or -1 (draw, or still running), decided_turn[g] = number of tics played when game g was
+ * decided, -1 while it is running.  A game that was already finished when the match begins is decided at turn 0 with winner
+ * -1 (the reference's loop fails on such a game). */
+typedef struct {
+  asz_net* net;          /* the side's value network (same board side and device as the engine), or NULL = stand-in player */
+  int32_t stub_word;     /* net == NULL: value of move a = 16 bits (16a..16a+15) of word stub_word (0 or 1) of the plane key,
+                            mapped to [-1, 1) (asz_search_stub_values uses word 1), then the obstacle mask */
+} asz_pit_player;
+/* starts a match on the current root games (encodes their planes; ASZ_STEP_KEYS when a stand-in plays) and synchronises;
+ * *h_running (may be NULL) = games running.  ASZ_ERR_ARG: a network of another board side or device, alice_snakes outside
+ * 0..S, stub_word not 0/1.  A new begin abandons a match in progress. */
+int asz_pit_begin(asz_engine* e, const asz_pit_player* alice, const asz_pit_player* bob, int32_t alice_snakes, int32_t* h_running,
+                  void* stream);
+/* one turn; spawn_mode ASZ_SPAWN_NATIVE / ASZ_SPAWN_REPLAY (d_spawn_cells [G], entries below -1 read as -1) / ASZ_SPAWN_NONE;
+ * d_moves [G*8] (may be NULL) receives the moves played this turn, 255 = no move; *h_running = games still running.  A turn
+ * when no game is running does nothing.  ASZ_ERR_STATE without a begin. */
+int asz_pit_turn(asz_engine* e, int32_t spawn_mode, const int32_t* d_spawn_cells, uint8_t* d_moves, int32_t* h_running,
+                 void* stream);
+/* ends the match: d_winners [G], d_decided_turn [G] (DEVICE, either may be NULL), *h_turns = turns played.  Synchronous.
+ * Returns ASZ_ERR_STATE, after writing the results, when games are still running. */
+int asz_pit_finish(asz_engine* e, int32_t* d_winners, int32_t* d_decided_turn, int32_t* h_turns, void* stream);
+/* the whole match: begin, native spawn until every game is decided (max_turns 0) or max_turns turns are played, finish
+ * (ASZ_ERR_STATE, only ever with the results so far written, when max_turns ends it with games running).  It abandons a
+ * match in progress, and its own match is closed when it returns, whatever the outcome. */
+int asz_pit_run(asz_engine* e, const asz_pit_player* alice, const asz_pit_player* bob, int32_t alice_snakes, int32_t max_turns,
+                int32_t* d_winners, int32_t* d_decided_turn, int32_t* h_turns, void* stream);
+/* counters of the current or last match: h_stats[4] = turns, rows valued by a network, rows valued by a stand-in player,
+ * milliseconds of the network forwards (CUDA events around each turn's forwards) */
+int asz_pit_stats(asz_engine* e, double* h_stats);
+
 #ifdef __cplusplus
 }
 #endif

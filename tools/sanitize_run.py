@@ -31,7 +31,24 @@ def main():
         st = eng.search_stats()
         assert st["evals"] > 0 and np.isfinite(q.cpu().numpy()).all()
         eng.close()
-        print("side %d ok: %d evals" % (side, st["evals"]))
+        # one pit per board size: the network against a stand-in player (asz_pit_*), stepwise with a replayed trace, then in one call
+        pit = Engine(side=side, snakes=S, health_dec=3, games=48, seed=2)
+        pit.reset()
+        pit.pit_begin(net._native, 0, S // 2)
+        moves = torch.empty(48, 8, dtype=torch.uint8, device="cuda")
+        cells = torch.full((48,), -1, dtype=torch.int32, device="cuda")
+        for _ in range(3):
+            pit.pit_turn(spawn_cells=cells, spawn_mode=_lib.SPAWN_REPLAY, moves=moves)
+        try:
+            pit.pit_finish()
+        except _lib.AszError:
+            pass                                  # games still running after three turns: the results so far are written
+        pit.reset()
+        w, d, turns = pit.pit_run(net._native, 1, S // 2)
+        torch.cuda.synchronize()
+        assert (d >= 1).all() and turns == d.max()
+        print("side %d ok: %d evals, pit of %d turns" % (side, st["evals"], turns))
+        pit.close()
 
 
 if __name__ == "__main__":
