@@ -56,8 +56,6 @@ SYMBOLS = [
     ("asz_env_step_host", C.c_int, [_vp, _u32, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     ("asz_env_submit_host", C.c_int, [_vp, _u32, _i32, _vp, _vp, _vp, _vp, _vp, _vp]),
     ("asz_env_wait_host", C.c_int, [_vp, _i32, _vp]),
-    ("asz_internal_set_hot_word", C.c_int, [_vp, _i32]),
-    ("asz_condition_l2", C.c_int, [_vp, _vp]),
     ("asz_get_totals", C.c_int, [_vp, _vp]),
     ("asz_internal_profile", C.c_int, [_vp, _vp]),
     ("asz_internal_state", C.c_int, [_vp, _vp]),

@@ -98,11 +98,6 @@ __device__ __forceinline__ int warp_excl_scan_i32(int v, int lane) {
 // ---- L2 residency hints ---------------------------------------------------------------------------------------------
 // The game records (21 MB at 65,536 games) are read and rewritten by every launch and fit in L2 many times over; the
 // planes (1 GB per launch) stream through it.  Records are accessed with an evict_last policy, planes with evict_first.
-__device__ __forceinline__ uint64_t l2_policy_evict_normal() {
-  uint64_t pol;
-  asm volatile("createpolicy.fractional.L2::evict_normal.b64 %0, 1.0;" : "=l"(pol));
-  return pol;
-}
 __device__ __forceinline__ uint64_t l2_policy_evict_last() {
   uint64_t pol;
   asm volatile("createpolicy.fractional.L2::evict_last.b64 %0, 1.0;" : "=l"(pol));

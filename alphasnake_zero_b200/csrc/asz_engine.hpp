@@ -43,6 +43,7 @@ struct NvtxRange {
   NvtxRange& operator=(const NvtxRange&) = delete;
 };
 constexpr int kMaxDevices = 64;   // per-device "kernel attributes configured" flags (function attributes are per device)
+constexpr size_t kSchedBytes = 128;   // asz_engine::row_count: the env kernel's two alternating scheduling words, 64 bytes apart
 
 // Device-resident game set: one record per game, structure-of-arrays over games.
 //   cells  [n][PC]  u16 stamps (asz_common.cuh)
@@ -69,13 +70,11 @@ struct asz_engine {
   // env-step scratch owned by the engine
   float* planes = nullptr;        // [G*S][pitch]
   int32_t* row_ids = nullptr;     // [G*S]
-  int32_t* row_count = nullptr;   // 8 MB buffer that holds the kernel's one hot 64-bit word (rows handed out | tickets handed out)
-  size_t sched_off = 0;           // byte offset of that word (tools/env_hot.py moves it around to map the L2 slices' atomic rates)
-  int sched_flip = 0;             // launches alternate between the word at sched_off and the one 64 bytes behind it (asz_env_step)
+  int32_t* row_count = nullptr;   // kSchedBytes: the kernel's 64-bit scheduling words (rows handed out | tickets handed out)
+  int sched_flip = 0;             // launches alternate between the word at byte 0 and the one at byte 64 (asz_env_step)
   // the word of the LAST launch: its low half is that launch's row count
-  int32_t* rows_ptr() const { return reinterpret_cast<int32_t*>(reinterpret_cast<char*>(row_count) + sched_off + (sched_flip ? 64 : 0)); }
-  unsigned long long* totals = nullptr;  // [8]
-  int device_hints = 1, host_hints = 0, step_hints = 1;   // L2 policy hints of env_step_kernel (asz_env.cu)
+  int32_t* rows_ptr() const { return reinterpret_cast<int32_t*>(reinterpret_cast<char*>(row_count) + (sched_flip ? 64 : 0)); }
+  unsigned long long* totals = nullptr;  // [32]: [0..15] totals (asz_get_totals), [16..23] the profile build's cycle sums
   // asz_env_submit_host / asz_env_wait_host: two steps in flight, the inputs of the next one copied under the kernel of this one
   struct HostPipe {
     bool ready = false;

@@ -5,16 +5,12 @@
 // (asz_game.cuh: warp_tic) and writes the record back -- for both games of its ticket -- then takes the ticket's rows of the
 // batch AND its next ticket with ONE 64-bit atomicAdd, and encodes the plane of every surviving snake (5,292 B each at 11x11)
 // into the network's input batch: the cells are scattered into a staged window in shared memory and the copy engine
-// (cp.async.bulk shared -> global) writes the plane, wall runs from a constant buffer.
-//   pitched rows (the engine's own buffers, asz_plane_pitch): planes start on 32-byte sectors, a game's planes are one
-//     sequence of bulk copies (warp_encode_game_v3b), no per-plane edge handling;
-//   dense rows (a caller's [rows][N][N][3] tensor): warp_encode_v2, three copies per plane + edge floats by single lanes.
+// (cp.async.bulk shared -> global) writes the plane, wall runs from a constant buffer.  Rows are asz_plane_pitch() floats apart:
+// planes start on 32-byte sectors and a game's planes are one sequence of bulk copies (warp_encode_game_v3b).
 // Roofline: HBM write bandwidth (planes are > 95 % of the bytes; SURVEY.md 8(d)).  What the kernel must NOT be bound by is the
 // rate at which one L2 slice serves atomics on one address (2.3 - 3.6 ns each): with one atomic per game that was the
 // bound, and the two values were the "two timing regimes" of rounds 1 and 2 (DESIGN.md 4.1).
 #include <algorithm>
-#include <cstdio>
-#include <cstdlib>
 #include <cstring>
 #include <mutex>
 #include <vector>
@@ -47,9 +43,7 @@ struct EnvParams {
   unsigned long long* sched_next;   // the word the NEXT launch uses: zeroed by this one (the engine alternates between two words, so no
                                     // memset node sits between two launches)
   unsigned long long* prof;   // ASZ_ENV_PROFILE builds only: per-phase cycle sums (tools/env_profile.py)
-  int hints;           // 1: L2 policies (planes evict_first, game records evict_last), 0: default policy everywhere
   int device, n_sm;    // the engine's device and its multiprocessor count (grid size of the persistent kernel)
-  int pitched;         // 1: plane rows are PitchGeo::PITCH floats apart (32-byte aligned rows), 0: dense rows of PLANE floats
   int row_base;        // rows of this launch are written at [row_base, row_base + n) of planes / row_ids / keys (max_rows is absolute)
   int pair_tickets, n_tickets;   // scheduling tickets of the launch (set by EnvLaunch::launch): the first pair_tickets are two games each
 };
@@ -63,29 +57,7 @@ struct EnvParams {
 #define ASZ_PROF(k) do { } while (0)
 #endif
 
-// ---- record load / store ------------------------------------------------------------------------------------------
-template <class G>
-__device__ __forceinline__ void load_board(const uint16_t* __restrict__ gcells, uint16_t* sb, int lane) {
-  if constexpr (G::CPL % 4 == 0) {
-    const uint2* src = reinterpret_cast<const uint2*>(gcells);
-    uint2* dst = reinterpret_cast<uint2*>(sb);
-#pragma unroll
-    for (int q = 0; q < G::CPL / 4; ++q) dst[lane * (G::CPL / 4) + q] = src[lane * (G::CPL / 4) + q];
-  } else {
-    const uint32_t* src = reinterpret_cast<const uint32_t*>(gcells);
-    uint32_t* dst = reinterpret_cast<uint32_t*>(sb);
-#pragma unroll
-    for (int q = 0; q < G::CPL / 2; ++q) dst[lane * (G::CPL / 2) + q] = src[lane * (G::CPL / 2) + q];
-  }
-}
-__device__ __forceinline__ Meta load_meta(const uint32_t* __restrict__ gm, int lane) {
-  const uint32_t v = (lane < 8) ? gm[lane] : 0u;
-  Meta m;
-  m.turn = __shfl_sync(kFull, v, 0); m.episode = __shfl_sync(kFull, v, 1); m.wall = __shfl_sync(kFull, v, 2);
-  m.body = __shfl_sync(kFull, v, 3); m.headc = __shfl_sync(kFull, v, 4); m.starve = __shfl_sync(kFull, v, 5);
-  m.eaten = __shfl_sync(kFull, v, 6); m.flags = __shfl_sync(kFull, v, 7);
-  return m;
-}
+// ---- record store ---------------------------------------------------------------------------------------------------
 __device__ __forceinline__ void store_meta(uint32_t* gm, const Meta& m, int lane) {
   if (lane < 8) {
     const uint32_t v = lane == 0 ? m.turn : lane == 1 ? m.episode : lane == 2 ? m.wall : lane == 3 ? m.body
@@ -97,23 +69,21 @@ __device__ __forceinline__ void store_meta(uint32_t* gm, const Meta& m, int lane
 // ---- the fused step kernel ----------------------------------------------------------------------------------------
 // Persistent: MINB CTAs per SM, every warp loops over games g = warp_global, warp_global + n_warps, ... so that the
 // staging buffers' wall background is written once per warp and bulk stores of one game overlap the tic of the next.
-// HINTS: plane stores carry an evict_first L2 policy and the game records (read and rewritten by every launch, 21 MB at
-// 65,536 games) an evict_last one (ASZ_ENV_HINTS / ASZ_ENV_HINTS_HOST = 0 select the plain instructions for experiments).
+// L2 policies: plane stores carry evict_first and the game records (read and rewritten by every launch, 21 MB at 65,536
+// games) evict_last.
 // ACTS: the caller supplies the actions (p.actions); false = none are read (in-kernel random actions, or no tic at all).
-// PITCHED: the plane rows are PitchGeo::PITCH floats apart (32-byte aligned rows: the engine's own buffers) and a game's planes
-// are emitted by warp_encode_game_v3; false = dense rows of PLANE floats (a caller's tensor), warp_encode_v2 per plane.
-template <int SIDE, bool PITCHED>
+template <int SIDE>
 struct EnvSmem {
   using G = Geo<SIDE>;
-  static constexpr int BG = PITCHED ? PitchGeo<G>::SEAMLEN : EncGeo<G>::BGLEN;          // per-CTA constant wall buffer (floats)
-  static constexpr int WSTAGE = PITCHED ? PitchGeo<G>::WSTAGE : EncGeo<G>::WSTAGE;      // floats per staging buffer
-  static constexpr int LUT_BYTES = PITCHED ? PitchLut<G>::BYTES : 0;                    // index / value tables of warp_encode_game_v3b
+  static constexpr int BG = PitchGeo<G>::SEAMLEN;          // per-CTA constant wall buffer (floats)
+  static constexpr int WSTAGE = PitchGeo<G>::WSTAGE;       // floats per staging buffer
+  static constexpr int LUT_BYTES = PitchLut<G>::BYTES;     // index / value tables of warp_encode_game_v3b
 };
 
-template <int SIDE, int WARPS, int MINB, bool HINTS, bool ACTS, bool PITCHED>
+template <int SIDE, int WARPS, int MINB, bool ACTS>
 __global__ void __launch_bounds__(WARPS * 32, MINB) env_step_kernel(const EnvParams p) {
   using G = Geo<SIDE>;
-  using SM = EnvSmem<SIDE, PITCHED>;
+  using SM = EnvSmem<SIDE>;
   extern __shared__ __align__(16) unsigned char smem_raw[];
   const int warp = (int)(threadIdx.x >> 5), lane = lane_id();
   // smem: [per-CTA wall pattern][per warp: 2 staging buffers][per warp: 2 boards][per-CTA body-value table]
@@ -123,34 +93,27 @@ __global__ void __launch_bounds__(WARPS * 32, MINB) env_step_kernel(const EnvPar
   float* s_lut = reinterpret_cast<float*>(reinterpret_cast<uint16_t*>(s_bg + SM::BG + WARPS * 2 * SM::WSTAGE) + WARPS * 2 * G::PC);
   for (int d = (int)threadIdx.x; d < G::PC + 8; d += WARPS * 32) s_lut[d] = (float)((double)d * 0.02);   // game.py:239, float64 product
   unsigned char* s_plut = reinterpret_cast<unsigned char*>(s_lut + G::PC + 8);
-  if constexpr (PITCHED) fill_pitch_luts<G>(s_plut, (int)threadIdx.x, WARPS * 32);
+  fill_pitch_luts<G>(s_plut, (int)threadIdx.x, WARPS * 32);
   const bool enc = (p.flags & ASZ_STEP_ENCODE) != 0;
   if (enc) {
-    if constexpr (PITCHED) fill_seam_pattern(s_bg, PitchGeo<G>::SEAM_AT, PitchGeo<G>::SEAMLEN, PitchGeo<G>::PITCH, G::PLANE, (int)threadIdx.x, WARPS * 32);
-    else fill_wall_pattern(s_bg, SM::BG, (int)threadIdx.x, WARPS * 32);
+    fill_seam_pattern(s_bg, PitchGeo<G>::SEAM_AT, PitchGeo<G>::SEAMLEN, PitchGeo<G>::PITCH, G::PLANE, (int)threadIdx.x, WARPS * 32);
     fill_wall_pattern(stage0, SM::WSTAGE, lane, 32);
     fill_wall_pattern(stage0 + SM::WSTAGE, SM::WSTAGE, lane, 32);
   }
   __syncthreads();
   if (blockIdx.x == 0 && threadIdx.x == 0) *p.sched_next = 0ull;
-  EncodeCtx<G> ctx;
   EncodeCtxP<G> ctxp;
-  // p.hints (experiments): 1 = both policies, 2 = planes evict_first only, 3 = records evict_last only
   ctxp.cur = stage0; ctxp.oth = stage0 + SM::WSTAGE; ctxp.seam = s_bg;
-  ctxp.policy = HINTS ? (p.hints == 3 ? l2_policy_evict_normal() : l2_policy_evict_first()) : 0ull;
+  ctxp.policy = l2_policy_evict_first();
   ctxp.lin = reinterpret_cast<const int16_t*>(s_plut);
   ctxp.hv = reinterpret_cast<const float*>(s_plut + PitchLut<G>::LIN * 2);
   ctxp.food = ctxp.hv + PitchLut<G>::HV;
   ctxp.cur_rot = ctxp.oth_rot = -1; ctxp.cur_base = ctxp.oth_base = 0;
-  ctx.cur = stage0; ctx.oth = stage0 + SM::WSTAGE; ctx.bg = s_bg; ctx.policy = HINTS ? l2_policy_evict_first() : 0ull;
-#pragma unroll
-  for (int q = 0; q < G::CPL; ++q) { ctx.prev_cur[q] = -1; ctx.prev_oth[q] = -1; }
   __shared__ uint32_t s_wtot[WARPS][12];         // per-warp totals (only lane 0 of the warp touches its row)
   if (lane < 12) s_wtot[warp][lane] = 0u;
 #ifdef ASZ_ENV_PROFILE
   __shared__ unsigned long long s_prof[WARPS][8];
   if (lane < 8) s_prof[warp][lane] = 0ull;
-  ctx.prof_wait = &s_prof[warp][6];
 #endif
   __syncwarp();
 
@@ -174,18 +137,12 @@ __global__ void __launch_bounds__(WARPS * 32, MINB) env_step_kernel(const EnvPar
   __shared__ uint64_t s_stash[WARPS][8];         // game A's snake records between its tic and its encode (game B's stay in registers)
   constexpr bool given_actions = ACTS;
   int pf_slot = 0, act_slot = 0;                 // slot the next prefetch writes / slot of the game being stepped
-  const uint64_t keep = HINTS ? (p.hints == 2 ? l2_policy_evict_normal() : l2_policy_evict_last()) : 0ull;
+  const uint64_t keep = l2_policy_evict_last();
   auto prefetch = [&](int gi) {
     const uint32_t* src = reinterpret_cast<const uint32_t*>(p.cells + (size_t)gi * G::PC);
-    if constexpr (HINTS) {
 #pragma unroll
-      for (int q = 0; q < BW; ++q) pf_board[q] = ld_hint_u32(src + lane * BW + q, keep);
-      if (lane < 8) { pf_snake = ld_hint_u64(p.snakes + (size_t)gi * 8 + lane, keep); pf_meta = ld_hint_u32(p.meta + (size_t)gi * 8 + lane, keep); }
-    } else {
-#pragma unroll
-      for (int q = 0; q < BW; ++q) pf_board[q] = src[lane * BW + q];
-      if (lane < 8) { pf_snake = p.snakes[(size_t)gi * 8 + lane]; pf_meta = p.meta[(size_t)gi * 8 + lane]; }
-    }
+    for (int q = 0; q < BW; ++q) pf_board[q] = ld_hint_u32(src + lane * BW + q, keep);
+    if (lane < 8) { pf_snake = ld_hint_u64(p.snakes + (size_t)gi * 8 + lane, keep); pf_meta = ld_hint_u32(p.meta + (size_t)gi * 8 + lane, keep); }
     if constexpr (given_actions) if (lane == 0) {
       asm volatile("cp.async.ca.shared.global [%0], [%1], 8;\ncp.async.commit_group;" ::"r"((uint32_t)__cvta_generic_to_shared(&s_act[warp][pf_slot][0])),
                    "l"(p.actions + (size_t)gi * 8)
@@ -265,15 +222,11 @@ __global__ void __launch_bounds__(WARPS * 32, MINB) env_step_kernel(const EnvPar
 #pragma unroll
           for (int q = 0; q < BW / 2; ++q) {
             const uint2 v = reinterpret_cast<const uint2*>(src)[lane * (BW / 2) + q];
-            if constexpr (HINTS) st_hint_v2u32(gc + 2 * (lane * (BW / 2) + q), v.x, v.y, keep);
-            else reinterpret_cast<uint2*>(gc)[lane * (BW / 2) + q] = v;
+            st_hint_v2u32(gc + 2 * (lane * (BW / 2) + q), v.x, v.y, keep);
           }
         } else {
 #pragma unroll
-          for (int q = 0; q < BW; ++q) {
-            if constexpr (HINTS) st_hint_u32(gc + lane * BW + q, src[lane * BW + q], keep);
-            else gc[lane * BW + q] = src[lane * BW + q];
-          }
+          for (int q = 0; q < BW; ++q) st_hint_u32(gc + lane * BW + q, src[lane * BW + q], keep);
         }
       }
       if (lane < 8) {
@@ -281,13 +234,8 @@ __global__ void __launch_bounds__(WARPS * 32, MINB) env_step_kernel(const EnvPar
                           : lane == 4 ? m.headc : lane == 5 ? m.starve : lane == 6 ? m.eaten : m.flags;
         const uint64_t rec = pack_snake(sn);
         if (stash != nullptr) stash[lane] = rec;
-        if constexpr (HINTS) {
-          st_hint_u64(p.snakes + (size_t)g * 8 + lane, rec, keep);
-          st_hint_u32(p.meta + (size_t)g * 8 + lane, mv, keep);
-        } else {
-          p.snakes[(size_t)g * 8 + lane] = rec;
-          p.meta[(size_t)g * 8 + lane] = mv;
-        }
+        st_hint_u64(p.snakes + (size_t)g * 8 + lane, rec, keep);
+        st_hint_u32(p.meta + (size_t)g * 8 + lane, mv, keep);
       }
     } else {
       if (p.flags & ASZ_STEP_TIC) {     // a finished game is not stepped: its results of this tic are "nothing happened"
@@ -298,40 +246,17 @@ __global__ void __launch_bounds__(WARPS * 32, MINB) env_step_kernel(const EnvPar
       rows_and_ticket();
     }
   };
-  // planes of one game into rows [row, row + n_rows) (rows of a game stay contiguous, ascending snake id)
+  // planes of one game into rows [row, row + n_rows) (rows of a game stay contiguous, ascending snake id); rows at or past
+  // p.max_rows are not written
   auto encode_game = [&](int g, const uint16_t* board, const Snake& sn, unsigned live_mask, int n_rows, int row) {
     if (n_rows <= 0) return;
     CellView<G> cv;
     warp_cell_view<G>(board, sn, cv, s_lut);
-    unsigned rest = live_mask;
-    if constexpr (PITCHED) {
-      rest = 0u;
-      const int n_emit = min(n_rows, p.max_rows - row);
-      if (n_emit > 0) {
-        float* gbase = p.planes + (size_t)row * PitchGeo<G>::PITCH;
-#ifdef ASZ_ENC_V3A       // A/B: the first pitched encode (per-lane restore bookkeeping, select chains, float64 products per plane)
-        if (p.flags & ASZ_STEP_KEYS) warp_encode_game_v3<G, true, HINTS>(cv, sn, live_mask, n_emit, ctx, gbase, p.keys + 2 * (size_t)row, p.row_ids + row, g * 8);
-        else warp_encode_game_v3<G, false, HINTS>(cv, sn, live_mask, n_emit, ctx, gbase, nullptr, p.row_ids + row, g * 8);
-#else
-        if (p.flags & ASZ_STEP_KEYS) warp_encode_game_v3b<G, true, HINTS>(cv, sn, live_mask, n_emit, ctxp, gbase, p.keys + 2 * (size_t)row, p.row_ids + row, g * 8);
-        else warp_encode_game_v3b<G, false, HINTS>(cv, sn, live_mask, n_emit, ctxp, gbase, nullptr, p.row_ids + row, g * 8);
-#endif
-      }
-    }
-    while (rest) {
-      const int vs = __ffs(rest) - 1;
-      rest &= rest - 1;
-      if (row < p.max_rows) {
-        uint64_t k0 = 0, k1 = 0;
-        if (p.flags & ASZ_STEP_KEYS) {
-          warp_encode_v2<G, true, HINTS>(cv, sn, vs, ctx, p.planes, (size_t)row * G::PLANE, &k0, &k1);
-          if (lane == 0) { p.keys[2 * (size_t)row] = k0; p.keys[2 * (size_t)row + 1] = k1; }
-        } else {
-          warp_encode_v2<G, false, HINTS>(cv, sn, vs, ctx, p.planes, (size_t)row * G::PLANE, nullptr, nullptr);
-        }
-        if (lane == 0) p.row_ids[row] = g * 8 + vs;
-      }
-      ++row;
+    const int n_emit = min(n_rows, p.max_rows - row);
+    if (n_emit > 0) {
+      float* gbase = p.planes + (size_t)row * PitchGeo<G>::PITCH;
+      if (p.flags & ASZ_STEP_KEYS) warp_encode_game_v3b<G, true>(cv, sn, live_mask, n_emit, ctxp, gbase, p.keys + 2 * (size_t)row, p.row_ids + row, g * 8);
+      else warp_encode_game_v3b<G, false>(cv, sn, live_mask, n_emit, ctxp, gbase, nullptr, p.row_ids + row, g * 8);
     }
   };
 
@@ -379,7 +304,7 @@ __global__ void __launch_bounds__(WARPS * 32, MINB) env_step_kernel(const EnvPar
       encode_game(gA + h, sb + h * G::PC, sn, h ? maskB : maskA, h ? nB : nA, (h + 1 < cnt) ? row + nB : row);
     }
     __syncwarp();   // the board buffers are reused by the next ticket
-    ASZ_PROF(5);   // plane encode (ASZ_PROF 6 inside: waiting for the copy engine to release a staging buffer)
+    ASZ_PROF(5);   // plane encode
     t = nxt;
   }
   if (lane == 0) {
@@ -410,82 +335,44 @@ __global__ void __launch_bounds__(WARPS * 32) env_reset_kernel(uint16_t* cells, 
   store_meta(meta + (size_t)g * 8, m, lane);
 }
 
-// ---- L2 read sweep (experiments) --------------------------------------------------------------------------------------
-// Reads ~1.25 GB, which leaves the L2 full of clean lines.  With one atomic per game the state of the L2 decided how fast the
-// slice of the kernel's hot word served its atomics (tools/env_hot.py reproduces the scan); the ticket kernel does not care.
-__global__ void __launch_bounds__(256) l2_sweep_kernel(const uint4* __restrict__ p, size_t n, int passes, unsigned long long* sink) {
-  unsigned long long acc = 0;
-  const size_t stride = (size_t)gridDim.x * blockDim.x;
-  for (int k = 0; k < passes; ++k)
-    for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) {
-      uint4 v;
-      asm volatile("ld.global.v4.u32 {%0, %1, %2, %3}, [%4];" : "=r"(v.x), "=r"(v.y), "=r"(v.z), "=r"(v.w) : "l"(p + i));   // volatile asm: every pass loads
-      acc += v.x ^ v.y ^ v.z ^ v.w;
-    }
-  if (acc == 0x9E3779B97F4A7C15ull) *sink = acc;     // never true in practice; keeps the loads alive
-}
-
 template <int SIDE>
 struct EnvLaunch {
-#ifndef ASZ_ENV_WARPS       // occupancy experiments (tools/env_profile.py build-variant NAME -DASZ_ENV_WARPS=.. -DASZ_ENV_MINB=..)
-#define ASZ_ENV_WARPS 8
-#endif
-#ifndef ASZ_ENV_MINB
-#define ASZ_ENV_MINB 3
-#endif
-  static constexpr int WARPS = (SIDE >= 19) ? 4 : ASZ_ENV_WARPS;
+  // 3 CTAs x 8 warps per SM at 80 registers (2 x 4 at 19x19).  Measured alternatives at 11x11 (tools/env_sustain.py, us per
+  // launch of 65,536 games): 8 warps x 3 CTAs 176.8 | 12 x 2 176.8 | 10 x 2 177.3 | 8 x 2 196.2 (too few warps) |
+  // 7 x 4 206.6, 5 x 5 211.1, 6 x 5 227.2, 8 x 4 233 (register spills)
+  static constexpr int WARPS = SIDE >= 19 ? 4 : 8;
+  static constexpr int MINB = SIDE >= 19 ? 2 : 3;
+  // the last kTailRounds games of every warp are handed out one by one, everything before in pairs (2: +2.5 us, 4 and 6: the
+  // same as 3)
+  static constexpr int kTailRounds = 3;
   using G = Geo<SIDE>;
-  template <bool PITCHED>
-  static size_t smem_bytes() {
-    using SM = EnvSmem<SIDE, PITCHED>;
-    return (size_t)(SM::BG + WARPS * 2 * SM::WSTAGE) * sizeof(float) + (size_t)WARPS * 2 * G::PC * sizeof(uint16_t) +
-           (size_t)(G::PC + 8) * sizeof(float) + (size_t)SM::LUT_BYTES;
-  }
-  template <int MINB, bool HINTS, bool ACTS, bool PITCHED>
+  using SM = EnvSmem<SIDE>;
+  static constexpr size_t kSmemBytes = (size_t)(SM::BG + WARPS * 2 * SM::WSTAGE) * sizeof(float) + (size_t)WARPS * 2 * G::PC * sizeof(uint16_t) +
+                                       (size_t)(G::PC + 8) * sizeof(float) + (size_t)SM::LUT_BYTES;
+  template <bool ACTS>
   static int launch(const EnvParams& p, cudaStream_t st) {
     // function attributes are per device: one flag per device and kernel instantiation (the caller holds a DeviceGuard)
     static bool configured[kMaxDevices] = {false};
     const int dev = p.device;
     if (dev < 0 || dev >= kMaxDevices || !configured[dev]) {
-      if (!cuda_ok(cudaFuncSetAttribute(env_step_kernel<SIDE, WARPS, MINB, HINTS, ACTS, PITCHED>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                        (int)smem_bytes<PITCHED>()), "cudaFuncSetAttribute(env_step_kernel)"))
+      if (!cuda_ok(cudaFuncSetAttribute(env_step_kernel<SIDE, WARPS, MINB, ACTS>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                        (int)kSmemBytes), "cudaFuncSetAttribute(env_step_kernel)"))
         return ASZ_ERR_CUDA;
-      if (!cuda_ok(cudaFuncSetAttribute(env_step_kernel<SIDE, WARPS, MINB, HINTS, ACTS, PITCHED>, cudaFuncAttributePreferredSharedMemoryCarveout,
+      if (!cuda_ok(cudaFuncSetAttribute(env_step_kernel<SIDE, WARPS, MINB, ACTS>, cudaFuncAttributePreferredSharedMemoryCarveout,
                                         cudaSharedmemCarveoutMaxShared), "cudaFuncSetAttribute(carveout)"))
         return ASZ_ERR_CUDA;
       if (dev >= 0 && dev < kMaxDevices) configured[dev] = true;
-      if (getenv("ASZ_DEBUG_OCC")) {   // experiments: CTAs the runtime expects to keep resident per SM with this shared-memory size
-        int nb = -1;
-        cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, env_step_kernel<SIDE, WARPS, MINB, HINTS, ACTS, PITCHED>, WARPS * 32, smem_bytes<PITCHED>());
-        cudaFuncAttributes fa;
-        cudaFuncGetAttributes(&fa, env_step_kernel<SIDE, WARPS, MINB, HINTS, ACTS, PITCHED>);
-        fprintf(stderr, "[asz] env_step_kernel<%d,%d,%d,%d,%d,%d>: %d CTAs/SM expected, %zu B dynamic + %zu B static smem, %d regs, carveout pref %d\n",
-                SIDE, WARPS, MINB, (int)HINTS, (int)ACTS, (int)PITCHED, nb, smem_bytes<PITCHED>(), fa.sharedSizeBytes, fa.numRegs,
-                fa.preferredShmemCarveout);
-      }
     }
     const int blocks = std::min((p.G + WARPS - 1) / WARPS, p.n_sm * MINB);
-    // the last `rounds` games of every warp are handed out one by one, everything before in pairs
-    static int rounds = -1;
-    if (rounds < 0) { const char* v = getenv("ASZ_ENV_TAIL_ROUNDS"); rounds = v ? std::max(0, atoi(v)) : 3; }   // 2: +2.5 us, 4 and 6: the same as 3
     EnvParams q = p;
-    q.pair_tickets = std::max(0, p.G - rounds * blocks * WARPS) / 2;
+    q.pair_tickets = std::max(0, p.G - kTailRounds * blocks * WARPS) / 2;
     q.n_tickets = p.G - q.pair_tickets;
-    env_step_kernel<SIDE, WARPS, MINB, HINTS, ACTS, PITCHED><<<blocks, WARPS * 32, smem_bytes<PITCHED>(), st>>>(q);
+    env_step_kernel<SIDE, WARPS, MINB, ACTS><<<blocks, WARPS * 32, kSmemBytes, st>>>(q);
     return cuda_ok(cudaGetLastError(), "env_step_kernel launch") ? ASZ_OK : ASZ_ERR_CUDA;
   }
   static int step(const EnvParams& p, cudaStream_t st) {
-    // 3 CTAs x 8 warps per SM at 80 registers (2 x 4 at 19x19).  Measured alternatives at 11x11 (tools/env_sustain.py, us per
-    // launch of 65,536 games): 8 warps x 3 CTAs 176.8 | 12 x 2 176.8 | 10 x 2 177.3 | 8 x 2 196.2 (too few warps) |
-    // 7 x 4 206.6, 5 x 5 211.1, 6 x 5 227.2, 8 x 4 233 (register spills)
-    constexpr int MINB = SIDE >= 19 ? 2 : ASZ_ENV_MINB;
     const bool acts = (p.flags & ASZ_STEP_TIC) && !(p.flags & ASZ_STEP_RANDOM_ACT);
-    if (p.pitched) {
-      if (p.hints) return acts ? launch<MINB, true, true, true>(p, st) : launch<MINB, true, false, true>(p, st);
-      return acts ? launch<MINB, false, true, true>(p, st) : launch<MINB, false, false, true>(p, st);
-    }
-    if (p.hints) return acts ? launch<MINB, true, true, false>(p, st) : launch<MINB, true, false, false>(p, st);
-    return acts ? launch<MINB, false, true, false>(p, st) : launch<MINB, false, false, false>(p, st);
+    return acts ? launch<true>(p, st) : launch<false>(p, st);
   }
   static int reset(const GameSet& gs, int S, uint64_t seed, cudaStream_t st) {
     const int blocks = (gs.n + WARPS - 1) / WARPS;
@@ -511,11 +398,6 @@ void gameset_free(GameSet& gs) {
 
 static int pc_of(int side) { return side == 7 ? Geo<7>::PC : side == 11 ? Geo<11>::PC : Geo<19>::PC; }
 
-// k-th candidate address (byte offset in the 8 MB counter buffer) of the kernel's hot word: other address bits 7..22 every time
-static size_t hot_word_offset(int k) {
-  return ((size_t)k * 4096 + (size_t)(k % 29) * 128 + (size_t)(k % 3) * ((size_t)1 << 21)) % (((size_t)8 << 20) - 128);
-}
-
 }  // namespace asz
 
 using namespace asz;
@@ -528,9 +410,6 @@ int asz_version(void) { return ASZ_VERSION; }
 // allocations of asz_engine_create; on failure the caller destroys the partially built engine (cudaFree(nullptr) is a no-op)
 static int engine_alloc(asz_engine* e, const asz_config* cfg) {
   e->cfg = *cfg;
-  { const char* v = getenv("ASZ_ENV_HINTS"); e->device_hints = v ? atoi(v) : 1; }            // experiments only
-  { const char* v = getenv("ASZ_ENV_HINTS_HOST"); e->host_hints = v ? atoi(v) : 1; }
-  e->step_hints = e->device_hints;
   ASZ_CUDA(cudaGetDevice(&e->device));
   ASZ_CUDA(cudaDeviceGetAttribute(&e->n_sm, cudaDevAttrMultiProcessorCount, e->device));
   e->pc = pc_of(cfg->side);
@@ -544,9 +423,9 @@ static int engine_alloc(asz_engine* e, const asz_config* cfg) {
   if (rc != ASZ_OK) return rc;
   ASZ_CUDA(cudaMalloc(&e->planes, rows * (size_t)e->pitch * sizeof(float) + 32));
   ASZ_CUDA(cudaMalloc(&e->row_ids, rows * sizeof(int32_t)));
-  // the kernel's scheduling word (low half: rows of the step, high half: tickets handed out) and its alternate; the rest is padding
-  ASZ_CUDA(cudaMalloc(&e->row_count, (size_t)8 << 20));
-  ASZ_CUDA(cudaMemset(e->row_count, 0, (size_t)8 << 20));            // every candidate pair of scheduling words starts at zero
+  // the kernel's scheduling word (low half: rows of the step, high half: tickets handed out) and its alternate, 64 bytes apart
+  ASZ_CUDA(cudaMalloc(&e->row_count, kSchedBytes));
+  ASZ_CUDA(cudaMemset(e->row_count, 0, kSchedBytes));
   ASZ_CUDA(cudaMalloc(&e->totals, 32 * sizeof(unsigned long long)));   // [0..15] totals, [16..23] profile build's cycle sums
   ASZ_CUDA(cudaMemset(e->totals, 0, 32 * sizeof(unsigned long long)));
   if (cfg->max_breadth > 0) {
@@ -609,7 +488,13 @@ int asz_env_step(asz_engine* e, const asz_step_args* a, void* stream) {
   if ((a->flags & ASZ_STEP_ENCODE) && (!a->d_planes || !a->d_row_ids || !a->d_row_count || a->max_rows <= 0)) {
     set_error("ASZ_STEP_ENCODE needs d_planes, d_row_ids, d_row_count and max_rows"); return ASZ_ERR_ARG;
   }
-  if ((a->flags & ASZ_STEP_ENCODE) && ((uintptr_t)a->d_planes & (uintptr_t)(4 * kEncGran - 1))) { set_error("d_planes must be 32-byte aligned"); return ASZ_ERR_ARG; }
+  if ((a->flags & ASZ_STEP_ENCODE) && ((uintptr_t)a->d_planes & 31u)) { set_error("d_planes must be 32-byte aligned"); return ASZ_ERR_ARG; }
+  // the encode writes whole rows of plane_pitch floats (pad included): a buffer sized for rows of any other length would be
+  // written past its end
+  if ((a->flags & ASZ_STEP_ENCODE) && a->plane_pitch != e->pitch) {
+    set_error("plane_pitch is " + std::to_string(a->plane_pitch) + ": it must equal asz_plane_pitch() = " + std::to_string(e->pitch));
+    return ASZ_ERR_ARG;
+  }
   if ((a->flags & ASZ_STEP_KEYS) && !a->d_keys) { set_error("ASZ_STEP_KEYS needs d_keys"); return ASZ_ERR_ARG; }
   if ((a->flags & ASZ_STEP_TIC) && !(a->flags & ASZ_STEP_RANDOM_ACT) && !a->d_actions) { set_error("d_actions is null"); return ASZ_ERR_ARG; }
   if ((a->flags & ASZ_STEP_TIC) && !(a->flags & ASZ_STEP_RANDOM_ACT) && ((uintptr_t)a->d_actions & 7u)) { set_error("d_actions must be 8-byte aligned"); return ASZ_ERR_ARG; }
@@ -626,23 +511,18 @@ int asz_env_step(asz_engine* e, const asz_step_args* a, void* stream) {
   p.actions = a->d_actions; p.spawn_cells = a->d_spawn_cells;
   if (a->row_base < 0 || ((a->flags & ASZ_STEP_ENCODE) && a->row_base > a->max_rows)) { set_error("row_base out of range"); return ASZ_ERR_ARG; }
   p.planes = a->d_planes; p.row_ids = a->d_row_ids; p.keys = a->d_keys; p.max_rows = a->max_rows; p.row_base = a->row_base;
-  if (a->plane_pitch != 0 && a->plane_pitch != e->plane && a->plane_pitch != e->pitch) {
-    set_error("plane_pitch must be 0 (dense rows) or asz_plane_pitch()"); return ASZ_ERR_ARG;
-  }
-  p.pitched = (a->plane_pitch == e->pitch && e->pitch != e->plane) ? 1 : 0;
   // Rows are always counted in the engine's own scheduling word and copied to the caller's d_row_count after the launch.  The
   // engine alternates between two words: this launch uses the one the previous launch zeroed and zeroes the other one (whose row
   // count every stream-ordered reader of the previous launch has consumed by the time this kernel runs), so there is no memset
   // node between two launches.
   const bool own_count = a->d_row_count != nullptr && reinterpret_cast<const char*>(a->d_row_count) >= reinterpret_cast<const char*>(e->row_count) &&
-                         reinterpret_cast<const char*>(a->d_row_count) < reinterpret_cast<const char*>(e->row_count) + ((size_t)8 << 20);
+                         reinterpret_cast<const char*>(a->d_row_count) < reinterpret_cast<const char*>(e->row_count) + kSchedBytes;
   const int flip = e->sched_flip ^ 1;                                // committed when the launch has been enqueued
-  char* const pair = reinterpret_cast<char*>(e->row_count) + e->sched_off;
+  char* const pair = reinterpret_cast<char*>(e->row_count);
   p.sched = reinterpret_cast<unsigned long long*>(pair + (flip ? 64 : 0));       // low word = the row count the callers read
   p.sched_next = reinterpret_cast<unsigned long long*>(pair + (flip ? 0 : 64));
   p.row_count = reinterpret_cast<int32_t*>(p.sched);
   p.ended = a->d_ended; p.rewards = a->d_rewards; p.totals = e->totals; p.prof = e->totals + 16;
-  p.hints = e->step_hints;
   int rc;
   switch (e->cfg.side) {
     case 7: rc = EnvLaunch<7>::step(p, st); break;
@@ -742,17 +622,13 @@ static int host_submit(asz_engine* e, uint32_t flags, int32_t spawn_mode, const 
   a.d_planes = e->planes; a.d_row_ids = e->row_ids; a.max_rows = (int32_t)(G * (size_t)e->cfg.snakes); a.plane_pitch = e->pitch;
   a.d_row_count = e->rows_ptr(); a.d_ended = hp.d_ended[slot]; a.d_rewards = hp.d_rewards[slot];
   // Result buffers in pinned (page-locked, UVA-mapped) host memory can be written by the kernel itself, one posted PCIe write
-  // per game while the launch runs, instead of by two device->host copies after it (ASZ_HOST_ZEROCOPY=0 disables).
-  static int zero_copy = -1;
-  if (zero_copy < 0) { const char* v = getenv("ASZ_HOST_ZEROCOPY"); zero_copy = v ? atoi(v) : 1; }
+  // per game while the launch runs, instead of by two device->host copies after it.
   bool zc_ended = false, zc_rewards = false;
-  if (!results_by_copy && zero_copy && (flags & ASZ_STEP_TIC)) {
+  if (!results_by_copy && (flags & ASZ_STEP_TIC)) {
     if (void* d = pinned_alias(h_ended)) { a.d_ended = static_cast<uint8_t*>(d); zc_ended = true; }
     if (void* d = pinned_alias(h_rewards)) { a.d_rewards = static_cast<int8_t*>(d); zc_rewards = true; }
   }
-  e->step_hints = e->host_hints;
   const int rc = asz_env_step(e, &a, stream);
-  e->step_hints = e->device_hints;
   if (rc != ASZ_OK) return rc;
   if (results_by_copy) {
     // the row count leaves the hot word before the next launch zeroes it; everything else waits for the kernel on the out stream
@@ -814,18 +690,6 @@ int asz_env_step_host(asz_engine* e, uint32_t flags, int32_t spawn_mode, const u
   return ASZ_OK;
 }
 
-int asz_condition_l2(asz_engine* e, void* stream) {
-  if (!e) { set_error("null engine"); return ASZ_ERR_ARG; }
-  DeviceGuard guard(e->device);
-  const size_t bytes = (size_t)e->cfg.games * e->cfg.snakes * e->pitch * sizeof(float);
-  if (bytes < ((size_t)192 << 20)) return ASZ_OK;      // a batch that fits the L2 does not stream through it: nothing to condition
-  const size_t want = (size_t)5 << 28;                 // 1.25 GB of read traffic (8x the L2 is what the experiments needed)
-  const int passes = (int)((want + bytes - 1) / bytes);
-  l2_sweep_kernel<<<e->n_sm * 8, 256, 0, (cudaStream_t)stream>>>(reinterpret_cast<const uint4*>(e->planes), bytes / 16, passes, e->totals + 31);
-  if (!cuda_ok(cudaGetLastError(), "l2_sweep_kernel")) return ASZ_ERR_CUDA;
-  return ASZ_OK;
-}
-
 int asz_get_totals(asz_engine* e, uint64_t* h_totals) {
   if (!e || !h_totals) { set_error("null argument"); return ASZ_ERR_ARG; }
   DeviceGuard guard(e->device);
@@ -843,16 +707,6 @@ int asz_internal_profile(asz_engine* e, uint64_t* h_cycles) {
   return ASZ_OK;
 }
 
-// experiments (tools/env_hot.py): put the kernel's hot word at candidate address k and keep it there
-int asz_internal_set_hot_word(asz_engine* e, int32_t k) {
-  if (!e || k < 0) { set_error("bad argument"); return ASZ_ERR_ARG; }
-  DeviceGuard guard(e->device);
-  ASZ_CUDA(cudaDeviceSynchronize());
-  e->sched_off = hot_word_offset(k);
-  e->sched_flip = 0;
-  ASZ_CUDA(cudaMemset(reinterpret_cast<char*>(e->row_count) + e->sched_off, 0, 128));   // both words of the pair start at zero
-  return ASZ_OK;
-}
 int asz_internal_state(asz_engine* e, void** d_ptrs) {
   if (!e || !d_ptrs) { set_error("null argument"); return ASZ_ERR_ARG; }
   d_ptrs[0] = e->root.cells; d_ptrs[1] = e->root.snakes; d_ptrs[2] = e->root.meta;

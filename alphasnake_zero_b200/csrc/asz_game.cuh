@@ -346,41 +346,19 @@ __device__ __forceinline__ void warp_encode(const CellView<G>& cv, const Snake& 
   }
 }
 
-
-// ---- plane encode, v2: window staging + bulk async stores --------------------------------------------------------
-// A plane is 21x21x3 floats of which only the 11 rows that intersect the board window are not pure wall background.
-// Those rows (one contiguous element range [W0, W1) of the plane) are staged in a per-warp buffer whose background is
-// written once per kernel (stage[s] = 1 iff s % 3 == 1); per plane the warp scatters its board cells into it, hands the
-// plane to the bulk-copy engine as three cp.async.bulk shared->global stores (wall before the window from a per-CTA
-// constant buffer, the window, wall after) and later restores the touched pixels.  The staging offset `off` makes the
-// shared and global addresses agree modulo 16 bytes (planes are only 4-byte aligned: 1323 floats) and modulo the 3-float
-// pixel pattern.  Compared with v1 the warp no longer fills and copies the whole plane with LSU instructions.
-// kEncGran: every bulk copy starts and ends on a multiple of this many floats of the OUTPUT address (4 = 16 bytes, the
-// copy engine's minimum; 8 = whole 32-byte sectors, so that no L2 sector is assembled from two different copies; must be
-// <= 16 because one lane stores one edge float).  Measured per launch of 65,536 games: 4: 176.8 us, 8: 175.3 us, 32 (whole
-// lines, with an edge loop): 191.8 us.
-constexpr int kEncGran = 8;
-template <class G>
-struct EncGeo {
-  static constexpr int WIN = G::SIDE * 3 * G::N;                       // floats of the window rows (693 at 11x11)
-  static constexpr int LEAD = kEncGran == 4 ? 12 : 24;                 // wall floats before the window (>= max staging offset)
-  static constexpr int WSTAGE = ((LEAD + WIN + kEncGran + 3) / 4) * 4; // staging floats per buffer
-  static constexpr int BGLEN = ((8 + (G::N - G::SIDE) * 3 * G::N + 2 * kEncGran + 3) / 4) * 4;   // per-CTA wall pattern
-};
-
-template <class G>
-struct EncodeCtx {
-  float* cur;            // staging buffer of the next plane
-  float* oth;            // the other buffer (its bulk store may still be in flight)
-  const float* bg;
-  uint64_t policy;       // L2 cache policy of the plane stores
-#ifdef ASZ_ENV_PROFILE
-  unsigned long long* prof_wait;
-#endif
-  int prev_cur[G::CPL];  // stage index of the pixel each of this lane's cells was scattered to in `cur` (-1 none)
-  int prev_oth[G::CPL];
-};
-
+// ---- plane encode of the env kernel: pitched rows, one emission per game -------------------------------------------
+// A plane at 11x11 is 21x21x3 floats of which only the 11 rows that intersect the board window are not pure wall background.  Those
+// rows (one contiguous element range [W0, W0 + WIN) of the plane) are staged in a per-warp buffer whose background is written
+// once per kernel (stage[s] = 1 iff s % 3 == 1); per plane the warp scatters its board cells into it, hands it to the bulk-copy
+// engine (cp.async.bulk shared -> global) and later restores the touched pixels.  Two staging buffers per warp alternate, so the
+// scatter of one plane overlaps the copy of the previous one.
+// The engine's plane buffers (the network's input batch, the record store) keep consecutive planes PITCH floats apart,
+// PITCH = PLANE rounded up to 8 floats (5,312 B instead of 5,292 B at 11x11): every plane starts on a 32-byte sector of HBM,
+// every copy starts and ends on one, and no sector is assembled from two different copies.  The planes of one game are
+// consecutive rows, so the game is emitted as ONE sequence of bulk copies: wall before the first window, then per plane its
+// window (from the staging buffer) and the wall run up to the next window -- the wall after plane k and the wall before plane
+// k+1 are one contiguous range, copied from a per-CTA constant "seam" buffer that holds a plane end, the pad floats and a plane
+// start.
 __device__ __forceinline__ void fill_wall_pattern(float* dst, int n_floats, int tid, int nthreads) {
   for (int q4 = tid; q4 < n_floats / 4; q4 += nthreads) {
     const int r = q4 % 3;   // element 4*q4 has phase (4*q4) % 3 == q4 % 3
@@ -396,129 +374,16 @@ __device__ __forceinline__ uint64_t l2_policy_evict_first() {
   asm volatile("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(pol));
   return pol;
 }
-template <bool kHint>
 __device__ __forceinline__ void bulk_s2g(float* gdst, const float* ssrc, uint32_t bytes, uint64_t policy) {
-  if constexpr (kHint) {
-    asm volatile("cp.async.bulk.global.shared::cta.bulk_group.L2::cache_hint [%0], [%1], %2, %3;" ::"l"(gdst),
-                 "r"((uint32_t)__cvta_generic_to_shared(ssrc)), "r"(bytes), "l"(policy)
-                 : "memory");
-  } else {
-    asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;" ::"l"(gdst),
-                 "r"((uint32_t)__cvta_generic_to_shared(ssrc)), "r"(bytes)
-                 : "memory");
-  }
+  asm volatile("cp.async.bulk.global.shared::cta.bulk_group.L2::cache_hint [%0], [%1], %2, %3;" ::"l"(gdst),
+               "r"((uint32_t)__cvta_generic_to_shared(ssrc)), "r"(bytes), "l"(policy)
+               : "memory");
 }
 __device__ __forceinline__ void bulk_commit() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
 template <int N>
 __device__ __forceinline__ void bulk_wait_read() { asm volatile("cp.async.bulk.wait_group.read %0;" ::"n"(N) : "memory"); }
 __device__ __forceinline__ void fence_proxy_async_smem() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
 
-template <class G, bool kWantKey, bool kHint = false>
-__device__ __forceinline__ void warp_encode_v2(const CellView<G>& cv, const Snake& sn, int vs, EncodeCtx<G>& ctx, float* out,
-                                               size_t gidx0, uint64_t* key0, uint64_t* key1) {
-  constexpr int SIDE = G::SIDE, CPL = G::CPL, CELLS = G::CELLS, N = G::N, PLANE = G::PLANE;
-  using E = EncGeo<G>;
-  const int lane = lane_id();
-  const int vhead = __shfl_sync(kFull, sn.head, vs);
-  const int vlen = __shfl_sync(kFull, sn.len, vs);
-  const int vhp = __shfl_sync(kFull, sn.health, vs);
-  const int vrot = __shfl_sync(kFull, sn.last, vs);
-  const int hy = vhead / SIDE, hx = vhead - hy * SIDE;
-  const float my_hv = (float)(((double)sn.len - ((double)vlen - 0.5)) * 0.04);
-  const float foodv = (float)((double)(101 - vhp) * 0.01);
-  // Recentring (game.py:249-251) and numpy.rot90 (game.py:257) are one affine map of the cell (y, x) to the output
-  // pixel p = i*N + j:  p = A*y + B*x + C with warp-uniform A, B, C; i0 = first output row of the board window.
-  int A, B, Cc, i0;
-  if (vrot == 0)      { A = N;  B = 1;  Cc = (SIDE - 1 - hy) * N + (SIDE - 1 - hx);             i0 = SIDE - 1 - hy; }
-  else if (vrot == 1) { A = 1;  B = -N; Cc = (N - SIDE + hx) * N + (SIDE - 1 - hy);             i0 = hx; }
-  else if (vrot == 2) { A = -N; B = -1; Cc = (N - SIDE + hy) * N + (N - SIDE + hx);             i0 = hy; }
-  else                { A = -1; B = N;  Cc = (SIDE - 1 - hx) * N + (N - SIDE + hy);             i0 = SIDE - 1 - hx; }
-  const int W0 = i0 * 3 * N, W1 = W0 + E::WIN;
-  constexpr int GR = kEncGran;
-  const int a0 = (int)(gidx0 & (GR - 1));       // misalignment of the plane's first float, in floats past a GR boundary
-  const int a = (a0 + W0) & (GR - 1);           // same for the window's first float
-  int off = (9 * (a & 3)) % 12;                 // staging offset of the window: off % 4 == a % 4 (shared and global
-  while (GR > 4 && off < a) off += 12;          // addresses agree modulo 16 bytes), off % 3 == 0 (pixel phase), off >= a
-  const int base3 = 3 * Cc - W0 + off;          // stage index of pixel p's channel 0 = 3*A*y + 3*B*x + base3
-  float* stage = ctx.cur;
-  // the bulk store that read this buffer two planes ago must have finished reading it
-#ifdef ASZ_ENV_PROFILE
-  const long long prof_w0 = clock64();
-#endif
-  if (lane == 0) bulk_wait_read<1>();
-  __syncwarp();
-#ifdef ASZ_ENV_PROFILE
-  if (ctx.prof_wait != nullptr && lane == 0) *ctx.prof_wait += (unsigned long long)(clock64() - prof_w0);
-#endif
-#pragma unroll
-  for (int q = 0; q < CPL; ++q) {
-    const int s = ctx.prev_cur[q];
-    if (s >= 0) { stage[s] = 0.0f; stage[s + 1] = 1.0f; stage[s + 2] = 0.0f; }
-  }
-  __syncwarp();
-  uint64_t k0 = 0, k1 = 0;
-#pragma unroll
-  for (int q = 0; q < CPL; ++q) {
-    const int c = lane * CPL + q;
-    const int hsq = cv.hs[q];
-    const float hv = __shfl_sync(kFull, my_hv, hsq < 0 ? 0 : hsq);
-    int sidx = -1;
-    if (c < CELLS) {
-      const int y = cv.cy[q], x = cv.cx[q];
-      float t0, t1, t2;
-      if (c == vhead) { t0 = t1 = t2 = -1.0f; }                           // game.py:248
-      else { t0 = (hsq >= 0) ? hv : 0.0f; t1 = cv.f1[q]; t2 = cv.food[q] ? foodv : 0.0f; }
-      if (out != nullptr) {
-        sidx = 3 * (A * y + B * x) + base3;
-        stage[sidx] = t0; stage[sidx + 1] = t1; stage[sidx + 2] = t2;
-      }
-      if (kWantKey) key_accumulate((uint32_t)(A * y + B * x + Cc), __float_as_uint(t0), __float_as_uint(t1), __float_as_uint(t2), k0, k1);
-    }
-    ctx.prev_cur[q] = sidx;
-  }
-  if (kWantKey) {
-    k0 = warp_sum_u64(k0); k1 = warp_sum_u64(k1);
-    if (k0 == 0) k0 = 1;
-    *key0 = k0; *key1 = k1;
-  }
-  if (out == nullptr) return;
-  fence_proxy_async_smem();
-  __syncwarp();
-  // plane-relative element ranges (32-bit): [eA, eE) is the GR-aligned interior of the plane, [EA, EE) the aligned cover of
-  // the window clipped to it
-  const int eA = (GR - a0) & (GR - 1), eE = PLANE - ((a0 + PLANE) & (GR - 1));
-  int EA = W0 - a, EE = W1 + ((GR - ((a0 + W1) & (GR - 1))) & (GR - 1));
-  if (EA < eA) EA = eA;
-  if (EE > eE) EE = eE;
-  float* obase = out + gidx0;
-  if (lane == 0) {
-    if (EA > eA) bulk_s2g<kHint>(obase + eA, ctx.bg + 4 * (eA % 3), (uint32_t)((EA - eA) * 4), ctx.policy);            // wall before the window
-    bulk_s2g<kHint>(obase + EA, stage + (EA - W0 + off), (uint32_t)((EE - EA) * 4), ctx.policy);                       // the window rows
-    if (eE > EE) bulk_s2g<kHint>(obase + EE, ctx.bg + 4 * (EE % 3), (uint32_t)((eE - EE) * 4), ctx.policy);            // wall after the window
-    bulk_commit();
-  }
-  if (lane >= 1 && lane <= 2 * (GR - 1)) {
-    // up to GR - 1 floats before the first and after the last GR boundary of the plane
-    const int k = lane - 1;                                                                          // head: 0..GR-2, tail: GR-1..
-    const bool is_head = k < GR - 1;
-    const int e = is_head ? k : eE + (k - (GR - 1));
-    const bool on = is_head ? (k < eA) : (e < PLANE);
-    if (on) obase[e] = (e >= W0 && e < W1) ? stage[e - W0 + off] : ((e % 3 == 1) ? 1.0f : 0.0f);      // PLANE % 3 == 0
-  }
-  ctx.cur = ctx.oth; ctx.oth = stage;
-#pragma unroll
-  for (int q = 0; q < CPL; ++q) { const int t = ctx.prev_cur[q]; ctx.prev_cur[q] = ctx.prev_oth[q]; ctx.prev_oth[q] = t; }
-}
-
-// ---- plane encode, v3: pitched planes, one emission per game -------------------------------------------------------
-// The engine's own plane buffers (the network's input batch, the record store) keep consecutive planes PITCH floats apart,
-// PITCH = PLANE rounded up to 8 floats (5,312 B instead of 5,292 B at 11x11): every plane then starts on a 32-byte sector of
-// HBM, which removes everything the 4-byte alignment of dense planes costs in v2 (per-plane edge floats stored by single
-// lanes, alignment arithmetic, three separate copies per plane).  The planes of one game are consecutive rows, so the game
-// is emitted as ONE sequence of bulk copies: wall before the first window, then per plane its window (from the staging
-// buffer) and the wall run up to the next window -- the wall after plane k and the wall before plane k+1 are one contiguous
-// range, copied from a per-CTA constant "seam" buffer that holds a plane end, the pad floats and a plane start.
-// Dense planes (a caller's own [rows][N][N][3] tensor) still go through v2.
 template <class G>
 struct PitchGeo {
   static constexpr int PITCH = ((G::PLANE + 7) / 8) * 8;
@@ -541,94 +406,11 @@ __device__ __forceinline__ void fill_seam_pattern(float* seam, int seam_at, int 
   }
 }
 
-// Encodes the planes of the first n_emit live snakes of one game to gbase (the game's first row: rows are PITCH apart).
-// keys (optional, when kWantKey): 2 words per row; row_ids (optional): game*8 + snake per row.
-template <class G, bool kWantKey, bool kHint>
-__device__ __forceinline__ void warp_encode_game_v3(const CellView<G>& cv, const Snake& sn, unsigned live_mask, int n_emit,
-                                                    EncodeCtx<G>& ctx, float* gbase, uint64_t* keys, int32_t* row_ids, int gid8) {
-  constexpr int SIDE = G::SIDE, CPL = G::CPL, CELLS = G::CELLS, N = G::N;
-  using P = PitchGeo<G>;
-  const int lane = lane_id();
-  int prev_end = 0;          // game-relative float offset up to which the output has been handed to the copy engine
-  unsigned rest = live_mask;
-  for (int k = 0; k < n_emit; ++k) {
-    const int vs = __ffs(rest) - 1;
-    rest &= rest - 1;
-    const int vhead = __shfl_sync(kFull, sn.head, vs);
-    const int vlen = __shfl_sync(kFull, sn.len, vs);
-    const int vhp = __shfl_sync(kFull, sn.health, vs);
-    const int vrot = __shfl_sync(kFull, sn.last, vs);
-    const int hy = vhead / SIDE, hx = vhead - hy * SIDE;
-    const float my_hv = (float)(((double)sn.len - ((double)vlen - 0.5)) * 0.04);      // game.py:229,232 in float64
-    const float foodv = (float)((double)(101 - vhp) * 0.01);                            // game.py:244
-    int A, B, Cc, i0;                                                                   // see warp_encode_v2
-    if (vrot == 0)      { A = N;  B = 1;  Cc = (SIDE - 1 - hy) * N + (SIDE - 1 - hx);             i0 = SIDE - 1 - hy; }
-    else if (vrot == 1) { A = 1;  B = -N; Cc = (N - SIDE + hx) * N + (SIDE - 1 - hy);             i0 = hx; }
-    else if (vrot == 2) { A = -N; B = -1; Cc = (N - SIDE + hy) * N + (N - SIDE + hx);             i0 = hy; }
-    else                { A = -1; B = N;  Cc = (SIDE - 1 - hx) * N + (N - SIDE + hy);             i0 = SIDE - 1 - hx; }
-    const int W0 = i0 * 3 * N;
-    const int a = W0 & 7;
-    const int off = stage_off(a);
-    const int base3 = 3 * Cc - W0 + off;
-    float* stage = ctx.cur;
-    if (lane == 0) bulk_wait_read<1>();      // the store that read this buffer two planes ago has finished reading it
-    __syncwarp();
-#pragma unroll
-    for (int q = 0; q < CPL; ++q) {
-      const int s = ctx.prev_cur[q];
-      if (s >= 0) { stage[s] = 0.0f; stage[s + 1] = 1.0f; stage[s + 2] = 0.0f; }
-    }
-    __syncwarp();
-    uint64_t k0 = 0, k1 = 0;
-#pragma unroll
-    for (int q = 0; q < CPL; ++q) {
-      const int c = lane * CPL + q;
-      const int hsq = cv.hs[q];
-      const float hv = __shfl_sync(kFull, my_hv, hsq < 0 ? 0 : hsq);
-      int sidx = -1;
-      if (c < CELLS) {
-        const int y = cv.cy[q], x = cv.cx[q];
-        float t0, t1, t2;
-        if (c == vhead) { t0 = t1 = t2 = -1.0f; }                           // game.py:248
-        else { t0 = (hsq >= 0) ? hv : 0.0f; t1 = cv.f1[q]; t2 = cv.food[q] ? foodv : 0.0f; }
-        sidx = 3 * (A * y + B * x) + base3;
-        stage[sidx] = t0; stage[sidx + 1] = t1; stage[sidx + 2] = t2;
-        if (kWantKey) key_accumulate((uint32_t)(A * y + B * x + Cc), __float_as_uint(t0), __float_as_uint(t1), __float_as_uint(t2), k0, k1);
-      }
-      ctx.prev_cur[q] = sidx;
-    }
-    if (kWantKey) {
-      k0 = warp_sum_u64(k0); k1 = warp_sum_u64(k1);
-      if (k0 == 0) k0 = 1;
-    }
-    fence_proxy_async_smem();
-    __syncwarp();
-    const int EA = W0 - a, EE = (W0 + P::WIN + 7) & ~7;      // 32-byte aligned cover of the window, plane relative
-    const int plane_off = k * P::PITCH;
-    if (lane == 0) {
-      const int run = plane_off + EA - prev_end;               // wall (and pad) floats between the last window and this one
-      if (run > 0) bulk_s2g<kHint>(gbase + prev_end, ctx.bg + P::SEAM_AT - (plane_off - prev_end), (uint32_t)(run * 4), ctx.policy);
-      bulk_s2g<kHint>(gbase + plane_off + EA, stage + (off - a), (uint32_t)((EE - EA) * 4), ctx.policy);
-      if (k == n_emit - 1 && EE < P::PITCH)                    // the wall after the game's last window
-        bulk_s2g<kHint>(gbase + plane_off + EE, ctx.bg + P::SEAM_AT - (P::PITCH - EE), (uint32_t)((P::PITCH - EE) * 4), ctx.policy);
-      bulk_commit();
-      if (row_ids != nullptr) row_ids[k] = gid8 + vs;
-      if (kWantKey) { keys[2 * k] = k0; keys[2 * k + 1] = k1; }
-    }
-    prev_end = plane_off + EE;
-    ctx.cur = ctx.oth; ctx.oth = stage;
-#pragma unroll
-    for (int q = 0; q < CPL; ++q) { const int t = ctx.prev_cur[q]; ctx.prev_cur[q] = ctx.prev_oth[q]; ctx.prev_oth[q] = t; }
-  }
-}
-
-// ---- v3b: the same emission with table-driven indices and no per-lane bookkeeping ------------------------------------
-// What v3 still spends per plane: the rotation / recentring select chains, two float64 products, the "which stage index did
-// each of my cells go to" arrays of both staging buffers (8 registers, swapped every plane, spilled) and the per-cell
-// own-head selects.  v3b keeps per staging buffer only the (rotation, base) pair of the plane it holds -- warp-uniform --
-// and reads the rotation-dependent linear term of a cell, 3 * (A*y + B*x), from a 1 KB table in shared memory, so the
-// restore pass recomputes its indices instead of remembering them; head and food values come from tables (same float64
-// products, evaluated once per CTA); the viewer's own head is patched by the one lane that owns the cell.
+// Per plane the encode is table driven and keeps no per-lane bookkeeping: per staging buffer only the (rotation, base) pair of
+// the plane it holds is kept -- warp-uniform -- and the rotation-dependent linear term of a cell, 3 * (A*y + B*x), is read from
+// a 1 KB table in shared memory, so the restore pass recomputes its indices instead of remembering them per lane (such
+// per-lane arrays would cost registers that the kernel's occupancy does not have); head and food values come from tables (the
+// same float64 products, evaluated once per CTA); the viewer's own head is patched by the one lane that owns the cell.
 template <class G>
 struct PitchLut {
   static constexpr int LIN = 4 * G::PC;                 // int16 [4 rotations][PC cells]: 3 * (A*y + B*x)
@@ -638,7 +420,8 @@ struct PitchLut {
 };
 template <class G>
 struct EncodeCtxP {
-  float* cur; float* oth;        // staging buffers (see EncodeCtx)
+  float* cur;                    // staging buffer of the next plane
+  float* oth;                    // the other buffer (its bulk store may still be in flight)
   const float* seam;
   uint64_t policy;
   const int16_t* lin; const float* hv; const float* food;
@@ -680,7 +463,9 @@ __device__ __forceinline__ void load_lin(const int16_t* lin, int rot, int lane, 
   }
 }
 
-template <class G, bool kWantKey, bool kHint>
+// Encodes the planes of the first n_emit live snakes of one game to gbase (the game's first row: rows are PITCH apart).
+// keys (optional, when kWantKey): 2 words per row; row_ids (optional): game*8 + snake per row.
+template <class G, bool kWantKey>
 __device__ __forceinline__ void warp_encode_game_v3b(const CellView<G>& cv, const Snake& sn, unsigned live_mask, int n_emit,
                                                      EncodeCtxP<G>& ctx, float* gbase, uint64_t* keys, int32_t* row_ids, int gid8) {
   constexpr int SIDE = G::SIDE, CPL = G::CPL, CELLS = G::CELLS, N = G::N, U = G::SIDE - 1;
@@ -699,8 +484,8 @@ __device__ __forceinline__ void warp_encode_game_v3b(const CellView<G>& cv, cons
     const float my_hv = ctx.hv[sn.len - vlen + CELLS];                                 // game.py:229,232
     const int fi = 101 - vhp;
     const float foodv = (unsigned)fi < (unsigned)PitchLut<G>::FOOD ? ctx.food[fi] : (float)((double)fi * 0.01);   // game.py:244
-    // recentring + rot90 (game.py:249-257), see warp_encode_v2: pixel of cell (y, x) = A*y + B*x + Cc, window row i0;
-    // D = 3*Cc - W0 in closed form per rotation
+    // recentring + rot90 (game.py:249-257) are one affine map of the cell (y, x) to the output pixel A*y + B*x + Cc with
+    // warp-uniform A, B, Cc; i0 = first output row of the board window, D = 3*Cc - W0 in closed form per rotation
     const int t = (vrot & 1) ? hy : hx;                      // rot0: hx, rot1: hy, rot2: hx, rot3: hy
     const int r = (vrot & 1) ? hx : hy;                      // rot0: hy, rot1: hx, rot2: hy, rot3: hx
     const bool flip_t = (vrot == 0) || (vrot == 1);          // D uses (U - t) for rot 0, 1 and (U + t) for rot 2, 3
@@ -755,10 +540,10 @@ __device__ __forceinline__ void warp_encode_game_v3b(const CellView<G>& cv, cons
     const int plane_off = k * P::PITCH;
     if (lane == 0) {
       const int run = plane_off + EA - prev_end;
-      if (run > 0) bulk_s2g<kHint>(gbase + prev_end, ctx.seam + P::SEAM_AT - (plane_off - prev_end), (uint32_t)(run * 4), ctx.policy);
-      bulk_s2g<kHint>(gbase + plane_off + EA, stage + (off - a), (uint32_t)((EE - EA) * 4), ctx.policy);
+      if (run > 0) bulk_s2g(gbase + prev_end, ctx.seam + P::SEAM_AT - (plane_off - prev_end), (uint32_t)(run * 4), ctx.policy);
+      bulk_s2g(gbase + plane_off + EA, stage + (off - a), (uint32_t)((EE - EA) * 4), ctx.policy);
       if (k == n_emit - 1 && EE < P::PITCH)
-        bulk_s2g<kHint>(gbase + plane_off + EE, ctx.seam + P::SEAM_AT - (P::PITCH - EE), (uint32_t)((P::PITCH - EE) * 4), ctx.policy);
+        bulk_s2g(gbase + plane_off + EE, ctx.seam + P::SEAM_AT - (P::PITCH - EE), (uint32_t)((P::PITCH - EE) * 4), ctx.policy);
       bulk_commit();
       if (row_ids != nullptr) row_ids[k] = gid8 + vs;
       if (kWantKey) { keys[2 * k] = k0; keys[2 * k + 1] = k1; }

@@ -9,7 +9,7 @@
 //   mirror_states = flip(states, axis=2)  (the width axis of [n, h, w, 3])      alpha_snake_zero_trainer.py:93-97
 //   mirror_values = flip(values, axis=1)  (left <-> right)                       alpha_snake_zero_trainer.py:99-100
 // Roofline: HBM bandwidth; algorithmic bytes per sampled record = plane read + 2 plane writes = 3 x 5,292 B at 11x11.
-// Stored planes are asz_plane_pitch() floats apart (written by the pitched fast path of the encode); batches are dense.
+// Stored planes are asz_plane_pitch() floats apart (as the encode writes them); batches are dense.
 #include <algorithm>
 #include <cstdio>
 #include <cstring>

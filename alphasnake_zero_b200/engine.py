@@ -69,7 +69,7 @@ class Engine:
     @property
     def planes(self):
         """[G*S, N, N, 3] float32 batch buffer (allocated on first use).  Rows are `pitch` floats apart (the plane size rounded
-        up to 8 floats: every plane starts on a 32-byte sector, the fast path of the encode kernel), so this is a strided
+        up to 8 floats: every plane starts on a 32-byte sector, the one layout the encode kernel writes), so this is a strided
         view; `.contiguous()` / indexing give dense copies."""
         if self._planes is None:
             # empty, not zeros: a 1.4 GB fill would leave the L2 full of dirty lines right before the first launch (DESIGN.md 4.1)
@@ -78,14 +78,13 @@ class Engine:
         return self._planes
 
     def _plane_pitch_of(self, t):
-        """0 for a dense [rows, N, N, 3] tensor, self.pitch for a view with the engine's row pitch"""
+        """self.pitch for a [rows, N, N, 3] view with the engine's row pitch (see `planes`); the encode writes whole rows of
+        `pitch` floats, so a tensor with any other layout is refused"""
         if tuple(t.shape[1:]) != (self.N, self.N, 3) or t.dtype != torch.float32:
             raise AszError("planes must be float32 [rows, %d, %d, 3]" % (self.N, self.N))
-        if t.shape[0] <= 1 or t.is_contiguous():
-            return 0 if t.is_contiguous() else self.pitch
-        if tuple(t.stride()) == (self.pitch, 3 * self.N, 3, 1):
-            return self.pitch
-        raise AszError("planes must be contiguous or have the engine's row pitch")
+        if tuple(t.stride()) != (self.pitch, 3 * self.N, 3, 1):
+            raise AszError("planes must have the engine's row pitch: rows %d floats apart (asz_plane_pitch)" % self.pitch)
+        return self.pitch
 
     def reset(self):
         check(self.L.asz_reset(self.h, self.stream))
@@ -151,10 +150,6 @@ class Engine:
         rows = C.c_int32(0)
         check(self.L.asz_env_wait_host(self.h, ticket, C.byref(rows)))
         return rows.value
-
-    def condition_l2(self):
-        """experiments (tools/env_hot.py): one read sweep that leaves the L2 full of clean lines"""
-        check(self.L.asz_condition_l2(self.h, self.stream))
 
     def totals(self):
         t = np.zeros(16, np.uint64)

@@ -98,7 +98,7 @@ typedef struct {
   const uint8_t* d_actions;      /* [G*8] relative move per (game, snake id); read where the snake is alive */
   const int32_t* d_spawn_cells;  /* [G] for ASZ_SPAWN_REPLAY */
   float* d_planes;               /* [max_rows][2*side-1][2*side-1][3] float32 NHWC, rows compacted; 32-byte aligned; rows are
-                                    plane_pitch floats apart */
+                                    plane_pitch floats apart (room for max_rows * plane_pitch floats) */
   int32_t* d_row_ids;            /* [max_rows] game*8 + snake of every row written */
   uint64_t* d_keys;              /* [max_rows*2] when ASZ_STEP_KEYS */
   int32_t max_rows;
@@ -109,10 +109,10 @@ typedef struct {
                                     this tic and was not stepped (may be NULL) */
   int32_t row_base;              /* rows are written at [row_base, row_base + n) of d_planes / d_row_ids / d_keys; max_rows
                                     stays the absolute capacity (rows past it are dropped, *d_row_count still counts them) */
-  int32_t plane_pitch;           /* floats between consecutive rows of d_planes: 0 (or asz_plane_floats) = dense rows;
-                                    asz_plane_pitch() = the plane size rounded up to 8 floats, so that every row starts on a
-                                    32-byte sector: the layout of the engine's own buffers and the fast path of the encode
-                                    (the pad floats after each plane are written but carry no meaning) */
+  int32_t plane_pitch;           /* floats between consecutive rows of d_planes; must equal asz_plane_pitch() with ASZ_STEP_ENCODE
+                                    (ASZ_ERR_ARG otherwise): the plane size rounded up to 8 floats, so that every row starts on a
+                                    32-byte sector, the layout of the engine's own buffers (the pad floats after each plane are
+                                    written but carry no meaning) */
 } asz_step_args;
 
 /* Enqueues one fused launch.  Row order inside d_planes is unspecified across games (rows of one game are
@@ -152,12 +152,8 @@ int asz_get_totals(asz_engine* e, uint64_t* h_totals);
  * iterating `games` for liveness (mp_game_runner.py:40-42). */
 /* measurement builds only (nvcc -DASZ_ENV_PROFILE, tools/env_profile.py): per-phase cycle sums of env_step_kernel since
  * the last call, h_cycles[8] = record wait, tic, write-back, work-counter wait + prefetch, cell view + row wait, encode,
- * staging-buffer wait (inside encode), unused; all zero in the product build.  Synchronous. */
+ * two unused slots; all zero in the product build.  Synchronous. */
 int asz_internal_profile(asz_engine* e, uint64_t* h_cycles);
-/* experiments only (tools/env_hot.py, DESIGN.md 4.1): the fused kernel's scheduling word at the k-th candidate address of its
- * buffer (another L2 slice), and one read sweep of ~1.25 GB over the engine's plane buffer (leaves the L2 full of clean lines) */
-int asz_internal_set_hot_word(asz_engine* e, int32_t k);
-int asz_condition_l2(asz_engine* e, void* stream);
 int asz_internal_state(asz_engine* e, void** d_ptrs);
 /* device pointer of the engine's internal plane buffer (capacity G*S rows, asz_plane_pitch() floats apart) and row-id buffer */
 float* asz_internal_planes(asz_engine* e);

@@ -49,25 +49,25 @@ def test_all_games_finished_produce_no_rows_and_no_moves():
     eng.close()
 
 
-def test_plane_batch_smaller_than_the_live_rows():
+def test_pitched_plane_batch_smaller_than_the_live_rows():
     """max_rows below the number of live snakes: the rows that fit are complete planes, the counter still says how many
     rows there were, nothing is written past the buffer"""
     import torch
-    from alphasnake_zero_b200 import _lib
     eng = _engine(side=11, snakes=4, games=256, seed=9)
     eng.reset()
-    full = torch.zeros(256 * 4, 21, 21, 3, device="cuda")
-    eng.step(tic=False, encode=True, planes=full)
+    eng.step(tic=False, encode=True)
     n = int(eng.row_count.item())
     assert n == 1024
     ids_full = eng.row_ids[:n].cpu().numpy().copy()
-    ref = {int(i): full[r].cpu().numpy() for r, i in enumerate(ids_full)}
-    small = torch.full((100 + 8, 21, 21, 3), 7.0, device="cuda")
-    eng.step(tic=False, encode=True, planes=small[:100])
+    full = eng.planes[:n].cpu().numpy()
+    ref = {int(i): full[r] for r, i in enumerate(ids_full)}
+    flat = torch.full(((100 + 8) * eng.pitch,), 7.0, device="cuda")
+    small = torch.as_strided(flat, (100, 21, 21, 3), (eng.pitch, 3 * 21, 3, 1))
+    eng.step(tic=False, encode=True, planes=small)
     assert int(eng.row_count.item()) == 1024            # rows that existed, not rows that fit
-    assert bool((small[100:] == 7.0).all().item())      # nothing past the 100 rows
+    assert bool((flat[100 * eng.pitch:] == 7.0).all().item())      # nothing past the 100 rows
     ids = eng.row_ids[:100].cpu().numpy()
-    got = small[:100].cpu().numpy()
+    got = small.cpu().numpy()
     for r in range(100):
         assert np.array_equal(got[r].view(np.uint32), ref[int(ids[r])].view(np.uint32))
     eng.close()
@@ -96,6 +96,7 @@ def torch_float32():
 
 
 def test_argument_errors_are_reported():
+    import torch
     from alphasnake_zero_b200 import _lib
     from alphasnake_zero_b200.engine import AszError
     eng = _engine(side=11, snakes=4, games=8, seed=1)
@@ -105,6 +106,19 @@ def test_argument_errors_are_reported():
     a.spawn_mode = _lib.SPAWN_NATIVE
     assert _lib.lib().asz_env_step(eng.h, C.byref(a), eng.stream) != 0
     assert b"d_actions" in _lib.lib().asz_last_error()
+    # the encode writes rows asz_plane_pitch() floats apart: dense rows (0 or the plane size) are refused, not reinterpreted
+    for pitch in (0, int(_lib.lib().asz_plane_floats(eng.h))):
+        a = _lib.StepArgs()
+        a.flags = _lib.STEP_ENCODE
+        a.d_planes = eng.planes.data_ptr()
+        a.d_row_ids = eng.row_ids.data_ptr()
+        a.d_row_count = eng.row_count.data_ptr()
+        a.max_rows = eng.max_rows
+        a.plane_pitch = pitch
+        assert _lib.lib().asz_env_step(eng.h, C.byref(a), eng.stream) != 0
+        assert b"asz_plane_pitch" in _lib.lib().asz_last_error()
+    with pytest.raises(AszError):
+        eng.step(tic=False, encode=True, planes=torch.zeros(8, 21, 21, 3, device="cuda"))
     with pytest.raises(AszError):
         eng.search(value_fn=None)                       # the engine was created without a search configuration
     eng.close()

@@ -6,24 +6,15 @@ warp-cycles per phase for: A device path, B encode only, C device path after B.
 import os, subprocess, sys
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 PROF_LIB = os.path.join(ROOT, "tools", "libasz_b200_prof.so")
-if len(sys.argv) > 2 and sys.argv[1] == "build-variant":       # python tools/env_profile.py build-variant NAME -DFLAG ...
-    csrc = os.path.join(ROOT, "alphasnake_zero_b200", "csrc")
-    out = os.path.join(ROOT, "tools", "libasz_b200_%s.so" % sys.argv[2])
-    subprocess.check_call(["nvcc", "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17", "-Xcompiler", "-fPIC",
-                           "--expt-relaxed-constexpr"] + sys.argv[3:] + ["-shared", "-o", out] +
-                          [os.path.join(csrc, f) for f in ("asz_env.cu", "asz_mcts.cu", "asz_net.cu", "asz_records.cu")] + ["-lcuda", "-ldl"])
-    print(out)
-    sys.exit(0)
+sys.path.insert(0, ROOT)
 if len(sys.argv) > 1 and sys.argv[1] == "build":
-    csrc = os.path.join(ROOT, "alphasnake_zero_b200", "csrc")
-    cmd = ["nvcc", "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17", "-Xcompiler", "-fPIC",
-           "--expt-relaxed-constexpr", "-DASZ_ENV_PROFILE", "-shared", "-o", PROF_LIB] + \
-          [os.path.join(csrc, f) for f in ("asz_env.cu", "asz_mcts.cu", "asz_net.cu", "asz_records.cu")] + ["-lcuda", "-ldl"]
+    from alphasnake_zero_b200 import build
+    cmd = ["nvcc"] + build.NVCC_FLAGS + ["-DASZ_ENV_PROFILE", "-shared", "-o", PROF_LIB] + \
+          [os.path.join(build.CSRC, f) for f in build.SOURCES] + ["-lcuda", "-ldl"]
     subprocess.check_call(cmd)
     print(PROF_LIB)
     sys.exit(0)
 os.environ.setdefault("ASZ_LIB", PROF_LIB)
-sys.path.insert(0, ROOT)
 import ctypes as C
 import numpy as np, torch
 from alphasnake_zero_b200 import _lib
@@ -32,7 +23,7 @@ G = 65536
 eng = Engine(side=11, snakes=4, health_dec=1, games=G, seed=1); eng.reset(); _ = eng.planes
 kw = dict(spawn_mode=2, tic=True, encode=True, auto_reset=True, random_actions=True)
 kw_enc = dict(tic=False, encode=True)
-names = ("record wait", "tic", "write-back", "counter wait+prefetch", "cell view+row wait", "encode", "  (staging wait)", "-")
+names = ("record wait", "tic", "write-back", "counter wait+prefetch", "cell view+row wait", "encode", "-", "-")
 def phase(name, kw, n=300):
     h = np.zeros(8, np.uint64)
     _lib.check(_lib.lib().asz_internal_profile(eng.h, h.ctypes.data_as(C.c_void_p)))
@@ -43,7 +34,7 @@ def phase(name, kw, n=300):
     us = e0.elapsed_time(e1) / n * 1000
     _lib.check(_lib.lib().asz_internal_profile(eng.h, h.ctypes.data_as(C.c_void_p)))
     tot = float(h[:6].sum())
-    print("%-22s %.1f us/launch | kcycles per game: %s" % (name, us, ", ".join("%s %.2f" % (names[k], h[k] / n / G / 1e3) for k in range(7))))
+    print("%-22s %.1f us/launch | kcycles per game: %s" % (name, us, ", ".join("%s %.2f" % (names[k], h[k] / n / G / 1e3) for k in range(6))))
 for _ in range(20): eng.step(**kw)
 phase("A tic+encode", kw); phase("A tic+encode", kw)
 phase("B encode only", kw_enc)

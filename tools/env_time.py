@@ -1,7 +1,6 @@
 """Per-launch timing of env_step_kernel on BASELINE.json configs[1] (65,536 games, tic + encode, in-kernel actions, in-place
 reset): median / p05 / p95 over per-launch CUDA events, the algorithmic GB/s and the fraction of the measured HBM copy peak.
-  [ASZ_LIB=tools/libasz_b200_<variant>.so] python tools/env_time.py [launches] [dense]
-`dense` times the dense-row path (a caller's contiguous tensor) instead of the engine's pitched buffer."""
+  [ASZ_LIB=tools/libasz_b200_<variant>.so] python tools/env_time.py [launches]"""
 import json
 import os
 import sys
@@ -13,7 +12,6 @@ import torch  # noqa: E402
 from alphasnake_zero_b200.engine import Engine  # noqa: E402
 
 n = int(sys.argv[1]) if len(sys.argv) > 1 else 600
-dense = len(sys.argv) > 2 and sys.argv[2] == "dense"
 G = 65536
 if "LOCAL_RANK" in os.environ:
     torch.cuda.set_device(int(os.environ["LOCAL_RANK"]))
@@ -33,8 +31,7 @@ eng.reset()
 if nccl_mode == "nccl_after":     # engine first
     _ = eng.planes
     nccl_init()
-planes = torch.empty(G * 4, 21, 21, 3, device="cuda") if dense else None
-kw = dict(spawn_mode=2, tic=True, encode=True, auto_reset=True, random_actions=True, planes=planes)
+kw = dict(spawn_mode=2, tic=True, encode=True, auto_reset=True, random_actions=True)
 for _ in range(50):
     eng.step(**kw)
 torch.cuda.synchronize()
@@ -56,6 +53,6 @@ try:
 except Exception:
     pass
 gbs = bytes_per_launch / (tot_us / n) / 1e3
-print("%s %s: %d launches, %.1f us/launch (events per launch: median %.1f, p05 %.1f, p95 %.1f, max %.1f) | %.0f MB algorithmic per launch, "
-      "%.0f GB/s = %.3f of %.0f GB/s | %.3e env steps/s" % (os.environ.get("ASZ_LIB", "libasz_b200.so"), "dense" if dense else "pitched", n, tot_us / n,
+print("%s pitched: %d launches, %.1f us/launch (events per launch: median %.1f, p05 %.1f, p95 %.1f, max %.1f) | %.0f MB algorithmic per launch, "
+      "%.0f GB/s = %.3f of %.0f GB/s | %.3e env steps/s" % (os.environ.get("ASZ_LIB", "libasz_b200.so"), n, tot_us / n,
        np.median(d), np.percentile(d, 5), np.percentile(d, 95), d.max(), bytes_per_launch / 1e6, gbs, gbs / peak, peak, tics / (tot_us * 1e-6)))
