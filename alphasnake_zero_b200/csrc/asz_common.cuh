@@ -22,9 +22,9 @@ constexpr unsigned kFull = 0xffffffffu;
 //   * make_state writes dist*0.02 tail->head so the topmost segment wins (game.py:236-241): exactly the stamp.
 constexpr uint16_t kFood = 0x8000u;
 constexpr uint16_t kDistMask = 0x0fffu;
-__device__ __forceinline__ bool cell_is_body(uint32_t v) { return v != 0u && v != kFood; }
-__device__ __forceinline__ int cell_owner(uint32_t v) { return (int)((v >> 12) & 7u); }
-__device__ __forceinline__ int cell_dist(uint32_t v) { return (int)(v & kDistMask); }
+__host__ __device__ __forceinline__ bool cell_is_body(uint32_t v) { return v != 0u && v != kFood; }
+__host__ __device__ __forceinline__ int cell_owner(uint32_t v) { return (int)((v >> 12) & 7u); }
+__host__ __device__ __forceinline__ int cell_dist(uint32_t v) { return (int)(v & kDistMask); }
 
 // ---- Philox4x32-10 ----------------------------------------------------------------------------------------------
 enum RngStream : uint32_t { RS_INIT = 0, RS_SPAWN = 1, RS_ACT_LO = 2, RS_ACT_HI = 3, RS_TREE = 4, RS_ROOT = 5 };
@@ -71,6 +71,23 @@ __host__ __device__ __forceinline__ void key_accumulate(uint32_t pix, uint32_t a
 __device__ __forceinline__ int argmax3(const float z[3]) {
   if (z[0] > z[1]) return (z[0] > z[2]) ? 0 : 2;
   return (z[1] > z[2]) ? 1 : 2;
+}
+// AlphaNNet.v's obstacle mask (alpha_nnet.py:63-76) on one plane: a move whose target cell next to the viewer's head holds a
+// body value (ch1) of at least 0.04 is valued -1.  numpy1_mask: compared in float64 (NumPy 1.18), otherwise in float32
+// (NumPy >= 2).  Only the masked entries of v are written.
+__device__ __forceinline__ void obstacle_mask3(const float* plane, int side, int numpy1_mask, float v[3]) {
+  const int N = 2 * side - 1, c = side - 1;
+  const float b[3] = {plane[((size_t)c * N + (c - 1)) * 3 + 1], plane[((size_t)(c - 1) * N + c) * 3 + 1], plane[((size_t)c * N + (c + 1)) * 3 + 1]};
+#pragma unroll
+  for (int k = 0; k < 3; ++k) {
+    const bool obs = numpy1_mask ? ((double)b[k] >= 0.04) : (b[k] >= 0.04f);
+    if (obs) v[k] = -1.0f;
+  }
+}
+// deterministic stand-in for the value network: three 16-bit fields of a plane-key word mapped to [-1, 1)
+__device__ __forceinline__ void stub_value3(uint64_t word, float v[3]) {
+#pragma unroll
+  for (int k = 0; k < 3; ++k) v[k] = ((float)(uint32_t)((word >> (16 * k)) & 0xFFFFull) - 32767.5f) * (1.0f / 32768.0f);
 }
 
 // ---- warp helpers -----------------------------------------------------------------------------------------------

@@ -57,15 +57,6 @@ struct EnvParams {
 #define ASZ_PROF(k) do { } while (0)
 #endif
 
-// ---- record store ---------------------------------------------------------------------------------------------------
-__device__ __forceinline__ void store_meta(uint32_t* gm, const Meta& m, int lane) {
-  if (lane < 8) {
-    const uint32_t v = lane == 0 ? m.turn : lane == 1 ? m.episode : lane == 2 ? m.wall : lane == 3 ? m.body
-                     : lane == 4 ? m.headc : lane == 5 ? m.starve : lane == 6 ? m.eaten : m.flags;
-    gm[lane] = v;
-  }
-}
-
 // ---- the fused step kernel ----------------------------------------------------------------------------------------
 // Persistent: MINB CTAs per SM, every warp loops over games g = warp_global, warp_global + n_warps, ... so that the
 // staging buffers' wall background is written once per warp and bulk stores of one game overlap the tic of the next.
@@ -154,11 +145,9 @@ __global__ void __launch_bounds__(WARPS * 32, MINB) env_step_kernel(const EnvPar
     uint32_t* dst = reinterpret_cast<uint32_t*>(board);
 #pragma unroll
     for (int q = 0; q < BW; ++q) dst[lane * BW + q] = pf_board[q];
-    sn.head = 0xFFFF; sn.len = 0; sn.health = 0; sn.last = 0; sn.alive = 0; sn.reward = 0;
+    sn = unpack_snake(kEmptySnake);
     if (lane < 8) sn = unpack_snake(pf_snake);
-    m.turn = __shfl_sync(kFull, pf_meta, 0); m.episode = __shfl_sync(kFull, pf_meta, 1); m.wall = __shfl_sync(kFull, pf_meta, 2);
-    m.body = __shfl_sync(kFull, pf_meta, 3); m.headc = __shfl_sync(kFull, pf_meta, 4); m.starve = __shfl_sync(kFull, pf_meta, 5);
-    m.eaten = __shfl_sync(kFull, pf_meta, 6); m.flags = __shfl_sync(kFull, pf_meta, 7);
+    m = meta_from_lanes(pf_meta);
     act_slot = pf_slot; pf_slot ^= 1;
     __syncwarp();
   };
@@ -171,7 +160,7 @@ __global__ void __launch_bounds__(WARPS * 32, MINB) env_step_kernel(const EnvPar
                        bool last, int n_before, int& row, int& nxt) {
     live_mask = 0u; n_rows = 0;
     auto rows_and_ticket = [&]() {
-      if (enc && !(m.flags & 1u)) {
+      if (enc && !(m.flags & kMetaDone)) {
         live_mask = __ballot_sync(kFull, sn.alive != 0);
         n_rows = __popc(live_mask);
       }
@@ -181,7 +170,7 @@ __global__ void __launch_bounds__(WARPS * 32, MINB) env_step_kernel(const EnvPar
         s_wtot[warp][8] += (uint32_t)(n_before + n_rows);
       }
     };
-    if ((p.flags & ASZ_STEP_TIC) && !(m.flags & 1u)) {
+    if ((p.flags & ASZ_STEP_TIC) && !(m.flags & kMetaDone)) {
       int move = 1;
       uint32_t spawn_r[2] = {0u, 0u};
       const bool merged_rng = (p.flags & ASZ_STEP_RANDOM_ACT) && p.spawn_mode == ASZ_SPAWN_NATIVE;
@@ -230,8 +219,7 @@ __global__ void __launch_bounds__(WARPS * 32, MINB) env_step_kernel(const EnvPar
         }
       }
       if (lane < 8) {
-        const uint32_t mv = lane == 0 ? m.turn : lane == 1 ? m.episode : lane == 2 ? m.wall : lane == 3 ? m.body
-                          : lane == 4 ? m.headc : lane == 5 ? m.starve : lane == 6 ? m.eaten : m.flags;
+        const uint32_t mv = meta_word(m, lane);
         const uint64_t rec = pack_snake(sn);
         if (stash != nullptr) stash[lane] = rec;
         st_hint_u64(p.snakes + (size_t)g * 8 + lane, rec, keep);
@@ -332,7 +320,8 @@ __global__ void __launch_bounds__(WARPS * 32) env_reset_kernel(uint16_t* cells, 
 #pragma unroll
   for (int q = 0; q < G::CPL; ++q) cells[(size_t)g * G::PC + lane * G::CPL + q] = sb[lane * G::CPL + q];
   if (lane < 8) snakes[(size_t)g * 8 + lane] = pack_snake(sn);
-  store_meta(meta + (size_t)g * 8, m, lane);
+  uint32_t* gm = meta + (size_t)g * 8;
+  if (lane < 8) gm[lane] = meta_word(m, lane);
 }
 
 template <int SIDE>
@@ -396,7 +385,12 @@ void gameset_free(GameSet& gs) {
   gs = GameSet();
 }
 
-static int pc_of(int side) { return side == 7 ? Geo<7>::PC : side == 11 ? Geo<11>::PC : Geo<19>::PC; }
+// cells, plane floats and plane pitch of the engine's buffers: the kernels' own geometry
+template <int SIDE>
+static void engine_geometry(asz_engine* e) {
+  using G = Geo<SIDE>;
+  e->pc = G::PC; e->plane = G::PLANE; e->pitch = PitchGeo<G>::PITCH;
+}
 
 }  // namespace asz
 
@@ -412,9 +406,11 @@ static int engine_alloc(asz_engine* e, const asz_config* cfg) {
   e->cfg = *cfg;
   ASZ_CUDA(cudaGetDevice(&e->device));
   ASZ_CUDA(cudaDeviceGetAttribute(&e->n_sm, cudaDevAttrMultiProcessorCount, e->device));
-  e->pc = pc_of(cfg->side);
-  e->plane = (2 * cfg->side - 1) * (2 * cfg->side - 1) * 3;
-  e->pitch = (e->plane + 7) / 8 * 8;   // PitchGeo::PITCH: rows of the engine's own plane buffers start on 32-byte sectors
+  switch (cfg->side) {
+    case 7: engine_geometry<7>(e); break;
+    case 11: engine_geometry<11>(e); break;
+    default: engine_geometry<19>(e); break;
+  }
   double th = (double)cfg->food_chance * 4294967296.0;
   // 0 = the reference's `food_spawn_chance > 0.0` guard is false (game.py:130): no spawning at all, not even on a board without food
   e->chance_thresh = cfg->food_chance <= 0.0f ? 0u : th >= 4294967295.0 ? 4294967295u : th < 1.0 ? 1u : (uint32_t)th;
@@ -730,18 +726,17 @@ static int gs_get_state(const asz_config& cfg, int pc, const GameSet& gs, int32_
   ASZ_CUDA(cudaMemcpy(meta, gs.meta + (size_t)game * 8, sizeof meta, cudaMemcpyDeviceToHost));
   for (int c = 0; c < C; ++c) {
     const uint16_t v = cells[c];
-    h_food[c] = v == 0x8000u; h_owner[c] = -1; h_dist[c] = 0;
-    if (v != 0 && v != 0x8000u) { h_owner[c] = (v >> 12) & 7; h_dist[c] = v & 0x0fff; }
+    h_food[c] = v == kFood; h_owner[c] = -1; h_dist[c] = 0;
+    if (cell_is_body(v)) { h_owner[c] = cell_owner(v); h_dist[c] = cell_dist(v); }
   }
   for (int s = 0; s < cfg.snakes; ++s) {
-    const uint64_t v = sn[s];
+    const Snake v = unpack_snake(sn[s]);
     int32_t* o = h_snake + 6 * s;
-    const int head = (int)(v & 0xFFFF), rw = (int)((v >> 43) & 3);
-    o[0] = (int)((v >> 42) & 1); o[1] = (int)(int16_t)(uint16_t)(((v >> 32) & 0xFF) | (((v >> 48) & 0xFF) << 8)); o[2] = (int)((v >> 16) & 0xFFFF);
-    o[3] = (int)((v >> 40) & 3); o[4] = head == 0xFFFF ? -1 : head; o[5] = rw == 1 ? 1 : rw == 2 ? -1 : 0;
+    o[0] = v.alive; o[1] = v.health; o[2] = v.len;
+    o[3] = v.last; o[4] = v.head == kNoHead ? -1 : v.head; o[5] = v.reward == 1 ? 1 : v.reward == 2 ? -1 : 0;
   }
-  for (int k = 0; k < 5; ++k) h_counters[k] = (int32_t)meta[2 + k];
-  h_counters[5] = (int32_t)meta[0]; h_counters[6] = (int32_t)meta[1]; h_counters[7] = (int32_t)(meta[7] & 1u);
+  for (int k = 0; k < 5; ++k) h_counters[k] = (int32_t)meta[META_WALL + k];
+  h_counters[5] = (int32_t)meta[META_TURN]; h_counters[6] = (int32_t)meta[META_EPISODE]; h_counters[7] = (int32_t)(meta[META_FLAGS] & kMetaDone);
   return ASZ_OK;
 }
 
@@ -752,31 +747,30 @@ static int gs_set_state(const asz_config& cfg, int pc, GameSet& gs, int32_t game
   std::vector<uint16_t> cells(pc, 0);
   uint64_t sn[8] = {0}; uint32_t meta[8] = {0};
   for (int c = 0; c < C; ++c) {
-    if (h_food[c]) cells[c] = 0x8000u;
+    if (h_food[c]) cells[c] = kFood;
     else if (h_owner[c] >= 0) {
-      if (h_owner[c] >= cfg.snakes || h_dist[c] <= 0 || h_dist[c] > 0x0fff) { set_error("bad cell stamp"); return ASZ_ERR_ARG; }
+      if (h_owner[c] >= cfg.snakes || h_dist[c] <= 0 || h_dist[c] > kDistMask) { set_error("bad cell stamp"); return ASZ_ERR_ARG; }
       cells[c] = (uint16_t)((h_owner[c] << 12) | h_dist[c]);
     }
   }
   int live = 0;
   for (int s = 0; s < 8; ++s) {
-    uint64_t v = 0xFFFFull;
+    uint64_t v = kEmptySnake;
     if (s < cfg.snakes) {
       const int32_t* o = h_snake + 6 * s;
-      const int alive = o[0] != 0;
+      const int alive = o[0] != 0, hp = alive ? o[1] : 0;
       live += alive;
-      const int head = (alive && o[4] >= 0) ? o[4] : 0xFFFF;
-      const int rw = o[5] > 0 ? 1 : o[5] < 0 ? 2 : 0;
-      const int hp = alive ? o[1] : 0;
       if (hp < -32768 || hp > 32767) { set_error("health out of range"); return ASZ_ERR_ARG; }
-      v = (uint64_t)(head & 0xFFFF) | ((uint64_t)((alive ? o[2] : 0) & 0xFFFF) << 16) | ((uint64_t)(hp & 0xFF) << 32) |
-          ((uint64_t)(o[3] & 3) << 40) | ((uint64_t)alive << 42) | ((uint64_t)rw << 43) | ((uint64_t)((hp >> 8) & 0xFF) << 48);
+      Snake r;
+      r.head = (alive && o[4] >= 0) ? o[4] : kNoHead; r.len = alive ? o[2] : 0; r.health = hp;
+      r.last = o[3]; r.alive = alive; r.reward = o[5] > 0 ? 1 : o[5] < 0 ? 2 : 0;
+      v = pack_snake(r);
     }
     sn[s] = v;
   }
-  meta[0] = (uint32_t)h_counters[5]; meta[1] = (uint32_t)h_counters[6];
-  for (int k = 0; k < 5; ++k) meta[2 + k] = (uint32_t)h_counters[k];
-  meta[7] = (h_counters[7] != 0 || live <= 1) ? 1u : 0u;
+  meta[META_TURN] = (uint32_t)h_counters[5]; meta[META_EPISODE] = (uint32_t)h_counters[6];
+  for (int k = 0; k < 5; ++k) meta[META_WALL + k] = (uint32_t)h_counters[k];
+  meta[META_FLAGS] = (h_counters[7] != 0 || live <= 1) ? kMetaDone : 0u;
   ASZ_CUDA(cudaDeviceSynchronize());
   ASZ_CUDA(cudaMemcpy(gs.cells + (size_t)game * pc, cells.data(), pc * sizeof(uint16_t), cudaMemcpyHostToDevice));
   ASZ_CUDA(cudaMemcpy(gs.snakes + (size_t)game * 8, sn, sizeof sn, cudaMemcpyHostToDevice));

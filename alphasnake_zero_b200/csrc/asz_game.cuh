@@ -23,33 +23,53 @@ struct Geo {
 };
 
 // ---- packed records in HBM ---------------------------------------------------------------------------------------
+// The one definition of the record format, for the kernels and for the host's state interchange alike.
 // snake: head:16 | len:16 | health low byte:8 | last_move:2 | alive:1 | reward:2 (0 none, 1 = +1, 2 = -1) | pad:3 |
 // health high byte:8.  Health is a SIGNED 16-bit value split over bits 32..39 and 48..55: the kill chain of game.py:156-165
 // is an elif chain, so the winner of a head-on collision skips the starvation check and can end a tic alive with
 // health <= 0 (down to 1 - 7*health_dec after seven wins in a row); it starves on the next tic it does not eat.
 struct Snake {
-  int head;    // cell index, 0xFFFF = none
+  int head;    // cell index, kNoHead = none
   int len;
   int health;
   int last;
   int alive;
   int reward;
 };
-__device__ __forceinline__ uint64_t pack_snake(const Snake& s) {
+constexpr int kNoHead = 0xFFFF;
+constexpr uint64_t kEmptySnake = (uint64_t)kNoHead;   // record of a slot without a snake: unpack_snake gives head kNoHead, all else 0
+__host__ __device__ __forceinline__ uint64_t pack_snake(const Snake& s) {
   return (uint64_t)(s.head & 0xFFFF) | ((uint64_t)(s.len & 0xFFFF) << 16) | ((uint64_t)(s.health & 0xFF) << 32) |
          ((uint64_t)(s.last & 3) << 40) | ((uint64_t)(s.alive & 1) << 42) | ((uint64_t)(s.reward & 3) << 43) |
          ((uint64_t)((s.health >> 8) & 0xFF) << 48);
 }
-__device__ __forceinline__ Snake unpack_snake(uint64_t v) {
+__host__ __device__ __forceinline__ Snake unpack_snake(uint64_t v) {
   Snake s;
   s.head = (int)(v & 0xFFFF); s.len = (int)((v >> 16) & 0xFFFF); s.health = (int)(int16_t)(uint16_t)(((v >> 32) & 0xFF) | (((v >> 48) & 0xFF) << 8));
   s.last = (int)((v >> 40) & 3); s.alive = (int)((v >> 42) & 1); s.reward = (int)((v >> 43) & 3);
   return s;
 }
-// game meta: 8 x u32 = turn(game_length), episode, wall, body, head, starve, food_eaten, flags (bit0 = done)
+__host__ __device__ __forceinline__ bool snake_alive(uint64_t v) { return (v >> 42) & 1ull; }
+
+// game meta: 8 x u32, one per slot; flags bit 0 = done
+enum MetaSlot : int { META_TURN = 0, META_EPISODE, META_WALL, META_BODY, META_HEAD, META_STARVE, META_EATEN, META_FLAGS };
+constexpr uint32_t kMetaDone = 1u;
 struct Meta {
   uint32_t turn, episode, wall, body, headc, starve, eaten, flags;
 };
+// the word of slot `slot` (lane `slot` of a warp writes slot `slot` of the record)
+__device__ __forceinline__ uint32_t meta_word(const Meta& m, int slot) {
+  return slot == META_TURN ? m.turn : slot == META_EPISODE ? m.episode : slot == META_WALL ? m.wall : slot == META_BODY ? m.body
+       : slot == META_HEAD ? m.headc : slot == META_STARVE ? m.starve : slot == META_EATEN ? m.eaten : m.flags;
+}
+// the record from the warp's lanes: lane k holds slot k
+__device__ __forceinline__ Meta meta_from_lanes(uint32_t v) {
+  Meta m;
+  m.turn = __shfl_sync(kFull, v, META_TURN); m.episode = __shfl_sync(kFull, v, META_EPISODE); m.wall = __shfl_sync(kFull, v, META_WALL);
+  m.body = __shfl_sync(kFull, v, META_BODY); m.headc = __shfl_sync(kFull, v, META_HEAD); m.starve = __shfl_sync(kFull, v, META_STARVE);
+  m.eaten = __shfl_sync(kFull, v, META_EATEN); m.flags = __shfl_sync(kFull, v, META_FLAGS);
+  return m;
+}
 
 struct TicResult {
   unsigned live_mask;   // snakes alive after the tic
@@ -88,7 +108,7 @@ __device__ __forceinline__ void warp_init_native(uint16_t* sb, Snake& sn, Meta& 
 #pragma unroll
   for (int q = 0; q < G::CPL; ++q) sb[lane * G::CPL + q] = 0;
   __syncwarp();
-  sn.head = 0xFFFF; sn.len = 0; sn.health = 0; sn.last = 0; sn.alive = 0; sn.reward = 0;
+  sn = unpack_snake(kEmptySnake);
   if (lane == 0) sb[(H / 2) * W + W / 2] = kFood;                     // game.py:43
   if (lane < S) {
     uint32_t vv = v[0], ww = w[0];
@@ -229,7 +249,7 @@ __device__ __forceinline__ TicResult warp_tic(uint16_t* sb, Snake& sn, Meta& m, 
     }
     __syncwarp();
   }
-  if (cause != 0) { sn.alive = 0; sn.reward = 2; sn.head = 0xFFFF; sn.len = 0; sn.health = 0; }
+  if (cause != 0) { sn.alive = 0; sn.reward = 2; sn.head = kNoHead; sn.len = 0; sn.health = 0; }
   else if (was_alive) { sb[nh] = (uint16_t)((lane << 12) | sn.len); sn.head = nh; }
   __syncwarp();
   // 7. terminate (game.py:197-205)
@@ -238,7 +258,7 @@ __device__ __forceinline__ TicResult warp_tic(uint16_t* sb, Snake& sn, Meta& m, 
   r.live_mask = __ballot_sync(kFull, sn.alive != 0);
   r.dead_mask = dead_mask;
   r.ended = __popc(r.live_mask) <= 1;
-  if (r.ended) { m.flags |= 1u; if (sn.alive) sn.reward = 1; }
+  if (r.ended) { m.flags |= kMetaDone; if (sn.alive) sn.reward = 1; }
   return r;
 }
 

@@ -163,18 +163,18 @@ __global__ void search_epoch_begin_kernel(const SearchParams p) {
   if (threadIdx.x < 8) {
     const uint64_t sv = p.r_snakes[(size_t)g * 8 + threadIdx.x];
     p.snakes[(size_t)sub * 8 + threadIdx.x] = sv;
-    const unsigned alive = __ballot_sync(0xffu, (sv >> 42) & 1ull);
+    const unsigned alive = __ballot_sync(0xffu, snake_alive(sv));
     // meta: sub-game counters restart (game.py:268 builds a fresh Game); done flag is inherited
-    const uint32_t rflags = p.r_meta[(size_t)g * 8 + 7];
-    const uint32_t repi = p.r_meta[(size_t)g * 8 + 1];
-    p.meta[(size_t)sub * 8 + threadIdx.x] = threadIdx.x == 1 ? repi : threadIdx.x == 7 ? (rflags & 1u) : 0u;
+    const uint32_t rflags = p.r_meta[(size_t)g * 8 + META_FLAGS];
+    const uint32_t repi = p.r_meta[(size_t)g * 8 + META_EPISODE];
+    p.meta[(size_t)sub * 8 + threadIdx.x] = threadIdx.x == META_EPISODE ? repi : threadIdx.x == META_FLAGS ? (rflags & kMetaDone) : 0u;
     p.path_len[(size_t)sub * 8 + threadIdx.x] = 0;
     p.row_slot[(size_t)sub * 8 + threadIdx.x] = kNoRow;
     if (threadIdx.x == 0) {
       p.sub_depth[sub] = p.D - 2 * (__popc(alive) - 2);   // agent.py:45
-      p.sub_left[sub] = (uint8_t)(rflags & 1u);
+      p.sub_left[sub] = (uint8_t)(rflags & kMetaDone);
       p.created[sub] = (uint8_t)alive;
-      if (!(rflags & 1u) && sub % p.P == 0) atomicAdd(&p.stats[ST_SUBGAMES], (unsigned long long)p.P);
+      if (!(rflags & kMetaDone) && sub % p.P == 0) atomicAdd(&p.stats[ST_SUBGAMES], (unsigned long long)p.P);
     }
   }
 }
@@ -206,15 +206,9 @@ __global__ void __launch_bounds__(WARPS * 32) search_step_kernel(const SearchPar
 #pragma unroll
     for (int q = 0; q < G::CPL / 2; ++q) dst[q * 32 + lane] = src[q * 32 + lane];
   }
-  Snake sn; sn.head = 0xFFFF; sn.len = 0; sn.health = 0; sn.last = 0; sn.alive = 0; sn.reward = 0;
+  Snake sn = unpack_snake(kEmptySnake);
   if (lane < 8) sn = unpack_snake(p.snakes[(size_t)sub * 8 + lane]);
-  Meta m;
-  {
-    const uint32_t v = (lane < 8) ? p.meta[(size_t)sub * 8 + lane] : 0u;
-    m.turn = __shfl_sync(kFull, v, 0); m.episode = __shfl_sync(kFull, v, 1); m.wall = __shfl_sync(kFull, v, 2);
-    m.body = __shfl_sync(kFull, v, 3); m.headc = __shfl_sync(kFull, v, 4); m.starve = __shfl_sync(kFull, v, 5);
-    m.eaten = __shfl_sync(kFull, v, 6); m.flags = __shfl_sync(kFull, v, 7);
-  }
+  Meta m = meta_from_lanes((lane < 8) ? p.meta[(size_t)sub * 8 + lane] : 0u);
   __syncwarp();
   const size_t ri = (size_t)sub * 8 + lane;   // (sub-game, snake) index of this lane, valid for lane < 8
   bool left = false;
@@ -242,9 +236,7 @@ __global__ void __launch_bounds__(WARPS * 32) search_step_kernel(const SearchPar
       for (int q = 0; q < G::CPL / 2; ++q) dst[q * 32 + lane] = src[q * 32 + lane];
       if (lane < 8) {
         p.snakes[ri] = pack_snake(sn);
-        const uint32_t v = lane == 0 ? m.turn : lane == 1 ? m.episode : lane == 2 ? m.wall : lane == 3 ? m.body
-                         : lane == 4 ? m.headc : lane == 5 ? m.starve : lane == 6 ? m.eaten : m.flags;
-        p.meta[ri] = v;
+        p.meta[ri] = meta_word(m, lane);
       }
     }
     if (left) {
@@ -389,9 +381,8 @@ __global__ void search_root_kernel(const SearchParams p) {
   const int g = i >> 3, s = i & 7;
   p.root_moves[i] = 255;
   if (s >= p.S) return;
-  if (p.r_meta[(size_t)g * 8 + 7] & 1u) return;
-  const uint64_t sv = p.r_snakes[(size_t)g * 8 + s];
-  if (!((sv >> 42) & 1ull)) return;
+  if (p.r_meta[(size_t)g * 8 + META_FLAGS] & kMetaDone) return;
+  if (!snake_alive(p.r_snakes[(size_t)g * 8 + s])) return;
   const size_t pi = ((size_t)g * p.P) * 8 + s;
   if (p.path_len[pi] == 0) return;
   const uint32_t slot = p.path_slot[pi * p.Dmax];
@@ -419,22 +410,10 @@ __global__ void search_root_kernel(const SearchParams p) {
 __global__ void stub_value_kernel(const uint64_t* keys, const float* planes, const int32_t* n_ptr, int side, int numpy1_mask, float* out) {
   const int i = (int)(blockIdx.x * blockDim.x + threadIdx.x);
   if (i >= *n_ptr) return;
-  const uint64_t k1 = keys[2 * (size_t)i + 1];
-  const int N = 2 * side - 1, c = side - 1;
-  const float* pl = planes + (size_t)i * N * N * 3;
+  const int N = 2 * side - 1;
   float v[3];
-#pragma unroll
-  for (int k = 0; k < 3; ++k) v[k] = ((float)(uint32_t)((k1 >> (16 * k)) & 0xFFFFull) - 32767.5f) * (1.0f / 32768.0f);
-  const float b0 = pl[((size_t)c * N + (c - 1)) * 3 + 1], b1 = pl[((size_t)(c - 1) * N + c) * 3 + 1], b2 = pl[((size_t)c * N + (c + 1)) * 3 + 1];
-  if (numpy1_mask) {
-    if ((double)b0 >= 0.04) v[0] = -1.0f;
-    if ((double)b1 >= 0.04) v[1] = -1.0f;
-    if ((double)b2 >= 0.04) v[2] = -1.0f;
-  } else {
-    if (b0 >= 0.04f) v[0] = -1.0f;
-    if (b1 >= 0.04f) v[1] = -1.0f;
-    if (b2 >= 0.04f) v[2] = -1.0f;
-  }
+  stub_value3(keys[2 * (size_t)i + 1], v);
+  obstacle_mask3(planes + (size_t)i * N * N * 3, side, numpy1_mask, v);
   out[3 * (size_t)i] = v[0]; out[3 * (size_t)i + 1] = v[1]; out[3 * (size_t)i + 2] = v[2];
 }
 
@@ -442,14 +421,8 @@ __global__ void stub_value_kernel(const uint64_t* keys, const float* planes, con
 __global__ void obstacle_mask_kernel(const float* planes, int n, int side, int numpy1_mask, float* v) {
   const int i = (int)(blockIdx.x * blockDim.x + threadIdx.x);
   if (i >= n) return;
-  const int N = 2 * side - 1, c = side - 1;
-  const float* pl = planes + (size_t)i * N * N * 3;
-  const float b[3] = {pl[((size_t)c * N + (c - 1)) * 3 + 1], pl[((size_t)(c - 1) * N + c) * 3 + 1], pl[((size_t)c * N + (c + 1)) * 3 + 1]};
-#pragma unroll
-  for (int k = 0; k < 3; ++k) {
-    const bool obs = numpy1_mask ? ((double)b[k] >= 0.04) : (b[k] >= 0.04f);
-    if (obs) v[3 * (size_t)i + k] = -1.0f;
-  }
+  const int N = 2 * side - 1;
+  obstacle_mask3(planes + (size_t)i * N * N * 3, side, numpy1_mask, v + 3 * (size_t)i);
 }
 
 // test hook: softermax + inverse-CDF draw + argmaxs on arbitrary rows (agent.py:114-137, numpy.random.choice)
@@ -785,28 +758,10 @@ int asz_search_finish(asz_engine* e, const uint8_t* d_root_trace, float* d_root_
   return ASZ_OK;
 }
 
-// Whole root-turn search with the stub value function, no host synchronisation inside the epoch/step loops.
-int asz_search_run_stub(asz_engine* e, uint8_t* d_trace, int32_t trace_mode, const uint8_t* d_root_trace, void* stream) {
-  int rc = asz_search_begin(e, stream);
-  if (rc != ASZ_OK) return rc;
-  SearchState* s = e->search;
-  for (int ep = 0; ep < s->E; ++ep) {
-    if ((rc = asz_search_epoch_begin(e, stream)) != ASZ_OK) return rc;
-    for (int st = 1; st <= s->Dmax + 1; ++st) {
-      if ((rc = asz_search_step_probe(e, nullptr, stream)) != ASZ_OK) return rc;
-      if (st <= s->Dmax) {
-        if ((rc = asz_search_stub_values(e, stream)) != ASZ_OK) return rc;
-        if ((rc = asz_search_step_sample(e, nullptr, d_trace, trace_mode, stream)) != ASZ_OK) return rc;
-      }
-    }
-  }
-  return asz_search_finish(e, d_root_trace, nullptr, nullptr, stream);
-}
-
-// Whole root-turn search with the hand-written value network: the epoch / step loops of Agent.make_moves (agent.py:37-58)
-// run here in native code; the only host synchronisation is the miss count of each step (it sizes the network batch).
-int asz_search_run_net(asz_engine* e, asz_net* net, uint8_t* d_trace, int32_t trace_mode, const uint8_t* d_root_trace, void* stream) {
-  if (!net) { set_error("asz_search_run_net: null network"); return ASZ_ERR_ARG; }
+// Whole root-turn search: the epoch / step loops of Agent.make_moves (agent.py:37-58) in native code.  net == nullptr: the stub
+// value function, with no host synchronisation inside the loops.  Otherwise the hand-written value network; the only host
+// synchronisation is the miss count of each step (it sizes the network batch).
+static int search_run(asz_engine* e, asz_net* net, uint8_t* d_trace, int32_t trace_mode, const uint8_t* d_root_trace, void* stream) {
   int rc = asz_search_begin(e, stream);
   if (rc != ASZ_OK) return rc;
   SearchState* s = e->search;
@@ -814,9 +769,11 @@ int asz_search_run_net(asz_engine* e, asz_net* net, uint8_t* d_trace, int32_t tr
     if ((rc = asz_search_epoch_begin(e, stream)) != ASZ_OK) return rc;
     for (int st = 1; st <= s->Dmax + 1; ++st) {
       int32_t n_miss = 0;
-      if ((rc = asz_search_step_probe(e, &n_miss, stream)) != ASZ_OK) return rc;
+      if ((rc = asz_search_step_probe(e, net ? &n_miss : nullptr, stream)) != ASZ_OK) return rc;
       if (st <= s->Dmax) {
-        if (n_miss > 0) {
+        if (!net) {
+          if ((rc = asz_search_stub_values(e, stream)) != ASZ_OK) return rc;
+        } else if (n_miss > 0) {
           if ((rc = asz_net_forward(net, s->eval_planes, n_miss, s->eval_values, stream)) != ASZ_OK) return rc;   // alpha_nnet.py:62
           if ((rc = asz_obstacle_mask(e, s->eval_planes, n_miss, s->eval_values, stream)) != ASZ_OK) return rc;   // alpha_nnet.py:63-76
         }
@@ -825,6 +782,15 @@ int asz_search_run_net(asz_engine* e, asz_net* net, uint8_t* d_trace, int32_t tr
     }
   }
   return asz_search_finish(e, d_root_trace, nullptr, nullptr, stream);
+}
+
+int asz_search_run_stub(asz_engine* e, uint8_t* d_trace, int32_t trace_mode, const uint8_t* d_root_trace, void* stream) {
+  return search_run(e, nullptr, d_trace, trace_mode, d_root_trace, stream);
+}
+
+int asz_search_run_net(asz_engine* e, asz_net* net, uint8_t* d_trace, int32_t trace_mode, const uint8_t* d_root_trace, void* stream) {
+  if (!net) { set_error("asz_search_run_net: null network"); return ASZ_ERR_ARG; }
+  return search_run(e, net, d_trace, trace_mode, d_root_trace, stream);
 }
 
 int asz_search_clear(asz_engine* e, void* stream) {

@@ -11,8 +11,8 @@
 #include <cstdio>
 #include <cstring>
 
-#include "asz_common.cuh"
 #include "asz_engine.hpp"
+#include "asz_game.cuh"
 
 namespace asz {
 
@@ -63,7 +63,7 @@ __global__ void pit_begin_kernel(const PitParams p) {
   const int g = (int)(blockIdx.x * blockDim.x + threadIdx.x);
   bool run = false;
   if (g < p.G) {
-    run = !(p.meta[(size_t)g * 8 + 7] & 1u);
+    run = !(p.meta[(size_t)g * 8 + META_FLAGS] & kMetaDone);
     p.running[g] = run ? 1 : 0;
     p.winner[g] = -1;
     p.decided[g] = run ? -1 : 0;
@@ -138,7 +138,7 @@ __global__ void pit_gather_kernel(const PitParams p, int n) {
 }
 
 // one thread per team-buffer row: the side's values (network outputs or the stand-in's key bits), AlphaNNet.v's obstacle mask
-// (alpha_nnet.py:63-76, the same compare as obstacle_mask_kernel), Agent.argmaxs (pit_agent.py:16-23), the move into its slot
+// (alpha_nnet.py:63-76), Agent.argmaxs (pit_agent.py:16-23), the move into its slot
 __global__ void pit_policy_kernel(const PitParams p, int n) {
   const int i = (int)(blockIdx.x * blockDim.x + threadIdx.x);
   if (i >= n) return;
@@ -147,18 +147,9 @@ __global__ void pit_policy_kernel(const PitParams p, int n) {
   if (word < 0) {
     v[0] = p.values[3 * (size_t)i]; v[1] = p.values[3 * (size_t)i + 1]; v[2] = p.values[3 * (size_t)i + 2];
   } else {
-    const uint64_t k = p.keys[2 * (size_t)p.src_of_dst[i] + word];
-#pragma unroll
-    for (int a = 0; a < 3; ++a) v[a] = ((float)(uint32_t)((k >> (16 * a)) & 0xFFFFull) - 32767.5f) * (1.0f / 32768.0f);
+    stub_value3(p.keys[2 * (size_t)p.src_of_dst[i] + word], v);
   }
-  const int N = 2 * p.side - 1, c = p.side - 1;
-  const float* pl = p.team + (size_t)i * p.pitch;
-  const float b[3] = {pl[((size_t)c * N + (c - 1)) * 3 + 1], pl[((size_t)(c - 1) * N + c) * 3 + 1], pl[((size_t)c * N + (c + 1)) * 3 + 1]};
-#pragma unroll
-  for (int a = 0; a < 3; ++a) {
-    const bool obs = p.numpy1_mask ? ((double)b[a] >= 0.04) : (b[a] >= 0.04f);
-    if (obs) v[a] = -1.0f;
-  }
+  obstacle_mask3(p.team + (size_t)i * p.pitch, p.side, p.numpy1_mask, v);
   const uint8_t mv = (uint8_t)argmax3(v);
   const int slot = p.slot_of_dst[i];
   p.actions[slot] = mv;
@@ -185,7 +176,7 @@ __global__ void pit_referee_kernel(const PitParams p) {
     } else {                               // :49-60 a team without live snakes: the lowest live id wins
       unsigned live = 0;
       for (int s = 0; s < p.S; ++s)
-        if ((p.snakes[(size_t)g * 8 + s] >> 42) & 1ull) live |= 1u << s;
+        if (snake_alive(p.snakes[(size_t)g * 8 + s])) live |= 1u << s;
       const unsigned amask = (1u << p.alice) - 1u;
       if (!(live & amask) || !(live & ~amask)) { done = true; w = live ? __ffs(live) - 1 : -1; }
     }
