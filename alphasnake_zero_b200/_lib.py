@@ -101,6 +101,9 @@ SYMBOLS = [
     ("asz_pit_finish", C.c_int, [_vp, _vp, _vp, _vp, _vp]),
     ("asz_pit_run", C.c_int, [_vp, C.POINTER(PitPlayer), C.POINTER(PitPlayer), _i32, _i32, _vp, _vp, _vp, _vp]),
     ("asz_pit_stats", C.c_int, [_vp, _vp]),
+    ("asz_copy_root_games", C.c_int, [_vp, _vp, _vp, _vp]),
+    ("asz_pit_set_search", C.c_int, [_vp, _i32, _vp]),
+    ("asz_pit_search_stats", C.c_int, [_vp, _vp]),
 ]
 
 

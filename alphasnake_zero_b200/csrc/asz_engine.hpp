@@ -95,6 +95,7 @@ struct asz_engine {
   asz::SearchState* search = nullptr;
   asz::RecordStore* records = nullptr;   // device-resident training records (asz_records_*)
   asz::PitState* pit = nullptr;          // two-network match (asz_pit_*), allocated by the first asz_pit_begin
+  asz_engine* pit_searcher[2] = {nullptr, nullptr};   // asz_pit_set_search: the search engine of Alice / Bob, not owned
 };
 
 namespace asz {
@@ -102,6 +103,8 @@ int gameset_alloc(GameSet& gs, int n, int pc);
 void gameset_free(GameSet& gs);
 int search_create(asz_engine* e);
 void search_destroy(asz_engine* e);
+// stand-in value function of asz_search_stub_values: which word of the plane key it reads (1 unless a pit side says otherwise)
+void search_set_stub_word(asz_engine* e, int word);
 void records_destroy(asz_engine* e);
 void pit_destroy(asz_engine* e);
 void host_pipe_destroy(asz_engine* e);

@@ -68,6 +68,7 @@ struct SearchState {
   float* root_q = nullptr;        // [G*8*3]
   uint8_t* root_moves = nullptr;  // [G*8]
   uint32_t root_turn = 0;         // current root turn (1-based while a search is open)
+  int stub_word = 1;              // word of the plane key the stand-in value function reads (a pit's stand-in side may pick 0)
   int epoch = -1, step = 0;
   bool open = false;
   // host copies of stats[ST_OCCUPIED], stats[ST_OVERFLOW] (refreshed wherever the host synchronises anyway)
@@ -407,12 +408,13 @@ __global__ void search_root_kernel(const SearchParams p) {
 
 // deterministic stand-in for the value network: value from the plane key, then AlphaNNet.v's obstacle mask
 // (alpha_nnet.py:63-76).  Used by the parity tests and the search-only throughput measurement.
-__global__ void stub_value_kernel(const uint64_t* keys, const float* planes, const int32_t* n_ptr, int side, int numpy1_mask, float* out) {
+__global__ void stub_value_kernel(const uint64_t* keys, int word, const float* planes, const int32_t* n_ptr, int side, int numpy1_mask,
+                                  float* out) {
   const int i = (int)(blockIdx.x * blockDim.x + threadIdx.x);
   if (i >= *n_ptr) return;
   const int N = 2 * side - 1;
   float v[3];
-  stub_value3(keys[2 * (size_t)i + 1], v);
+  stub_value3(keys[2 * (size_t)i + word], v);
   obstacle_mask3(planes + (size_t)i * N * N * 3, side, numpy1_mask, v);
   out[3 * (size_t)i] = v[0]; out[3 * (size_t)i + 1] = v[1]; out[3 * (size_t)i + 2] = v[2];
 }
@@ -537,6 +539,8 @@ int search_create(asz_engine* e) {
   ASZ_CUDA(cudaMemset(s->root_q, 0, (size_t)c.games * 8 * 3 * sizeof(float)));
   return ASZ_OK;
 }
+
+void search_set_stub_word(asz_engine* e, int word) { e->search->stub_word = word; }
 
 void search_destroy(asz_engine* e) {
   SearchState* s = e->search;
@@ -701,8 +705,8 @@ int asz_search_stub_values(asz_engine* e, void* stream) {
   DeviceGuard guard(e->device);
   SearchState* s = e->search;
   const int n = s->max_rows;   // the kernel reads the live count from device memory: no host sync
-  stub_value_kernel<<<(n + 127) / 128, 128, 0, (cudaStream_t)stream>>>(s->eval_keys, s->eval_planes, s->n_miss, e->cfg.side,
-                                                                      e->cfg.numpy1_mask, s->eval_values);
+  stub_value_kernel<<<(n + 127) / 128, 128, 0, (cudaStream_t)stream>>>(s->eval_keys, s->stub_word, s->eval_planes, s->n_miss,
+                                                                      e->cfg.side, e->cfg.numpy1_mask, s->eval_values);
   return cuda_ok(cudaGetLastError(), "stub_value_kernel") ? ASZ_OK : ASZ_ERR_CUDA;
 }
 

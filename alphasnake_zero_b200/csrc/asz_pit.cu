@@ -7,9 +7,16 @@
 //   pit_mp_game_runner.py:44-60  winner bookkeeping, early exit       pit_referee_kernel
 // The host waits once per turn, for one 12-byte line: the row counts of the two teams (they size the forwards) and the number of
 // games still running.
+// A side with a searcher engine attached (asz_pit_set_search) plays the search Agent instead (agent.py:25-111, training=False):
+//   asz_copy_root_games                 the running games into the searcher (the others arrive finished)   copy_root_games_kernel
+//   Agent.make_moves                    root-turn search with the side's network or stand-in              asz_search_run_net / _stub
+//   agent.py:98-99 argmaxs of root Q    the side's moves from the searcher's root moves                   pit_policy_kernel
+// A search waits on the host once per search step (asz_search_run_net), on top of the turn's one wait.
 #include <algorithm>
+#include <chrono>
 #include <cstdio>
 #include <cstring>
+#include <string>
 
 #include "asz_engine.hpp"
 #include "asz_game.cuh"
@@ -37,15 +44,18 @@ struct PitState {
   cudaEvent_t fwd_begin = nullptr, fwd_end = nullptr;
   asz_net* net[2] = {nullptr, nullptr};
   int word[2] = {-1, -1};              // stand-in key word per side, -1 = network
+  asz_engine* searcher[2] = {nullptr, nullptr};   // the match's searcher per side (asz_pit_set_search at asz_pit_begin)
   int alice = 0;
   bool open = false;
   int turn = 0;
   double n_net_rows = 0.0, n_stub_rows = 0.0, fwd_ms = 0.0;
+  double n_search_rows = 0.0, search_ms = 0.0;
 };
 
 struct PitParams {
   int G, S, rows, alice, side, pitch, numpy1_mask, nA, turn;
   int word_a, word_b;
+  const uint8_t* root_moves_a; const uint8_t* root_moves_b;   // a searched side's moves by slot, null = argmax of its values
   const uint64_t* snakes; const uint32_t* meta;
   uint8_t* running; int32_t* winner; int32_t* decided;
   uint8_t* actions; uint8_t* moves;
@@ -128,32 +138,60 @@ __global__ void __launch_bounds__(kPartThreads) pit_partition_kernel(const PitPa
   if (threadIdx.x == 0) { p.line[0] = totals[0]; p.line[1] = totals[1]; }
 }
 
-// one warp per team-buffer row: copy the plane (pitch floats, 16-byte aligned rows)
-__global__ void pit_gather_kernel(const PitParams p, int n) {
-  const int w = (int)((blockIdx.x * blockDim.x + threadIdx.x) >> 5);
-  if (w >= n) return;
+// one warp per team-buffer row of [first, first + n): copy the plane (pitch floats, 16-byte aligned rows)
+__global__ void pit_gather_kernel(const PitParams p, int first, int n) {
+  const int k = (int)((blockIdx.x * blockDim.x + threadIdx.x) >> 5);
+  if (k >= n) return;
+  const int w = first + k;
   const float4* src = reinterpret_cast<const float4*>(p.planes + (size_t)p.src_of_dst[w] * p.pitch);
   float4* dst = reinterpret_cast<float4*>(p.team + (size_t)w * p.pitch);
   for (int i = lane_id(); i < p.pitch / 4; i += 32) dst[i] = src[i];
 }
 
 // one thread per team-buffer row: the side's values (network outputs or the stand-in's key bits), AlphaNNet.v's obstacle mask
-// (alpha_nnet.py:63-76), Agent.argmaxs (pit_agent.py:16-23), the move into its slot
+// (alpha_nnet.py:63-76), Agent.argmaxs (pit_agent.py:16-23), the move into its slot.  A searched side's row takes its searcher's
+// root move instead; a row the search dropped (Q table overflow, reported as ASZ_ERR_CAPACITY) plays straight, as it does in the
+// search's own sub-games.
 __global__ void pit_policy_kernel(const PitParams p, int n) {
   const int i = (int)(blockIdx.x * blockDim.x + threadIdx.x);
   if (i >= n) return;
-  const int word = i < p.nA ? p.word_a : p.word_b;
-  float v[3];
-  if (word < 0) {
-    v[0] = p.values[3 * (size_t)i]; v[1] = p.values[3 * (size_t)i + 1]; v[2] = p.values[3 * (size_t)i + 2];
-  } else {
-    stub_value3(p.keys[2 * (size_t)p.src_of_dst[i] + word], v);
-  }
-  obstacle_mask3(p.team + (size_t)i * p.pitch, p.side, p.numpy1_mask, v);
-  const uint8_t mv = (uint8_t)argmax3(v);
   const int slot = p.slot_of_dst[i];
+  const uint8_t* root_moves = i < p.nA ? p.root_moves_a : p.root_moves_b;
+  uint8_t mv;
+  if (root_moves) {
+    mv = root_moves[slot];
+    if (mv > 2) mv = 1;
+  } else {
+    const int word = i < p.nA ? p.word_a : p.word_b;
+    float v[3];
+    if (word < 0) {
+      v[0] = p.values[3 * (size_t)i]; v[1] = p.values[3 * (size_t)i + 1]; v[2] = p.values[3 * (size_t)i + 2];
+    } else {
+      stub_value3(p.keys[2 * (size_t)p.src_of_dst[i] + word], v);
+    }
+    obstacle_mask3(p.team + (size_t)i * p.pitch, p.side, p.numpy1_mask, v);
+    mv = (uint8_t)argmax3(v);
+  }
   p.actions[slot] = mv;
   if (p.moves) p.moves[slot] = mv;
+}
+
+// asz_copy_root_games: block g copies game g's packed record (cells, snakes, meta), the block copy of search_epoch_begin_kernel.  A
+// game whose flag byte reads `skip_if_set` (nonzero / zero) arrives finished (kMetaDone), so a search on the copy leaves it alone.
+__global__ void copy_root_games_kernel(const uint16_t* __restrict__ src_cells, const uint64_t* __restrict__ src_snakes,
+                                       const uint32_t* __restrict__ src_meta, uint16_t* cells, uint64_t* snakes, uint32_t* meta, int pc,
+                                       const uint8_t* flags, int skip_if_set) {
+  const int g = (int)blockIdx.x;
+  const uint4* src = reinterpret_cast<const uint4*>(src_cells + (size_t)g * pc);   // pc is a multiple of 32 cells: 64-byte records
+  uint4* dst = reinterpret_cast<uint4*>(cells + (size_t)g * pc);
+  for (int i = (int)threadIdx.x; i < pc / 8; i += (int)blockDim.x) dst[i] = src[i];
+  if (threadIdx.x < 8) {
+    const size_t k = (size_t)g * 8 + threadIdx.x;
+    snakes[k] = src_snakes[k];
+    uint32_t m = src_meta[k];
+    if (threadIdx.x == META_FLAGS && flags && ((flags[g] != 0) == (skip_if_set != 0))) m |= kMetaDone;
+    meta[k] = m;
+  }
 }
 
 // the loop replays np.maximum(spawn_trace[turn], -1)
@@ -242,7 +280,36 @@ static PitParams make_params(asz_engine* e) {
   return p;
 }
 
-static bool stub_plays(const PitState* s) { return s->word[0] >= 0 || s->word[1] >= 0; }
+// a stand-in side without a searcher values the engine's own encode: the encode writes plane keys
+static bool stub_plays(const PitState* s) {
+  return (s->word[0] >= 0 && !s->searcher[0]) || (s->word[1] >= 0 && !s->searcher[1]);
+}
+
+static int copy_root_games(asz_engine* dst, const asz_engine* src, const uint8_t* flags, int skip_if_set, cudaStream_t st) {
+  copy_root_games_kernel<<<src->cfg.games, 64, 0, st>>>(src->root.cells, src->root.snakes, src->root.meta, dst->root.cells,
+                                                         dst->root.snakes, dst->root.meta, src->pc, flags, skip_if_set);
+  return cuda_ok(cudaGetLastError(), "copy_root_games_kernel") ? ASZ_OK : ASZ_ERR_CUDA;
+}
+
+// one searched side's turn: the running games into its searcher, the root-turn search with the side's network (or stand-in with
+// the side's key word), the root moves left in the searcher's buffer for pit_policy_kernel
+static int pit_search_side(asz_engine* e, int side, cudaStream_t st) {
+  PitState* s = e->pit;
+  asz_engine* q = s->searcher[side];
+  const auto t0 = std::chrono::steady_clock::now();
+  int rc = copy_root_games(q, e, s->running, 0, st);
+  if (rc != ASZ_OK) return rc;
+  if (s->net[side]) {
+    rc = asz_search_run_net(q, s->net[side], nullptr, 0, nullptr, st);
+  } else {
+    search_set_stub_word(q, s->word[side]);
+    rc = asz_search_run_stub(q, nullptr, 0, nullptr, st);
+    search_set_stub_word(q, 1);
+  }
+  // every search ends in a host synchronisation (asz_search_finish), so the host clock spans the device work
+  s->search_ms += std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
+  return rc;
+}
 
 // Game.tic of every unfinished game (tic) and the planes of every live snake into the engine's plane buffer
 static int pit_step(asz_engine* e, bool tic, int32_t spawn_mode, const int32_t* spawn, cudaStream_t st) {
@@ -292,6 +359,27 @@ static int check_player(const asz_engine* e, const asz_pit_player* pl, const cha
   return ASZ_OK;
 }
 
+// games of the same shape on the same device: the packed records of one engine are records of the other
+static bool same_games(const asz_engine* a, const asz_engine* b) {
+  return a->cfg.side == b->cfg.side && a->cfg.snakes == b->cfg.snakes && a->cfg.games == b->cfg.games && a->device == b->device;
+}
+
+static int check_searcher(const asz_engine* e, const asz_engine* q, const char* who) {
+  if (!q) return ASZ_OK;
+  char msg[200];
+  const char* why = nullptr;
+  if (q == e) why = "is the match's own engine";
+  else if (!q->search) why = "has no search configured (max_breadth 0)";
+  else if (q->cfg.training) why = "is a training search (a pit plays with training = 0)";
+  else if (!same_games(e, q)) why = "differs from the engine in board side, snake count, game count or device";
+  else if (q->cfg.health_dec != e->cfg.health_dec || q->cfg.numpy1_mask != e->cfg.numpy1_mask)
+    why = "differs from the engine in health_dec or numpy1_mask (its sub-games would not be the match's games)";
+  if (!why) return ASZ_OK;
+  snprintf(msg, sizeof msg, "asz_pit_begin: %s's searcher %s", who, why);
+  set_error(msg);
+  return ASZ_ERR_ARG;
+}
+
 }  // namespace asz
 
 using namespace asz;
@@ -305,17 +393,27 @@ int asz_pit_begin(asz_engine* e, const asz_pit_player* alice, const asz_pit_play
   int rc;
   if ((rc = check_player(e, alice, "Alice")) != ASZ_OK || (rc = check_player(e, bob, "Bob")) != ASZ_OK) return rc;
   if (alice_snakes < 0 || alice_snakes > e->cfg.snakes) { set_error("asz_pit_begin: alice_snakes must be in 0..S"); return ASZ_ERR_ARG; }
+  if ((rc = check_searcher(e, e->pit_searcher[0], "Alice")) != ASZ_OK || (rc = check_searcher(e, e->pit_searcher[1], "Bob")) != ASZ_OK)
+    return rc;
+  if (e->pit_searcher[0] && e->pit_searcher[0] == e->pit_searcher[1]) {
+    set_error("asz_pit_begin: one searcher is attached to both sides (each side needs its own Q table)");
+    return ASZ_ERR_ARG;
+  }
   DeviceGuard guard(e->device);
   NvtxRange nvtx("asz:pit begin");
   if ((rc = pit_create(e)) != ASZ_OK) { pit_destroy(e); return rc; }   // a later begin allocates afresh
   PitState* s = e->pit;
   s->net[0] = alice->net; s->net[1] = bob->net;
   s->word[0] = alice->net ? -1 : alice->stub_word; s->word[1] = bob->net ? -1 : bob->stub_word;
+  s->searcher[0] = e->pit_searcher[0]; s->searcher[1] = e->pit_searcher[1];
   s->alice = alice_snakes;
   s->turn = 0;
   s->n_net_rows = s->n_stub_rows = s->fwd_ms = 0.0;
+  s->n_search_rows = s->search_ms = 0.0;
   if (stub_plays(s) && !s->keys) ASZ_CUDA(cudaMalloc(&s->keys, (size_t)s->rows * 2 * sizeof(uint64_t)));
   cudaStream_t st = (cudaStream_t)stream;
+  for (int side = 0; side < 2; ++side)   // Agent.clear (agent.py:140-147): a match does not depend on earlier matches
+    if (s->searcher[side] && (rc = asz_search_clear(s->searcher[side], stream)) != ASZ_OK) return rc;
   ASZ_CUDA(cudaMemsetAsync(s->line, 0, 4 * sizeof(int32_t), st));
   const PitParams p = make_params(e);
   pit_begin_kernel<<<(s->G + 255) / 256, 256, 0, st>>>(p);
@@ -345,24 +443,40 @@ int asz_pit_turn(asz_engine* e, int32_t spawn_mode, const int32_t* d_spawn_cells
   PitParams p = make_params(e);
   p.nA = nA; p.moves = d_moves;
   int rc;
+  int overflow = ASZ_OK;           // a searcher's Q table overflowed: the turn is played out, then reported
+  std::string overflow_msg;
   bool timed = false;
   if (n > 0) {
-    pit_gather_kernel<<<(n + 7) / 8, 256, 0, st>>>(p, n);
-    if (!cuda_ok(cudaGetLastError(), "pit_gather_kernel")) return ASZ_ERR_CUDA;
-    // pit_agent.py:11 nnet.v(states): one forward per side, or one over both segments when the sides share a network
     const int seg_begin[2] = {0, nA}, seg_len[2] = {nA, nB};
-    const bool shared = s->net[0] && s->net[0] == s->net[1];
-    timed = (s->net[0] && nA > 0) || (s->net[1] && nB > 0);
+    const bool searched[2] = {s->searcher[0] != nullptr, s->searcher[1] != nullptr};
+    for (int side = 0; side < 2; ++side) {
+      if (!searched[side] || seg_len[side] == 0) continue;   // a side with no snake to move does not search
+      rc = pit_search_side(e, side, st);
+      if (rc == ASZ_ERR_CAPACITY) { overflow = rc; overflow_msg = asz_last_error(); }
+      else if (rc != ASZ_OK) return rc;
+      (side == 0 ? p.root_moves_a : p.root_moves_b) = asz_search_root_moves(s->searcher[side]);
+      s->n_search_rows += seg_len[side];
+    }
+    // the rows the sides without a searcher value: Alice's segment, Bob's, or both (contiguous either way)
+    const int g0 = searched[0] ? nA : 0, g1 = searched[1] ? nA : n;
+    if (g1 > g0) {
+      pit_gather_kernel<<<(g1 - g0 + 7) / 8, 256, 0, st>>>(p, g0, g1 - g0);
+      if (!cuda_ok(cudaGetLastError(), "pit_gather_kernel")) return ASZ_ERR_CUDA;
+    }
+    // pit_agent.py:11 nnet.v(states): one forward per side, or one over both segments when the sides share a network
+    const bool shared = s->net[0] && s->net[0] == s->net[1] && !searched[0] && !searched[1];
+    timed = (s->net[0] && !searched[0] && nA > 0) || (s->net[1] && !searched[1] && nB > 0);
     if (timed) ASZ_CUDA(cudaEventRecord(s->fwd_begin, st));
     for (int side = 0; side < (shared ? 1 : 2); ++side) {
       const int begin = seg_begin[side], len = shared ? n : seg_len[side];
-      if (!s->net[side] || len == 0) continue;
+      if (!s->net[side] || searched[side] || len == 0) continue;
       if ((rc = asz_net_forward_pitched(s->net[side], s->team + (size_t)begin * e->pitch, e->pitch, len, s->values + (size_t)begin * 3,
                                         stream)) != ASZ_OK)
         return rc;
     }
     if (timed) ASZ_CUDA(cudaEventRecord(s->fwd_end, st));
-    for (int side = 0; side < 2; ++side) (s->net[side] ? s->n_net_rows : s->n_stub_rows) += seg_len[side];
+    for (int side = 0; side < 2; ++side)
+      if (!searched[side]) (s->net[side] ? s->n_net_rows : s->n_stub_rows) += seg_len[side];
     pit_policy_kernel<<<(n + 127) / 128, 128, 0, st>>>(p, n);
     if (!cuda_ok(cudaGetLastError(), "pit_policy_kernel")) return ASZ_ERR_CUDA;
   }
@@ -385,7 +499,8 @@ int asz_pit_turn(asz_engine* e, int32_t spawn_mode, const int32_t* d_spawn_cells
     s->fwd_ms += ms;
   }
   if (h_running) *h_running = s->h_line[2];
-  return ASZ_OK;
+  if (overflow != ASZ_OK) set_error(overflow_msg);
+  return overflow;
 }
 
 int asz_pit_finish(asz_engine* e, int32_t* d_winners, int32_t* d_decided_turn, int32_t* h_turns, void* stream) {
@@ -417,7 +532,15 @@ int asz_pit_run(asz_engine* e, const asz_pit_player* alice, const asz_pit_player
   int rc = asz_pit_begin(e, alice, bob, alice_snakes, &running, stream);
   if (rc != ASZ_OK) return rc;
   for (int t = 0; running > 0 && (max_turns == 0 || t < max_turns); ++t) {
-    if ((rc = asz_pit_turn(e, ASZ_SPAWN_NATIVE, nullptr, nullptr, &running, stream)) != ASZ_OK) {
+    rc = asz_pit_turn(e, ASZ_SPAWN_NATIVE, nullptr, nullptr, &running, stream);
+    if (rc == ASZ_ERR_CAPACITY) {     // a searcher's table overflowed: the match stops with the results so far written
+      const std::string msg = asz_last_error();
+      const int frc = asz_pit_finish(e, d_winners, d_decided_turn, h_turns, stream);
+      if (frc != ASZ_OK && frc != ASZ_ERR_STATE) return frc;
+      set_error(msg);
+      return rc;
+    }
+    if (rc != ASZ_OK) {
       e->pit->open = false;           // the match is over either way; ASZ_ERR_STATE stays reserved for "results written"
       return rc;
     }
@@ -431,6 +554,31 @@ int asz_pit_stats(asz_engine* e, double* h_stats) {
   h_stats[0] = s ? s->turn : 0; h_stats[1] = s ? s->n_net_rows : 0.0; h_stats[2] = s ? s->n_stub_rows : 0.0;
   h_stats[3] = s ? s->fwd_ms : 0.0;
   return ASZ_OK;
+}
+
+int asz_pit_search_stats(asz_engine* e, double* h_stats) {
+  if (!e || !h_stats) { set_error("null argument"); return ASZ_ERR_ARG; }
+  const PitState* s = e->pit;
+  h_stats[0] = s ? s->n_search_rows : 0.0; h_stats[1] = s ? s->search_ms : 0.0;
+  return ASZ_OK;
+}
+
+int asz_pit_set_search(asz_engine* e, int32_t side, asz_engine* searcher) {
+  if (!e) { set_error("null engine"); return ASZ_ERR_ARG; }
+  if (side != 0 && side != 1) { set_error("asz_pit_set_search: side must be 0 (Alice) or 1 (Bob)"); return ASZ_ERR_ARG; }
+  e->pit_searcher[side] = searcher;   // checked against the engine by asz_pit_begin
+  return ASZ_OK;
+}
+
+int asz_copy_root_games(asz_engine* dst, const asz_engine* src, const uint8_t* d_skip, void* stream) {
+  if (!dst || !src) { set_error("null engine"); return ASZ_ERR_ARG; }
+  if (!same_games(dst, src)) {
+    set_error("asz_copy_root_games: the engines differ in board side, snake count, game count or device");
+    return ASZ_ERR_ARG;
+  }
+  if (dst == src) { set_error("asz_copy_root_games: an engine cannot be copied onto itself"); return ASZ_ERR_ARG; }
+  DeviceGuard guard(dst->device);
+  return copy_root_games(dst, src, d_skip, 1, (cudaStream_t)stream);
 }
 
 }  // extern "C"

@@ -50,6 +50,7 @@ class Engine:
         self.rewards = torch.zeros(games, 8, dtype=torch.int8, device=dev)
         self.keys = None
         self._pit_open = False
+        self._pit_searchers = [None, None]     # attached searcher engines, kept alive while attached
 
     def close(self):
         if getattr(self, "h", None):
@@ -308,12 +309,13 @@ class Engine:
         return running.value
 
     def _pit_results(self, rc_of, written_on_state):
-        """written_on_state: ASZ_ERR_STATE from this call means 'games still running, results so far written'"""
+        """written_on_state: ASZ_ERR_STATE from this call means 'games still running, results so far written' (and so does
+        ASZ_ERR_CAPACITY, a searcher's Q table overflow, from asz_pit_run)"""
         winners = torch.empty(self.G, dtype=torch.int32, device=self.device)
         decided = torch.empty(self.G, dtype=torch.int32, device=self.device)
         turns = C.c_int32(0)
         rc = rc_of(_ptr(winners), _ptr(decided), C.byref(turns))
-        if rc != 0 and not (rc == _lib.ASZ_ERR_STATE and written_on_state):
+        if rc != 0 and not (rc in (_lib.ASZ_ERR_STATE, _lib.ASZ_ERR_CAPACITY) and written_on_state):
             check(rc)                     # nothing was written
         res = (winners.cpu().numpy(), decided.cpu().numpy(), turns.value)
         if rc != 0:
@@ -339,7 +341,24 @@ class Engine:
     def pit_stats(self):
         s = np.zeros(4, np.float64)
         check(self.L.asz_pit_stats(self.h, _np(s)))
-        return dict(turns=int(s[0]), net_rows=int(s[1]), stub_rows=int(s[2]), forward_ms=float(s[3]))
+        r = np.zeros(2, np.float64)
+        check(self.L.asz_pit_search_stats(self.h, _np(r)))
+        return dict(turns=int(s[0]), net_rows=int(s[1]), stub_rows=int(s[2]), forward_ms=float(s[3]), search_rows=int(r[0]),
+                    search_ms=float(r[1]))
+
+    def pit_set_search(self, side, searcher):
+        """asz_pit_set_search: `searcher` (an Engine with search configured and training=False, or None to detach) plays side 0
+        (Alice) or 1 (Bob) of the next pit_begin / pit_run as the search Agent, valued by that side's player (its network, or
+        the stand-in reading key word 0 / 1)."""
+        check(self.L.asz_pit_set_search(self.h, int(side), searcher.h if searcher is not None else None))
+        self._pit_searchers[int(side)] = searcher
+
+    def copy_root_games_from(self, src, skip=None):
+        """asz_copy_root_games: this engine's root games become copies of `src`'s (same board side, snake count, game count and
+        device); skip: bool / uint8 cuda tensor [G], games where it is set arrive finished, so a search here leaves them alone."""
+        if skip is not None:
+            skip = skip.to(device=self.device, dtype=torch.uint8).contiguous()
+        check(self.L.asz_copy_root_games(self.h, src.h, _ptr(skip), self.stream))
 
     # ---- helpers for the drop-in classes ---------------------------------------------------------------------------
     def alive_mask(self):

@@ -74,12 +74,7 @@ class Agent:
         if eng is None:
             raise TypeError("Agent.make_moves needs the games of an engine-backed MPGameRunner (no CPU path)")
         self._engine = eng
-        value_fn = native = None
-        if self.nnet is not None and not getattr(self.nnet, "is_stub", False):
-            if getattr(self.nnet, "backend", "native") == "torch":
-                value_fn = self.nnet.v_device          # explicit PyTorch reference network: Python-driven loop
-            else:
-                native = self.nnet._get_native()       # product path: the whole root turn in one native call
+        value_fn, native = self.search_values()
         q, mv = eng.search(value_fn=value_fn, net=native)
         mvh = mv.cpu().numpy()                         # the only per-turn device -> host traffic: G x 8 bytes of moves
         moves = [int(mvh[g, s]) for g, s in ids]
@@ -103,6 +98,15 @@ class Agent:
                 self.records.append(ph[row_of[(g, s)]])
                 self.values.append(qh[g, s].copy())
         return moves
+
+    def search_values(self):
+        """(value_fn, native network) of Engine.search for this agent's network: both None for no network or a StubNet (the
+        engine's stub value function)."""
+        if self.nnet is None or getattr(self.nnet, "is_stub", False):
+            return None, None
+        if getattr(self.nnet, "backend", "native") == "torch":
+            return self.nnet.v_device, None            # explicit PyTorch reference network: Python-driven loop
+        return None, self.nnet._get_native()           # product path: the whole root turn in one native call
 
     # agent.py:114-122 (host restatement for callers that use it directly)
     def softermax(self, z):

@@ -286,7 +286,8 @@ int asz_net_forward_pitched(asz_net* net, const float* d_planes, int32_t plane_p
 int asz_net_debug_layer(asz_net* net, const float* d_planes, int32_t count, int32_t layer, float* d_act, void* stream);
 
 /* ---- pit: pit_mp_game_runner.MPGameRunner.run(Alice, Bob, Alice_snake_cnt) (pit_mp_game_runner.py:14-63) with
- * pit_agent.Agent (pit_agent.py:10-28) on both sides, played on the engine's root games without planes through the host -----
+ * pit_agent.Agent (pit_agent.py:10-28) on both sides, played on the engine's root games without planes through the host (either
+ * side may play the search Agent instead: asz_pit_set_search below) --------------------------------------------------------
  * Snakes with id < alice_snakes are Alice's, the others Bob's.  One turn: the rows of the running games are gathered into one
  * team buffer (Alice's, then Bob's, each in (game, snake) order), each side's network values its segment (one forward when
  * both sides share a network), AlphaNNet.v's obstacle mask and Agent.argmaxs pick the moves (every other slot plays 1, as in
@@ -300,7 +301,8 @@ int asz_net_debug_layer(asz_net* net, const float* d_planes, int32_t count, int3
 typedef struct {
   asz_net* net;          /* the side's value network (same board side and device as the engine), or NULL = stand-in player */
   int32_t stub_word;     /* net == NULL: value of move a = 16 bits (16a..16a+15) of word stub_word (0 or 1) of the plane key,
-                            mapped to [-1, 1) (asz_search_stub_values uses word 1), then the obstacle mask */
+                            mapped to [-1, 1) (asz_search_stub_values uses word 1, a searched stand-in side this word),
+                            then the obstacle mask */
 } asz_pit_player;
 /* starts a match on the current root games (encodes their planes; ASZ_STEP_KEYS when a stand-in plays) and synchronises;
  * *h_running (may be NULL) = games running.  ASZ_ERR_ARG: a network of another board side or device, alice_snakes outside
@@ -323,6 +325,28 @@ int asz_pit_run(asz_engine* e, const asz_pit_player* alice, const asz_pit_player
 /* counters of the current or last match: h_stats[4] = turns, rows valued by a network, rows valued by a stand-in player,
  * milliseconds of the network forwards (CUDA events around each turn's forwards) */
 int asz_pit_stats(asz_engine* e, double* h_stats);
+
+/* ---- pit with search agents: either side plays utils/agent.Agent (agent.py:25-111) with training=False --------------------
+ * A searched side's turn: the match's running games are copied into the side's searcher engine (the others arrive finished,
+ * so the search leaves them alone), one root-turn search runs on it with the side's network (asz_search_run_net) or, for a
+ * stand-in side, the stub value function reading key word stub_word, and the side's snakes play the argmaxs of their root Q
+ * (the searcher's root moves).  Every snake inside that search is modelled with the side's network; the other side's moves
+ * from it are discarded.  The rest of the turn is the pit above.  asz_pit_begin clears both searchers' tables; across the
+ * turns of a match a table ages and evicts as agent.py:30-31, 101-110.  A side without a searcher plays argmax as before.
+ * A searcher's Q table overflow is ASZ_ERR_CAPACITY from asz_pit_turn after the turn is played (a row the search dropped
+ * moves straight) and from asz_pit_run after the results so far are written. */
+/* copies the packed root records (cells, snakes, meta) of src into dst on their device; a game with d_skip[g] != 0
+ * (DEVICE [G], may be NULL) arrives with its finished flag set.  ASZ_ERR_ARG: board side, snake count, game count or
+ * device differ, or dst == src. */
+int asz_copy_root_games(asz_engine* dst, const asz_engine* src, const uint8_t* d_skip, void* stream);
+/* attaches (searcher != NULL) or detaches the searcher of side 0 (Alice) or 1 (Bob) for e's next asz_pit_begin / asz_pit_run.
+ * A searcher is an engine with search configured (max_depth / max_breadth / softmax_base of the side's Agent), training = 0, and
+ * the board side, snake count, game count, device, health_dec and numpy1_mask of e; it must stay alive while attached.
+ * asz_pit_begin refuses (ASZ_ERR_ARG) a searcher that does not match, e itself, and one searcher on both sides. */
+int asz_pit_set_search(asz_engine* e, int32_t side, asz_engine* searcher);
+/* counters of the current or last match: h_stats[2] = rows moved by a search, milliseconds of the searched sides' copies
+ * and searches (host clock; each search ends in a host synchronisation) */
+int asz_pit_search_stats(asz_engine* e, double* h_stats);
 
 #ifdef __cplusplus
 }
