@@ -51,8 +51,13 @@ __global__ void __launch_bounds__(256) records_gather_kernel(const float* __rest
   const int plane = N * N * 3;
   float* x0 = X + (size_t)i * plane;
   float* x1 = X + (size_t)(n + i) * plane;
-  if (r < 0 || r >= count) {            // out-of-range index: an all-NaN record is easier to notice than a silent zero
-    for (int e = (int)threadIdx.x; e < plane; e += (int)blockDim.x) { x0[e] = __int_as_float(0x7fc00000); if (mirror) x1[e] = __int_as_float(0x7fc00000); }
+  if (r < 0 || r >= count) {            // out-of-range index: an all-NaN record (planes and values) is easier to notice than a silent zero
+    const float nan = __int_as_float(0x7fc00000);
+    for (int e = (int)threadIdx.x; e < plane; e += (int)blockDim.x) { x0[e] = nan; if (mirror) x1[e] = nan; }
+    if (threadIdx.x < 3) {
+      V[3 * (size_t)i + threadIdx.x] = nan;
+      if (mirror) V[3 * (size_t)(n + i) + threadIdx.x] = nan;
+    }
     return;
   }
   const float* src = planes + (size_t)r * pitch;
