@@ -439,6 +439,54 @@ void oenv_run(ogame **games, int G, int H, int W, int S, int health_dec, uint32_
   free(jobs); free(th);
 }
 
+/* batch encode: every live snake's og_make_state plane of G games, dense rows in (game, snake id) order */
+typedef struct {
+  ogame **games; int g0, g1; const int *row0; float *planes; int32_t *ids; size_t plen;
+} oenc_job;
+
+static void *oenc_worker(void *arg) {
+  const oenc_job *jb = (const oenc_job *)arg;
+  for (int gi = jb->g0; gi < jb->g1; ++gi) {
+    const ogame *g = jb->games[gi];
+    if (!g) continue;
+    for (int k = 0; k < g->n_live; ++k) {   /* the live list is in ascending snake id */
+      const size_t r = (size_t)jb->row0[gi] + (size_t)k;
+      og_make_state(g, k, jb->planes + r * jb->plen);
+      jb->ids[r] = (int32_t)(gi * 8 + g->live[k]);
+    }
+  }
+  return NULL;
+}
+
+int oenv_encode(ogame **games, int G, int n_threads, float *planes, int32_t *ids) {
+  int *row0 = (int *)malloc(sizeof(int) * (size_t)(G > 0 ? G : 1));
+  int n = 0;
+  size_t plen = 0;
+  for (int gi = 0; gi < G; ++gi) {
+    row0[gi] = n;
+    if (!games[gi]) continue;
+    n += games[gi]->n_live;
+    plen = (size_t)3 * (2 * games[gi]->H - 1) * (2 * games[gi]->W - 1);
+  }
+  if (planes && ids && n > 0) {
+    if (n_threads < 1) n_threads = 1;
+    if (n_threads > G) n_threads = G;
+    oenc_job *jobs = (oenc_job *)calloc((size_t)n_threads, sizeof(oenc_job));
+    pthread_t *th = (pthread_t *)calloc((size_t)n_threads, sizeof(pthread_t));
+    for (int t = 0; t < n_threads; ++t) {
+      oenc_job *jb = &jobs[t];
+      jb->games = games; jb->g0 = (int)((long long)G * t / n_threads); jb->g1 = (int)((long long)G * (t + 1) / n_threads);
+      jb->row0 = row0; jb->planes = planes; jb->ids = ids; jb->plen = plen;
+      if (t > 0) pthread_create(&th[t], NULL, oenc_worker, jb);
+    }
+    oenc_worker(&jobs[0]);
+    for (int t = 1; t < n_threads; ++t) pthread_join(th[t], NULL);
+    free(jobs); free(th);
+  }
+  free(row0);
+  return n;
+}
+
 /* ------------------------------------------------------------------------ */
 /* softermax / argmaxs / choice                                               */
 /* ------------------------------------------------------------------------ */

@@ -74,6 +74,10 @@ typedef struct {
  * allocate internally and discard).  encode != 0 => every live snake's plane is produced each tic. */
 void oenv_run(ogame **games, int G, int H, int W, int S, int health_dec, uint32_t chance_thresh, uint64_t seed,
               int tics, int encode, int n_threads, oenv_stats *stats);
+/* og_make_state of every live snake of G games, dense rows of (2H-1)*(2W-1)*3 floats in (game, snake id) order, with
+ * ids[r] = game * 8 + snake id; games share one shape.  A NULL entry of games emits no rows (a finished game that was not
+ * restarted).  Threads split the games.  planes / ids NULL: rows are only counted.  Returns the number of rows. */
+int oenv_encode(ogame **games, int G, int n_threads, float *planes, int32_t *ids);
 
 /* --- search (agent.py + mp_game_runner.py:79-115) -------------------------- */
 typedef struct oagent oagent;

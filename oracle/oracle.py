@@ -61,6 +61,7 @@ def lib():
         L.og_stub_value.argtypes = [vp, vp]
         L.og_obstacle_mask.argtypes = [vp, i32, i32, vp]
         L.oenv_run.argtypes = [vp, i32, i32, i32, i32, i32, u32, u64, i32, i32, i32, C.POINTER(EnvStats)]
+        L.oenv_encode.restype = i32; L.oenv_encode.argtypes = [vp, i32, i32, vp, vp]
         L.oa_new.restype = vp; L.oa_new.argtypes = [C.c_double, i32, i32, i32, vp, vp]
         L.oa_free.argtypes = [vp]; L.oa_clear.argtypes = [vp]
         L.oa_set_rhat_mode.argtypes = [vp, i32]
@@ -187,6 +188,19 @@ def env_run(G, H=11, W=11, S=4, health_dec=1, chance=0.15, seed=0, tics=100, enc
                    C.byref(st))
     return dict(steps=st.steps, planes=st.planes, episodes=st.episodes, plane_checksum=st.plane_checksum,
                 counters=list(st.counters))
+
+
+def env_encode(games, n_threads=1):
+    """make_state of every live snake of every game, in (game, snake id) order: (ids int32 [n] = game * 8 + snake id,
+    planes float32 [n, 2H-1, 2W-1, 3]).  games: OracleGame or None (a finished game: no rows); all of one shape."""
+    arr = (C.c_void_p * len(games))(*[g.h if g is not None else None for g in games])
+    shape = next(((2 * g.H - 1, 2 * g.W - 1, 3) for g in games if g is not None), (1, 1, 3))
+    n = lib().oenv_encode(arr, len(games), 1, None, None) if len(games) else 0
+    planes = np.empty((n,) + shape, dtype=np.float32)
+    ids = np.empty(n, dtype=np.int32)
+    if n:
+        lib().oenv_encode(arr, len(games), n_threads, _p(planes), _p(ids))
+    return ids, planes
 
 
 def env_handles(games):

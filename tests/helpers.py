@@ -32,6 +32,21 @@ def golden_dump(z, t):
     return dict(snake=z["snake"][t], owner=z["owner"][t], dist=z["dist"][t], food=z["food"][t], counters=z["counters"][t])
 
 
+SENTINEL = 0x7FBADBAD        # a NaN with a payload no encoder writes: fills plane buffers to mark the words nobody wrote
+
+
+def plane_features(planes):
+    """What a set of rows exercises: board window on each plane edge, other snakes' heads, food, food above 1.0."""
+    P = np.asarray(planes)
+    board = ~((P[..., 0] == 0) & (P[..., 1] == 1) & (P[..., 2] == 0))
+    c = P.shape[1] // 2
+    off = np.ones(P.shape[1:3], bool); off[c, c] = False
+    return dict(edges={e for e, v in (("top", board[:, 0, :]), ("bottom", board[:, -1, :]), ("left", board[:, :, 0]),
+                                      ("right", board[:, :, -1])) if v.any()},
+                heads=bool((P[:, off, 0] != 0).any()), food=bool((P[:, off, 2] != 0).any()),
+                food_above_1=bool((P[:, off, 2] > 1.0).any()))
+
+
 # ---- deterministic stand-in value functions (AlphaNNet.v contract, alpha_nnet.py:61-76) -------------------------------
 # Defined on the plane bytes; tests/golden/make_golden.py gives these to the reference's agents, the GPU tests give them
 # to the mirror's agents, so both sides see identical values for identical planes.

@@ -264,9 +264,10 @@ def test_food_chance_zero_never_spawns():
 @pytest.mark.parametrize("side,S,dec,G,tics", [(11, 4, 1, 4096, 120), (7, 4, 9, 1024, 80), (19, 8, 1, 512, 150),
                                                (11, 2, 3, 1000, 60), (7, 8, 1, 333, 60),
                                                (11, 4, 1, 65536, 24),       # BASELINE.json configs[1] at full size
-                                               # odd game counts just above two games per resident warp: scheduling tickets of two
-                                               # games, single games at the end of the launch and an odd last game, on every board size
-                                               (11, 4, 1, 9001, 30), (19, 8, 1, 3001, 20), (7, 4, 9, 8001, 24)])
+                                               # odd game counts above the single-game tail of a launch (3 games per resident warp):
+                                               # scheduling tickets of two games, single games at the end of the launch and an odd
+                                               # last game, on every board size
+                                               (11, 4, 1, 20001, 30), (19, 8, 1, 4001, 20), (7, 4, 9, 12001, 24)])
 def test_native_run_against_oracle(side, S, dec, G, tics):
     """Seeded native runs (engine RNG for layouts, actions and food; auto reset): every game's final state, the
     totals and an order-free checksum over every plane written must equal the oracle's, bit for bit."""
@@ -275,6 +276,10 @@ def test_native_run_against_oracle(side, S, dec, G, tics):
     seed = 1234 + side
     eng = _engine(side=side, snakes=S, health_dec=dec, games=G, seed=seed)
     eng.reset()
+    if G % 2 and G > 4000:     # the odd game counts: pair tickets first, then single games, the last of them alone in its ticket
+        from tests.test_gpu_env_planes import launch_layout
+        pairs, _ = launch_layout(side, G, torch.cuda.get_device_properties(eng.device).multi_processor_count)
+        assert pairs > 0 and 2 * pairs < G and (G - 2 * pairs) % 2 == 1, (G, pairs)
     csum = torch.zeros((), dtype=torch.int64, device="cuda")
     planes = 0
     # initial planes are not part of the oracle's env_run accounting (it encodes after every tic)

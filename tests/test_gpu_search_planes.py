@@ -11,10 +11,7 @@ import os
 import numpy as np
 import pytest
 
-from tests.helpers import assert_dump_equal, load
-
-SENTINEL = 0x7FBADBAD        # a NaN with a payload no encoder writes: marks the evaluation-batch words nobody wrote
-
+from tests.helpers import SENTINEL, assert_dump_equal, load, plane_features
 
 def eval_row_floats(eng):
     """Floats between consecutive rows of the evaluation batch (asz_search_eval_planes): dense planes."""
@@ -63,18 +60,6 @@ def compare_step(label, got, want, got_keys=None, want_keys=None, limit=4):
         if len(diff) > limit:
             fails.append("%s: %d rows differ in all" % (label, len(diff)))
     return fails
-
-
-def plane_features(planes):
-    """What a set of rows exercises: board window on each plane edge, other snakes' heads, food, food above 1.0."""
-    P = np.asarray(planes)
-    board = ~((P[..., 0] == 0) & (P[..., 1] == 1) & (P[..., 2] == 0))
-    c = P.shape[1] // 2
-    off = np.ones(P.shape[1:3], bool); off[c, c] = False
-    return dict(edges={e for e, v in (("top", board[:, 0, :]), ("bottom", board[:, -1, :]), ("left", board[:, :, 0]),
-                                      ("right", board[:, :, -1])) if v.any()},
-                heads=bool((P[:, off, 0] != 0).any()), food=bool((P[:, off, 2] != 0).any()),
-                food_above_1=bool((P[:, off, 2] > 1.0).any()))
 
 
 # ---- the device side: one root turn through the C ABI, the per-step loop of Engine.search -----------------------------------
