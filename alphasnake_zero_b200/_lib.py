@@ -36,6 +36,10 @@ class NetWeights(C.Structure):
                 ("dense1_b", C.c_void_p), ("dense2_w", C.c_void_p), ("dense2_b", C.c_void_p)]
 
 
+class NetWeightsFP8(C.Structure):
+    _fields_ = [("w", NetWeights), ("act_scale", C.c_float * 9)]
+
+
 class PitPlayer(C.Structure):
     _fields_ = [("net", C.c_void_p), ("stub_word", C.c_int32)]
 
@@ -96,6 +100,8 @@ SYMBOLS = [
     ("asz_net_forward", C.c_int, [_vp, _vp, _i32, _vp, _vp]),
     ("asz_net_forward_pitched", C.c_int, [_vp, _vp, _i32, _i32, _vp, _vp]),
     ("asz_net_debug_layer", C.c_int, [_vp, _vp, _i32, _i32, _vp, _vp]),
+    ("asz_net_create_fp8", C.c_int, [C.POINTER(_vp), C.POINTER(NetWeightsFP8), _i32]),
+    ("asz_net_update_weights_fp8", C.c_int, [_vp, C.POINTER(NetWeightsFP8), _vp]),
     ("asz_pit_begin", C.c_int, [_vp, C.POINTER(PitPlayer), C.POINTER(PitPlayer), _i32, _vp, _vp]),
     ("asz_pit_turn", C.c_int, [_vp, _i32, _vp, _vp, _vp, _vp]),
     ("asz_pit_finish", C.c_int, [_vp, _vp, _vp, _vp, _vp]),

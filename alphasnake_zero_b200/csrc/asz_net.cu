@@ -17,9 +17,17 @@
 //                the ReLU (alpha_nnet.py:22-47), zero the padding positions and store bf16 in the same layout; the
 //                last convolution instead applies the 1x1 head convolution + BN + ReLU (alpha_nnet.py:49-50).
 //   dense head   Flatten + Dense(128) + ReLU + Dense(3) + tanh (alpha_nnet.py:52-54): 8 images per CTA, fp32.
+//
+// fp8 networks (asz_net_create_fp8, opt-in; DESIGN.md 4.3): the same kernel with F8 = true.  Activations are e4m3,
+// act[8][pos][16] (16 channels per 16-byte chunk, the same byte geometry), each layer's stored with a power-of-two scale;
+// convolutions 1..8 contract e4m3 x e4m3 with tcgen05.mma kind::f8f6f4 (M256 N128 K32), the first keeps bf16 operands and
+// only stores e4m3.  The epilogue is y = acc * scale' + bias (+ residual * res_scale), ReLU, mask, e4m3(y / act_scale).
 #include <cuda_bf16.h>
+#include <cuda_fp16.h>
+#include <cuda_fp8.h>
 
 #include <algorithm>
+#include <cmath>
 #include <cstring>
 #include <vector>
 
@@ -118,6 +126,17 @@ __device__ __forceinline__ void umma_bf16_pair(uint32_t tmem_d, uint64_t adesc, 
       "}\n" ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate), "r"(z)
       : "memory");
 }
+// the same with e4m3 A and B (kind::f8f6f4): K = 32 per instruction, the same 32 bytes of each row as a bf16 K = 16 step
+__device__ __forceinline__ void umma_f8_pair(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
+  const uint32_t z = 0;
+  asm volatile(
+      "{\n"
+      ".reg .pred p;\n"
+      "setp.ne.b32 p, %4, 0;\n"
+      "tcgen05.mma.cta_group::2.kind::f8f6f4 [%0], %1, %2, %3, {%5, %5, %5, %5, %5, %5, %5, %5}, p;\n"
+      "}\n" ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate), "r"(z)
+      : "memory");
+}
 // arrives on the barrier at this shared-memory offset in both CTAs once every MMA issued so far has completed
 __device__ __forceinline__ void umma_commit_pair(uint64_t* bar) {
   const uint16_t mask = 3;
@@ -129,6 +148,8 @@ __device__ __forceinline__ void umma_commit_pair(uint64_t* bar) {
 // instruction descriptor kind::f16: D fp32 (bits 4-5 = 1), A and B bf16 (bits 7-9, 10-12 = 1), both K-major,
 // N >> 3 at bits 17-22, M >> 4 at bits 24-28
 constexpr uint32_t kIdescPair = (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(kC >> 3) << 17) | ((uint32_t)((2 * kTileM) >> 4) << 24);
+// kind::f8f6f4: the same with A and B e4m3 (format code 0 in bits 7-9 and 10-12)
+constexpr uint32_t kIdescPairF8 = (1u << 4) | ((uint32_t)(kC >> 3) << 17) | ((uint32_t)((2 * kTileM) >> 4) << 24);
 
 // ---- convolution kernel -----------------------------------------------------------------------------------------
 struct ConvParams {
@@ -146,6 +167,8 @@ struct ConvParams {
   int real;                    // real rows / cols per image (21)
   int P_tot;                   // rows of every activation array (guards included)
   int P_real;                  // positions that belong to images of this launch
+  float res_scale;             // F8: the residual's stored e4m3 values times this are its values
+  float out_inv_scale;         // F8: 1 / act_scale of this layer (the stored e4m3 values are y * out_inv_scale)
 };
 
 // ---- persistent convolution kernel over CTA pairs -----------------------------------------------------------------------
@@ -172,17 +195,19 @@ struct ConvParams {
 // tried, with bulk-copy fills running; the first version of this loop spent 196 SASS instructions per 8 MMAs rebuilding
 // descriptors and walking divergence waterfalls and reached 46 % of that.)  So: the whole warp runs the loop in uniform
 // control flow, one elected lane issues; loops have compile-time trip counts; a descriptor's low word is base + constant.
-template <int HALO>
+// IN8: e4m3 operands, 16 channels per 16-byte chunk, so the halo tile and a weight chunk (half a tap) take half the bytes
+template <int HALO, bool IN8 = false>
 struct UmmaSmem {
   static constexpr int kSuper = 256;                               // positions per CTA and weight pass
   static constexpr int rows = kSuper + 2 * HALO;
-  static constexpr size_t a_bytes = (size_t)kKC * rows * 16;       // one halo tile, managed as two channel halves
+  static constexpr int kc = IN8 ? kKC / 2 : kKC;                   // 16-byte channel chunks of a row
+  static constexpr size_t a_bytes = (size_t)kc * rows * 16;        // one halo tile, managed as two channel halves
   static constexpr int b_rows = kC / 2;                            // output channels whose weights this CTA holds
-  static constexpr size_t b_chunk = (size_t)8 * b_rows * 16;       // half a tap: 8 KB per CTA
+  static constexpr size_t b_chunk = (size_t)(kc / 2) * b_rows * 16;   // half a tap: 8 KB per CTA (IN8: 4 KB)
   static constexpr int max_stages = 18;                            // 18 = every weight chunk of a 3x3 layer (9 taps x 2 channel halves)
   static constexpr size_t tail = 3 * kC * sizeof(float) + (8 + 2 * max_stages) * sizeof(uint64_t) + 64;
   static constexpr int raw_stages = (int)((232448 - a_bytes - tail) / b_chunk);
-  static constexpr int b_stages = raw_stages > max_stages ? max_stages : raw_stages;   // 18 (HALO 24) / 17 (HALO 40)
+  static constexpr int b_stages = raw_stages > max_stages ? max_stages : raw_stages;   // 18 (HALO 24) / 17 (HALO 40); IN8: 18
   static constexpr size_t total = a_bytes + b_stages * b_chunk + tail;
 };
 
@@ -209,15 +234,19 @@ __device__ __forceinline__ uint64_t desc64(uint32_t lo, uint32_t hi) { return ((
 // (8 channels of tap 2j | 8 channels of tap 2j+1) of every row with the matching weight rows.  Five MMAs (the fifth pairs tap 8
 // with zero weights) instead of an im2col buffer: the layer reads 16 B per position where the im2col rows were 64 B, and the
 // separate im2col pass (write 64 B + read 64 B per position) is gone.  Weights: two chunks per tile, K steps 0..3 and K step 4.
-template <int HALO, bool FIRST>
+// F8 = a layer of an fp8 network: it stores (and adds as residual) e4m3 activations; unless FIRST it also reads e4m3 ones and
+// contracts them with e4m3 weights (IN8): a half is 4 chunks of 16 channels, one K = 32 MMA per 2 chunks, so the issue loop,
+// its descriptors and the weight ring are those of bf16 with 4 instead of 8 chunks per half.
+template <int HALO, bool FIRST, bool F8 = false>
 __global__ void __launch_bounds__(320, 1) conv_umma_kernel(const ConvParams p, int n_tiles) {
-  using SM = UmmaSmem<HALO>;
+  constexpr bool IN8 = F8 && !FIRST;
+  using SM = UmmaSmem<HALO, IN8>;
   constexpr int NS = SM::b_stages;
-  constexpr int KC_HALF = FIRST ? 1 : 8;                           // channel chunks of A per half
+  constexpr int KC_HALF = FIRST ? 1 : SM::kc / 2;                  // channel chunks of A per half
   constexpr int HALVES = FIRST ? 1 : 2;
   constexpr int TAPS = FIRST ? 2 : 9;                              // weight chunks per half (FIRST: K steps 0..3, K step 4)
   constexpr int TILE = 2 * SM::kSuper;                             // positions per work unit (pair super-tile)
-  constexpr uint32_t chunk_bytes = (uint32_t)(8 * SM::b_rows * 16);          // a full weight chunk: 8 K chunks
+  constexpr uint32_t chunk_bytes = (uint32_t)SM::b_chunk;          // a full weight chunk: 8 K chunks (IN8: 4)
   constexpr uint32_t last_chunk_bytes = FIRST ? (uint32_t)(2 * SM::b_rows * 16) : chunk_bytes;   // FIRST: K step 4 alone
   // RESW: the CTA's half of the layer's weights (9 taps x 2 halves x 8 KB = 144 KB) fits next to the halo tile (HALO 24: 7x7 and
   // 11x11 boards): it is loaded ONCE per launch and stays resident, instead of streaming through the stage ring once per super-tile
@@ -360,7 +389,8 @@ __global__ void __launch_bounds__(320, 1) conv_umma_kernel(const ConvParams p, i
                     const uint64_t ad = desc64(a_t + (uint32_t)(sub * kTileM + 2 * ks * SM::rows), desc_hi);
                     const uint64_t bd = desc64(b_s + (uint32_t)(2 * ks * SM::b_rows), desc_hi);
                     const uint32_t acc = (t == 0 && ks == 0) ? (uint32_t)c : 1u;
-                    umma_bf16_pair(tmem_d + (uint32_t)(sub * kC), ad, bd, kIdescPair, acc);
+                    if constexpr (IN8) umma_f8_pair(tmem_d + (uint32_t)(sub * kC), ad, bd, kIdescPairF8, acc);
+                    else umma_bf16_pair(tmem_d + (uint32_t)(sub * kC), ad, bd, kIdescPair, acc);
                   }
                 }
               }
@@ -410,10 +440,11 @@ __global__ void __launch_bounds__(320, 1) conv_umma_kernel(const ConvParams p, i
       const bool valid = pos < p.P_real && y < p.real && x < p.real;
       const size_t grow = (size_t)kGuard + (size_t)pos;
       // the residual row does not depend on the accumulator: fetch it while the MMAs of this super-tile run
-      uint4 rv[kKC];
+      constexpr int RKC = F8 ? kKC / 2 : kKC;                      // 16-byte chunks of a stored row
+      uint4 rv[RKC];
       if (p.res != nullptr) {
 #pragma unroll
-        for (int kc = 0; kc < kKC; ++kc) rv[kc] = *reinterpret_cast<const uint4*>(p.res + ((size_t)kc * p.P_tot + grow) * 8);
+        for (int kc = 0; kc < RKC; ++kc) rv[kc] = *reinterpret_cast<const uint4*>(p.res + ((size_t)kc * p.P_tot + grow) * 8);
       }
       mbar_wait(&acc_full[buf], (it >> 1) & 1u);
       tc_fence_after();
@@ -422,29 +453,63 @@ __global__ void __launch_bounds__(320, 1) conv_umma_kernel(const ConvParams p, i
       for (int cb = 0; cb < kC / 32; ++cb) {
         uint32_t v[32];
         tmem_ld32(tmem_base + (uint32_t)(buf * 256 + sub * kC + cb * 32) + ((uint32_t)(q * 32) << 16), v);
+        if constexpr (F8) {
 #pragma unroll
-        for (int j8 = 0; j8 < 4; ++j8) {
-          const int kc = cb * 4 + j8;
-          float f[8];
+          for (int j16 = 0; j16 < 2; ++j16) {
+            const int kc = cb * 2 + j16;                           // 16-channel chunk
+            float f[16];
 #pragma unroll
-          for (int j = 0; j < 8; ++j) f[j] = __uint_as_float(v[j8 * 8 + j]) * s_scale[kc * 8 + j] + s_bias[kc * 8 + j];
-          if (p.res != nullptr) {
-            const __nv_bfloat162* rb = reinterpret_cast<const __nv_bfloat162*>(&rv[kc]);
+            for (int j = 0; j < 16; ++j) f[j] = __uint_as_float(v[j16 * 16 + j]) * s_scale[kc * 16 + j] + s_bias[kc * 16 + j];
+            if (p.res != nullptr) {
+              const __nv_fp8x2_storage_t* rb = reinterpret_cast<const __nv_fp8x2_storage_t*>(&rv[kc]);
 #pragma unroll
-            for (int j = 0; j < 4; ++j) { const float2 t2 = __bfloat1622float2(rb[j]); f[2 * j] += t2.x; f[2 * j + 1] += t2.y; }
+              for (int j = 0; j < 8; ++j) {
+                const __half2_raw h = __nv_cvt_fp8x2_to_halfraw2(rb[j], __NV_E4M3);   // exact: e4m3 -> f16 -> f32
+                const float2 t2 = __half22float2(__half2(h));
+                f[2 * j] += t2.x * p.res_scale; f[2 * j + 1] += t2.y * p.res_scale;   // power-of-two scale: exact product
+              }
+            }
+#pragma unroll
+            for (int j = 0; j < 16; ++j) f[j] = valid ? fmaxf(f[j], 0.0f) : 0.0f;
+            if (p.out != nullptr) {
+              uint4 ov;
+              __nv_fp8x2_storage_t* ob = reinterpret_cast<__nv_fp8x2_storage_t*>(&ov);
+#pragma unroll
+              for (int j = 0; j < 8; ++j)       // cvt.rn.satfinite.e4m3x2.f32: nearest even, +-448 past the range
+                ob[j] = __nv_cvt_float2_to_fp8x2(make_float2(f[2 * j] * p.out_inv_scale, f[2 * j + 1] * p.out_inv_scale), __NV_SATFINITE,
+                                                 __NV_E4M3);
+              *reinterpret_cast<uint4*>(p.out + ((size_t)kc * p.P_tot + grow) * 8) = ov;
+            }
+            if (p.head_out != nullptr) {
+#pragma unroll
+              for (int j = 0; j < 16; ++j) head_acc = fmaf(__bfloat162float(__float2bfloat16_rn(f[j])), s_head[kc * 16 + j], head_acc);
+            }
           }
+        } else {
 #pragma unroll
-          for (int j = 0; j < 8; ++j) f[j] = valid ? fmaxf(f[j], 0.0f) : 0.0f;
-          if (p.out != nullptr) {
-            uint4 ov;
-            __nv_bfloat162* ob = reinterpret_cast<__nv_bfloat162*>(&ov);
+          for (int j8 = 0; j8 < 4; ++j8) {
+            const int kc = cb * 4 + j8;
+            float f[8];
 #pragma unroll
-            for (int j = 0; j < 4; ++j) ob[j] = __floats2bfloat162_rn(f[2 * j], f[2 * j + 1]);
-            *reinterpret_cast<uint4*>(p.out + ((size_t)kc * p.P_tot + grow) * 8) = ov;
-          }
-          if (p.head_out != nullptr) {
+            for (int j = 0; j < 8; ++j) f[j] = __uint_as_float(v[j8 * 8 + j]) * s_scale[kc * 8 + j] + s_bias[kc * 8 + j];
+            if (p.res != nullptr) {
+              const __nv_bfloat162* rb = reinterpret_cast<const __nv_bfloat162*>(&rv[kc]);
 #pragma unroll
-            for (int j = 0; j < 8; ++j) head_acc = fmaf(__bfloat162float(__float2bfloat16_rn(f[j])), s_head[kc * 8 + j], head_acc);
+              for (int j = 0; j < 4; ++j) { const float2 t2 = __bfloat1622float2(rb[j]); f[2 * j] += t2.x; f[2 * j + 1] += t2.y; }
+            }
+#pragma unroll
+            for (int j = 0; j < 8; ++j) f[j] = valid ? fmaxf(f[j], 0.0f) : 0.0f;
+            if (p.out != nullptr) {
+              uint4 ov;
+              __nv_bfloat162* ob = reinterpret_cast<__nv_bfloat162*>(&ov);
+#pragma unroll
+              for (int j = 0; j < 4; ++j) ob[j] = __floats2bfloat162_rn(f[2 * j], f[2 * j + 1]);
+              *reinterpret_cast<uint4*>(p.out + ((size_t)kc * p.P_tot + grow) * 8) = ov;
+            }
+            if (p.head_out != nullptr) {
+#pragma unroll
+              for (int j = 0; j < 8; ++j) head_acc = fmaf(__bfloat162float(__float2bfloat16_rn(f[j])), s_head[kc * 8 + j], head_acc);
+            }
           }
         }
       }
@@ -584,32 +649,36 @@ __global__ void dense1_raster_kernel(const float* __restrict__ w1, int real, int
 
 
 
-template <int HALO, bool FIRST>
+template <int HALO, bool FIRST, bool F8>
+constexpr size_t conv_smem_bytes() { return UmmaSmem<HALO, F8 && !FIRST>::total; }
+template <int HALO, bool FIRST, bool F8>
 static int configure_one() {
-  return cuda_ok(cudaFuncSetAttribute(conv_umma_kernel<HALO, FIRST>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                      (int)UmmaSmem<HALO>::total), "cudaFuncSetAttribute(conv_umma_kernel)") ? ASZ_OK : ASZ_ERR_CUDA;
+  return cuda_ok(cudaFuncSetAttribute(conv_umma_kernel<HALO, FIRST, F8>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                      (int)conv_smem_bytes<HALO, FIRST, F8>()), "cudaFuncSetAttribute(conv_umma_kernel)") ? ASZ_OK : ASZ_ERR_CUDA;
 }
+template <bool F8>
 static int configure_umma_kernels() {
   int rc = ASZ_OK;
-  if ((rc = configure_one<24, false>()) != ASZ_OK) return rc;
-  if ((rc = configure_one<24, true>()) != ASZ_OK) return rc;
-  if ((rc = configure_one<kHalo, false>()) != ASZ_OK) return rc;
-  if ((rc = configure_one<kHalo, true>()) != ASZ_OK) return rc;
+  if ((rc = configure_one<24, false, F8>()) != ASZ_OK) return rc;
+  if ((rc = configure_one<24, true, F8>()) != ASZ_OK) return rc;
+  if ((rc = configure_one<kHalo, false, F8>()) != ASZ_OK) return rc;
+  if ((rc = configure_one<kHalo, true, F8>()) != ASZ_OK) return rc;
   return rc;
 }
-template <int HALO, bool FIRST>
+template <int HALO, bool FIRST, bool F8>
 static int launch_one(int grid, const ConvParams& p, int n_tiles, cudaStream_t st) {
   cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3((unsigned)grid); cfg.blockDim = dim3(320); cfg.dynamicSmemBytes = UmmaSmem<HALO>::total; cfg.stream = st;
+  cfg.gridDim = dim3((unsigned)grid); cfg.blockDim = dim3(320); cfg.dynamicSmemBytes = conv_smem_bytes<HALO, FIRST, F8>(); cfg.stream = st;
   cudaLaunchAttribute at[1];
   at[0].id = cudaLaunchAttributeClusterDimension;
   at[0].val.clusterDim.x = 2; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
   cfg.attrs = at; cfg.numAttrs = 1;
-  return cuda_ok(cudaLaunchKernelEx(&cfg, conv_umma_kernel<HALO, FIRST>, p, n_tiles), "conv_umma_kernel") ? ASZ_OK : ASZ_ERR_CUDA;
+  return cuda_ok(cudaLaunchKernelEx(&cfg, conv_umma_kernel<HALO, FIRST, F8>, p, n_tiles), "conv_umma_kernel") ? ASZ_OK : ASZ_ERR_CUDA;
 }
+template <bool F8>
 static int launch_umma(bool big, bool first, int grid, const ConvParams& p, int n_tiles, cudaStream_t st) {
-  if (!big) return first ? launch_one<24, true>(grid, p, n_tiles, st) : launch_one<24, false>(grid, p, n_tiles, st);
-  return first ? launch_one<kHalo, true>(grid, p, n_tiles, st) : launch_one<kHalo, false>(grid, p, n_tiles, st);
+  if (!big) return first ? launch_one<24, true, F8>(grid, p, n_tiles, st) : launch_one<24, false, F8>(grid, p, n_tiles, st);
+  return first ? launch_one<kHalo, true, F8>(grid, p, n_tiles, st) : launch_one<kHalo, false, F8>(grid, p, n_tiles, st);
 }
 
 }  // namespace asz
@@ -629,6 +698,8 @@ struct asz_net {
   int device = 0;                 // the device this network lives on (asz_net_create's current device)
   __nv_bfloat16* w_pair[9] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
   __nv_bfloat16* w_first_pair = nullptr;   // first-layer weights, tap-paired and split for CTA pairs (first_weight_layout_kernel)
+  bool fp8 = false;               // asz_net_create_fp8: e4m3 activations and residual-layer weights
+  float act_scale[9] = {1, 1, 1, 1, 1, 1, 1, 1, 1};   // fp8: stored e4m3 value of layer i's output = output / act_scale[i]
 };
 
 static int net_forward_impl(asz_net* n, const float* d_planes, int32_t count, float* d_values, int stop_layer, float* d_act, cudaStream_t st,
@@ -648,8 +719,10 @@ static int net_derive(asz_net* n, cudaStream_t st) {
   first_weight_layout_kernel<<<(10 * kC + 255) / 256, 256, 0, st>>>(reinterpret_cast<const __nv_bfloat16*>(n->w.w_conv[0]), n->w_first_pair);
   if (!cuda_ok(cudaGetLastError(), "first_weight_layout_kernel")) return ASZ_ERR_CUDA;
   for (int l = 1; l < 9; ++l) {
-    const int total = 9 * kKC * kC;
-    pair_weight_layout_kernel<<<(total + 255) / 256, 256, 0, st>>>(reinterpret_cast<const __nv_bfloat16*>(n->w.w_conv[l]), n->w_pair[l], 9, kKC);
+    // fp8 [tap][8][128][16 B] read as [tap * 2 + half][4][128][16 B]: the pair layout [tap][half][rank][4][64][16 B] of the
+    // 4 KB weight chunks of conv_umma_kernel<.., F8>
+    const int taps = n->fp8 ? 18 : 9, kc_in = n->fp8 ? kKC / 4 : kKC, total = taps * kc_in * kC;
+    pair_weight_layout_kernel<<<(total + 255) / 256, 256, 0, st>>>(reinterpret_cast<const __nv_bfloat16*>(n->w.w_conv[l]), n->w_pair[l], taps, kc_in);
     if (!cuda_ok(cudaGetLastError(), "pair_weight_layout_kernel")) return ASZ_ERR_CUDA;
   }
   return ASZ_OK;
@@ -663,7 +736,7 @@ static int net_alloc(asz_net* n, const asz_net_weights* w, int32_t chunk_images)
   const size_t P = (size_t)chunk_images * n->img_stride;
   const size_t P_pad = (P + 511) / 512 * 512;                 // whole pair super-tiles
   n->P_tot = (int)(kGuard + P_pad + kGuard + kHalo);
-  const size_t act_bytes = (size_t)kKC * n->P_tot * 8 * sizeof(__nv_bfloat16);
+  const size_t act_bytes = (size_t)(n->fp8 ? kKC / 2 : kKC) * n->P_tot * 16;
   for (int i = 0; i < 3; ++i) {
     ASZ_CUDA(cudaMalloc(&n->act[i], act_bytes));
     ASZ_CUDA(cudaMemset(n->act[i], 0, act_bytes));
@@ -679,7 +752,7 @@ static int net_alloc(asz_net* n, const asz_net_weights* w, int32_t chunk_images)
     n->n_sm = prop.multiProcessorCount;
     n->device = dev;
   }
-  { int rc = configure_umma_kernels(); if (rc != ASZ_OK) return rc; }
+  { int rc = n->fp8 ? configure_umma_kernels<true>() : configure_umma_kernels<false>(); if (rc != ASZ_OK) return rc; }
   ASZ_CUDA(cudaFuncSetAttribute(dense_head_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024));
   ASZ_CUDA(cudaMalloc(&n->w1r, (size_t)n->img_stride * 128 * sizeof(float)));
   for (int l = 1; l < 9; ++l) ASZ_CUDA(cudaMalloc(&n->w_pair[l], (size_t)9 * kKC * kC * 16));
@@ -690,15 +763,36 @@ static int net_alloc(asz_net* n, const asz_net_weights* w, int32_t chunk_images)
 }
 
 
-int asz_net_create(asz_net** out, const asz_net_weights* w, int32_t chunk_images) {
+static int net_create(asz_net** out, const asz_net_weights* w, const float* act_scale, int32_t chunk_images) {
   if (!out || !w) { set_error("null argument"); return ASZ_ERR_ARG; }
   if (w->side != 7 && w->side != 11 && w->side != 19) { set_error("side must be 7, 11 or 19"); return ASZ_ERR_ARG; }
   if (chunk_images < 1) { set_error("chunk_images must be >= 1"); return ASZ_ERR_ARG; }
   asz_net* n = new asz_net();
+  if (act_scale) { n->fp8 = true; std::copy(act_scale, act_scale + 9, n->act_scale); }
   const int rc = net_alloc(n, w, chunk_images);
   if (rc != ASZ_OK) { asz_net_destroy(n); return rc; }
   *out = n;
   return ASZ_OK;
+}
+
+int asz_net_create(asz_net** out, const asz_net_weights* w, int32_t chunk_images) { return net_create(out, w, nullptr, chunk_images); }
+
+// an fp8 activation scale: a power of two whose reciprocal is a normal fp32 number too (so both products are exact)
+static bool act_scales_ok(const float* s) {
+  for (int i = 0; i < 9; ++i) {
+    int e = 0;
+    if (!(s[i] > 0.0f) || !std::isfinite(s[i]) || std::frexp(s[i], &e) != 0.5f || e < -124 || e > 127) {
+      set_error("act_scale must hold positive powers of two in [2^-125, 2^126]");
+      return false;
+    }
+  }
+  return true;
+}
+
+int asz_net_create_fp8(asz_net** out, const asz_net_weights_fp8* w, int32_t chunk_images) {
+  if (!out || !w) { set_error("null argument"); return ASZ_ERR_ARG; }
+  if (!act_scales_ok(w->act_scale)) return ASZ_ERR_ARG;
+  return net_create(out, &w->w, w->act_scale, chunk_images);
 }
 
 // New weights for an existing network (the per-generation weight push, alpha_snake_zero_trainer.py:52-57, 79-83): the
@@ -707,8 +801,20 @@ int asz_net_create(asz_net** out, const asz_net_weights* w, int32_t chunk_images
 int asz_net_update_weights(asz_net* n, const asz_net_weights* w, void* stream) {
   if (!n || !w) { set_error("null argument"); return ASZ_ERR_ARG; }
   if (w->side != n->side) { set_error("asz_net_update_weights: board side differs from the network's"); return ASZ_ERR_ARG; }
+  if (n->fp8) { set_error("asz_net_update_weights: an fp8 network takes asz_net_update_weights_fp8"); return ASZ_ERR_ARG; }
   DeviceGuard guard(n->device);
   n->w = *w;
+  return net_derive(n, (cudaStream_t)stream);
+}
+
+int asz_net_update_weights_fp8(asz_net* n, const asz_net_weights_fp8* w, void* stream) {
+  if (!n || !w) { set_error("null argument"); return ASZ_ERR_ARG; }
+  if (w->w.side != n->side) { set_error("asz_net_update_weights_fp8: board side differs from the network's"); return ASZ_ERR_ARG; }
+  if (!n->fp8) { set_error("asz_net_update_weights_fp8: a bf16 network takes asz_net_update_weights"); return ASZ_ERR_ARG; }
+  if (!act_scales_ok(w->act_scale)) return ASZ_ERR_ARG;
+  DeviceGuard guard(n->device);
+  n->w = w->w;
+  std::copy(w->act_scale, w->act_scale + 9, n->act_scale);
   return net_derive(n, (cudaStream_t)stream);
 }
 
@@ -736,7 +842,10 @@ static int launch_conv(asz_net* n, int layer, const __nv_bfloat16* in, const __n
   const bool big = n->pitch + 1 > 24;
   const int n_tiles = (p.P_real + 511) / 512;                   // pair super-tiles
   const int grid = 2 * std::min(n_tiles, n->n_sm / 2);
-  return launch_umma(big, layer == 0, grid, p, n_tiles, st);
+  if (!n->fp8) return launch_umma<false>(big, layer == 0, grid, p, n_tiles, st);
+  p.res_scale = res ? n->act_scale[layer - 2] : 1.0f;            // the residual of layer 2b+2 is the output of layer 2b
+  p.out_inv_scale = 1.0f / n->act_scale[layer];
+  return launch_umma<true>(big, layer == 0, grid, p, n_tiles, st);
 }
 
 int asz_net_forward(asz_net* n, const float* d_planes, int32_t count, float* d_values, void* stream) {
@@ -765,9 +874,10 @@ int asz_net_debug_layer(asz_net* n, const float* d_planes, int32_t count, int32_
 }  // extern "C"
 
 namespace asz {
-// activation buffer -> fp32 [n][real][real][128] (debug / tests)
+// activation buffer -> fp32 [n][real][real][128] (debug / tests); F8: e4m3 act[8][pos][16] times `scale` (exact)
+template <bool F8 = false>
 __global__ void export_act_kernel(const __nv_bfloat16* act, const float* head, int n_img, int real, int pitch, int img_stride, int P_tot,
-                                  float* out) {
+                                  float* out, float scale = 1.0f) {
   const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
   const size_t per = (size_t)real * real * (head ? 1 : kC);
   if (i >= (size_t)n_img * per) return;
@@ -777,7 +887,12 @@ __global__ void export_act_kernel(const __nv_bfloat16* act, const float* head, i
   if (!head) { c = (int)(r % kC); r /= kC; }
   const int y = (int)(r / real), x = (int)(r % real);
   const size_t grow = (size_t)kGuard + (size_t)n * img_stride + (size_t)y * pitch + x;
-  out[i] = head ? head[grow] : __bfloat162float(act[((size_t)(c >> 3) * P_tot + grow) * 8 + (c & 7)]);
+  if constexpr (F8) {
+    const __nv_fp8_storage_t* a8 = reinterpret_cast<const __nv_fp8_storage_t*>(act);
+    out[i] = head ? head[grow] : __half2float(__half(__nv_cvt_fp8_to_halfraw(a8[((size_t)(c >> 4) * P_tot + grow) * 16 + (c & 15)], __NV_E4M3))) * scale;
+  } else {
+    out[i] = head ? head[grow] : __bfloat162float(act[((size_t)(c >> 3) * P_tot + grow) * 8 + (c & 7)]);
+  }
 }
 }  // namespace asz
 
@@ -786,7 +901,11 @@ static int net_forward_impl(asz_net* n, const float* d_planes, int32_t count, fl
   const size_t plane = plane_stride ? plane_stride : (size_t)n->real * n->real * 3;     // floats between consecutive input planes
   auto dump = [&](const __nv_bfloat16* act, const float* head, int m) -> int {
     const size_t tot = (size_t)m * n->real * n->real * (head ? 1 : kC);
-    export_act_kernel<<<(unsigned)((tot + 255) / 256), 256, 0, st>>>(act, head, m, n->real, n->pitch, n->img_stride, n->P_tot, d_act);
+    if (n->fp8)
+      export_act_kernel<true><<<(unsigned)((tot + 255) / 256), 256, 0, st>>>(act, head, m, n->real, n->pitch, n->img_stride, n->P_tot, d_act,
+                                                                              n->act_scale[stop_layer]);
+    else
+      export_act_kernel<<<(unsigned)((tot + 255) / 256), 256, 0, st>>>(act, head, m, n->real, n->pitch, n->img_stride, n->P_tot, d_act);
     return cuda_ok(cudaGetLastError(), "export_act_kernel") ? ASZ_OK : ASZ_ERR_CUDA;
   };
   // balanced passes: ceil(count / chunk) passes of (almost) equal size, so that no pass is a sliver that leaves SMs idle

@@ -5,6 +5,8 @@ through the hand-written sm_100a kernels of libasz_b200.so (backend "native", th
 tcgen05 tensor cores, bf16 operands, fp32 accumulation; it raises when the library or a GPU is missing) or, only when asked
 for by name, through plain PyTorch ops (backend "torch": the library baseline and fp32 reference of the numerics tests).  Weights are kept in the Keras layouts the reference's .h5 files use
 (conv kernels HWIO, dense (in, out), BN gamma/beta/moving_mean/moving_variance).
+dtype="fp8" selects the native fp8 (e4m3) tower instead (net.py; opt-in: its values are outside the bf16 network's 2e-2
+accuracy, DESIGN.md 4.3); it has no PyTorch path.
 """
 import numpy as np
 import torch
@@ -74,10 +76,15 @@ class _VNet:
 class AlphaNNet:
 
     def __init__(self, model_name=None, input_shape=None, device=None, backend="auto", dtype="bf16", seed=None,
-                 weights=None):
+                 weights=None, calibration=None):
+        """calibration: device planes [n, N, N, 3] on which dtype="fp8" calibrates its activation scales (default: the
+        seeded set of net.calibration_planes)"""
+        if dtype == "fp8" and backend == "torch":
+            raise ValueError("dtype='fp8' runs on the native backend only: there is no PyTorch fp8 path")
         self.device = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
         self.backend = backend
         self.dtype = dtype
+        self.calibration = calibration
         self.weights = None
         self._torch = None
         self._native = None
@@ -142,12 +149,14 @@ class AlphaNNet:
     def _get_native(self):
         if self._native is None:
             from ..net import NativeNet          # raises if libasz_b200.so is missing: no fallback
-            self._native = NativeNet(self.weights, self.device)
+            self._native = NativeNet(self.weights, self.device, dtype="fp8" if self.dtype == "fp8" else "bf16",
+                                     calibration=self.calibration)
         return self._native
 
     def set_weights(self, weights):
         """replace the weight dictionary and refresh every device copy `v` uses (the native network's operands through
-        asz_net_update_weights, the PyTorch parameters by rebuilding them): the per-generation weight push"""
+        asz_net_update_weights, re-quantized and re-calibrated for fp8; the PyTorch parameters by rebuilding them): the
+        per-generation weight push"""
         self.weights = weights
         self._torch = None
         if self._native is not None:
@@ -181,7 +190,8 @@ class AlphaNNet:
     def copy_and_compile(self, learning_rate=0.0001, TPU=None):
         """alpha_nnet.py:78-106: a copy with a fresh optimizer state (piecewise-constant LR x0.25 every 20 steps)."""
         import copy
-        c = AlphaNNet(device=self.device, backend=self.backend, dtype=self.dtype, weights=copy.deepcopy(self.weights))
+        c = AlphaNNet(device=self.device, backend=self.backend, dtype=self.dtype, weights=copy.deepcopy(self.weights),
+                      calibration=self.calibration)
         c.lr = learning_rate
         return c
 

@@ -26,9 +26,11 @@ def main():
     ap.add_argument("--depth", type=int, default=8)
     ap.add_argument("--pit-games", type=int, default=100)
     ap.add_argument("--name", default="Example")
+    ap.add_argument("--dtype", default="bf16", choices=["bf16", "fp8"],
+                    help="value network of the native backend: bf16 (reference) or the opt-in fp8 tower")
     a = ap.parse_args()
     iteration, health_dec, lr = 0, 9, 1e-4                                 # train.py:6-13, trainer :42-47
-    nnet = AlphaNNet(input_shape=(21, 21, 3)).copy_and_compile()
+    nnet = AlphaNNet(input_shape=(21, 21, 3), dtype=a.dtype).copy_and_compile()
     t0 = time()
     Alice = Agent(nnet, 2 + iteration, True, a.depth, a.breadth)           # :52
     gr = MPGameRunner(11, 11, 4, health_dec, a.games, verbose=False)       # :53

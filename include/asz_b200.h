@@ -285,6 +285,23 @@ int asz_net_forward_pitched(asz_net* net, const float* d_planes, int32_t plane_p
  * that layer's output as float32 [count][2*side-1][2*side-1][128] ([..][1] for layer 8: the fused 1x1 head conv) */
 int asz_net_debug_layer(asz_net* net, const float* d_planes, int32_t count, int32_t layer, float* d_act, void* stream);
 
+/* fp8 networks (opt-in; outside the bf16 network's accuracy, DESIGN.md 4.3): activations stored as e4m3, residual
+ * convolutions 1..8 with e4m3 operands and fp32 accumulation; the first convolution, the head and the dense layers as above.
+ * Fields of w that differ from asz_net_weights':
+ *   w_conv[1..8]  e4m3 [9][8][128][16]  [tap][cin / 16][cout][cin % 16], the weights divided by a per-output-channel scale
+ *   scale[i]      fp32 [128]            folded BatchNorm scale times that weight scale times act_scale[i-1] (i >= 1)
+ *   act_scale[i]  the power of two by which layer i's outputs are divided before they are stored as e4m3 (saturating at
+ *                 +-448); ASZ_ERR_ARG unless every entry is one in [2^-125, 2^126] (act_scale[8] is not used: layer 8
+ *                 is the fused head)
+ * Every other entry point taking an asz_net* works on an fp8 network unchanged (asz_net_debug_layer exports the stored values
+ * times act_scale: exact in fp32).  asz_net_update_weights refuses an fp8 network and asz_net_update_weights_fp8 a bf16 one. */
+typedef struct {
+  asz_net_weights w;
+  float act_scale[9];
+} asz_net_weights_fp8;
+int asz_net_create_fp8(asz_net** out, const asz_net_weights_fp8* w, int32_t chunk_images);
+int asz_net_update_weights_fp8(asz_net* net, const asz_net_weights_fp8* w, void* stream);
+
 /* ---- pit: pit_mp_game_runner.MPGameRunner.run(Alice, Bob, Alice_snake_cnt) (pit_mp_game_runner.py:14-63) with
  * pit_agent.Agent (pit_agent.py:10-28) on both sides, played on the engine's root games without planes through the host (either
  * side may play the search Agent instead: asz_pit_set_search below) --------------------------------------------------------

@@ -1,4 +1,6 @@
-"""Value-network throughput: hand-written tcgen05 path vs PyTorch (cuDNN) bf16/fp32.  python tools/bench_net.py [n]"""
+"""Value-network throughput: hand-written tcgen05 path vs PyTorch (cuDNN) bf16/fp32.
+python tools/bench_net.py [n [side [chunk]]] [--dtype bf16|fp8|both] [--chunks] [--no-torch]   (or --dtype=...)
+--dtype both times the bf16 and the fp8 native networks in alternating rounds and adds their ratio."""
 import json
 import os
 import sys
@@ -14,7 +16,17 @@ FLOPS = {7: None, 11: 1043724288, 19: 3240040448}
 
 
 def main():
-    argv = [a for a in sys.argv[1:] if not a.startswith("--")]
+    args = sys.argv[1:]
+    dt = "bf16"
+    for i, a in enumerate(args):                # --dtype=X or --dtype X
+        if a.startswith("--dtype="):
+            dt = a.split("=", 1)[1]
+        elif a == "--dtype" and i + 1 < len(args):
+            dt = args[i + 1]
+            args[i + 1] = "--"
+    if dt not in ("bf16", "fp8", "both"):
+        sys.exit("--dtype must be bf16, fp8 or both")
+    argv = [a for a in args if not a.startswith("--")]
     n = int(argv[0]) if len(argv) > 0 else 16384
     side = int(argv[1]) if len(argv) > 1 else 11
     chunk = int(argv[2]) if len(argv) > 2 else 4096
@@ -35,12 +47,20 @@ def main():
         e1.record()
         torch.cuda.synchronize()
         return e0.elapsed_time(e1) / reps * 1e-3
+    dtypes = ["bf16", "fp8"] if dt == "both" else [dt]
     for ch in sorted({chunk, 4 * chunk} if "--chunks" in sys.argv else {chunk}):
-        nat = NativeNet(w, "cuda", chunk_images=ch)
-        t = timeit(lambda: nat.forward(x))
-        out["native_bf16_chunk%d" % ch] = {"evals_per_s": n / t, "tflops": n / t * FLOPS[side] / 1e12 if FLOPS[side] else None,
-                                           "ms": t * 1e3}
-        del nat
+        nats = {d: NativeNet(w, "cuda", chunk_images=ch, dtype=d) for d in dtypes}
+        times = {d: [] for d in dtypes}
+        for _ in range(3):                      # alternating rounds: both dtypes see the same clocks and neighbours
+            for d in dtypes:
+                times[d].append(timeit(lambda: nats[d].forward(x)))
+        for d in dtypes:
+            t = min(times[d])
+            out["native_%s_chunk%d" % (d, ch)] = {"evals_per_s": n / t, "tflops": n / t * FLOPS[side] / 1e12 if FLOPS[side] else None,
+                                                 "ms": t * 1e3, "ms_rounds": [r * 1e3 for r in times[d]]}
+        if len(dtypes) == 2:
+            out["fp8_over_bf16_chunk%d" % ch] = min(times["bf16"]) / min(times["fp8"])
+        del nats
     if "--no-torch" in sys.argv:
         print(json.dumps({"n": n, "side": side, "chunk": chunk, **out}))
         return

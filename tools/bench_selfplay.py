@@ -1,7 +1,7 @@
 """Self-play throughput of one BASELINE.json configuration on this process's GPU (one process per GPU under torchrun;
 games shard by game id with no collective on the hot path, SURVEY.md 8(e)).
 
-  python tools/bench_selfplay.py --config 3|4|5 [--world 8] [--turns 2]
+  python tools/bench_selfplay.py --config 3|4|5 [--world 8] [--turns 2] [--dtype bf16|fp8]
   python -m torch.distributed.run --nproc-per-node N --master-addr 127.0.0.1 tools/bench_selfplay.py --config 4
 
 --world: number of GPUs the configuration is sharded over; the per-GPU share of the games is what runs here
@@ -29,6 +29,8 @@ def main():
     ap.add_argument("--turns", type=int, default=2)
     ap.add_argument("--stub", action="store_true", help="stub value function (search kernels only)")
     ap.add_argument("--prewarm-tics", type=int, default=32, help="uniform-random tics (with reset) before the search starts")
+    ap.add_argument("--dtype", default="bf16", choices=["bf16", "fp8"],
+                    help="value network: bf16 (reference) or the opt-in fp8 tower (built and calibrated before the timed turns)")
     args = ap.parse_args()
     import torch
     rank = int(os.environ.get("RANK", "0")); nproc = int(os.environ.get("WORLD_SIZE", "1"))
@@ -40,8 +42,23 @@ def main():
         import torch.distributed as dist
         dist.init_process_group("nccl", device_id=torch.device("cuda", torch.cuda.current_device()))
         dist.barrier()
-    r = bench.selfplay_leg(rank, games, c["breadth"], 8, args.turns, 1, use_net=not args.stub, side=c["side"], snakes=c["snakes"],
-                           label="%s, 1/%d of the games per GPU" % (c["label"], world), prewarm_tics=args.prewarm_tics)
+    from alphasnake_zero_b200.utils import alpha_nnet
+    bf16_net = alpha_nnet.AlphaNNet
+    if args.dtype != "bf16":
+        # bench.selfplay_leg builds its AlphaNNet by name from this module: hand it one of the requested dtype for this call
+        class Net(bf16_net):
+            def __init__(self, *a, **k):
+                super().__init__(*a, dtype=args.dtype, **k)
+        alpha_nnet.AlphaNNet = Net
+    try:
+        r = bench.selfplay_leg(rank, games, c["breadth"], 8, args.turns, 1, use_net=not args.stub, side=c["side"], snakes=c["snakes"],
+                               label="%s, 1/%d of the games per GPU" % (c["label"], world), prewarm_tics=args.prewarm_tics)
+    finally:
+        alpha_nnet.AlphaNNet = bf16_net
+    if args.dtype != "bf16" and not args.stub:
+        r["workload"] = r["workload"].replace("bf16 tcgen05 value net", "%s tcgen05 value net" % args.dtype)
+        r.pop("net_roofline", None)                       # its peak is the bf16 one
+    r["dtype"] = "stub" if args.stub else args.dtype
     r["ranks_run"] = nproc
     if nproc > 1:
         rates = ("sims_per_sec", "node_visits_per_sec", "nn_evals_per_sec", "subgame_tics_per_sec")

@@ -45,9 +45,18 @@ __device__ __forceinline__ void tmem_dealloc(uint32_t taddr, uint32_t cols) {
   if (CG == 1) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(cols) : "memory");
   else asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(cols) : "memory");
 }
-template <int CG>
+// F8: kind::f8f6f4 with e4m3 A and B, K = 32 per MMA (the same 32 bytes of a row as a bf16 K = 16 step)
+template <int CG, bool F8>
 __device__ __forceinline__ void umma(uint32_t d, uint64_t a, uint64_t b, uint32_t idesc, uint32_t acc) {
-  if (CG == 1) {
+  if (F8 && CG == 1) {
+    asm volatile("{\n.reg .pred p;\nsetp.ne.b32 p, %4, 0;\ntcgen05.mma.cta_group::1.kind::f8f6f4 [%0], %1, %2, %3, p;\n}\n" ::"r"(d),
+                 "l"(a), "l"(b), "r"(idesc), "r"(acc)
+                 : "memory");
+  } else if (F8) {
+    asm volatile("{\n.reg .pred p;\nsetp.ne.b32 p, %4, 0;\ntcgen05.mma.cta_group::2.kind::f8f6f4 [%0], %1, %2, %3, p;\n}\n" ::"r"(d),
+                 "l"(a), "l"(b), "r"(idesc), "r"(acc)
+                 : "memory");
+  } else if (CG == 1) {
     asm volatile("{\n.reg .pred p;\nsetp.ne.b32 p, %4, 0;\ntcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n}\n" ::"r"(d), "l"(a),
                  "l"(b), "r"(idesc), "r"(acc)
                  : "memory");
@@ -76,7 +85,8 @@ __device__ __forceinline__ uint64_t desc(uint32_t saddr, uint32_t lbo, uint32_t 
 // MODE 1: 128-byte swizzle, K-major (rows of 128 B = 64 bf16, SBO 1024)
 // MODE 2: like 0 but the descriptors are rebuilt from integers for every MMA (the product kernel's issue loop)
 // FILL > 0: a second thread keeps FILL bytes per MMA of bulk copies (global -> shared) in flight, as the producer does
-template <int CG, int N, int MODE, int FILL>
+// F8: the same chain with kind::f8f6f4 (e4m3, K = 32: twice the MACs per MMA of a bf16 K = 16 step)
+template <int CG, int N, int MODE, int FILL, bool F8 = false>
 __global__ void __launch_bounds__(128, 1) probe_kernel(int iters, const unsigned char* gsrc, long long* out) {
   extern __shared__ __align__(1024) unsigned char smem[];
   unsigned char* sA = smem;                 // 80 KB
@@ -100,7 +110,7 @@ __global__ void __launch_bounds__(128, 1) probe_kernel(int iters, const unsigned
   const uint32_t tmem = s_tmem;
   const uint32_t rank = CG == 2 ? cluster_ctarank() : 0;
   constexpr int M = CG == 2 ? 256 : 128;
-  constexpr uint32_t idesc = (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(N >> 3) << 17) | ((uint32_t)(M >> 4) << 24);
+  constexpr uint32_t idesc = (1u << 4) | (F8 ? 0u : (1u << 7) | (1u << 10)) | ((uint32_t)(N >> 3) << 17) | ((uint32_t)(M >> 4) << 24);
   constexpr int NB = CG == 2 ? N / 2 : N;    // rows of B in this CTA
   if (warp == 1 && lane == 0 && rank == 0) {
     const uint32_t a_base = smem_u32(sA), b_base = smem_u32(sB);
@@ -125,7 +135,7 @@ __global__ void __launch_bounds__(128, 1) probe_kernel(int iters, const unsigned
           ad = desc(a_addr, 304 * 16, 128, 0);
           bd = desc(b_addr, NB * 16, 128, 0);
         }
-        umma<CG>(tmem + (uint32_t)((i & 1) * N), ad, bd, idesc, acc);
+        umma<CG, F8>(tmem + (uint32_t)((i & 1) * N), ad, bd, idesc, acc);
         acc = 1;
       }
     }
@@ -152,11 +162,11 @@ __global__ void __launch_bounds__(128, 1) probe_kernel(int iters, const unsigned
   if (warp == 0) { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); tmem_dealloc<CG>(tmem, 512); }
 }
 
-template <int CG, int N, int MODE, int FILL>
+template <int CG, int N, int MODE, int FILL, bool F8 = false>
 static void run(const char* name, int grid, const unsigned char* gsrc, long long* d_out) {
   const int iters = 512;
   const size_t smem = 208 * 1024;
-  cudaFuncSetAttribute(probe_kernel<CG, N, MODE, FILL>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  cudaFuncSetAttribute(probe_kernel<CG, N, MODE, FILL, F8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   cudaMemset(d_out, 0, 148 * sizeof(long long));
   cudaLaunchConfig_t cfg = {};
   cfg.gridDim = dim3(grid); cfg.blockDim = dim3(128); cfg.dynamicSmemBytes = smem;
@@ -164,7 +174,7 @@ static void run(const char* name, int grid, const unsigned char* gsrc, long long
   at[0].id = cudaLaunchAttributeClusterDimension; at[0].val.clusterDim.x = CG; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
   cfg.attrs = at; cfg.numAttrs = 1;
   for (int rep = 0; rep < 2; ++rep) {
-    cudaError_t e = cudaLaunchKernelEx(&cfg, probe_kernel<CG, N, MODE, FILL>, iters, gsrc, d_out);
+    cudaError_t e = cudaLaunchKernelEx(&cfg, probe_kernel<CG, N, MODE, FILL, F8>, iters, gsrc, d_out);
     if (e != cudaSuccess) { printf("%s: launch error %s\n", name, cudaGetErrorString(e)); return; }
     e = cudaDeviceSynchronize();
     if (e != cudaSuccess) { printf("%s: error %s\n", name, cudaGetErrorString(e)); exit(1); }
@@ -174,9 +184,10 @@ static void run(const char* name, int grid, const unsigned char* gsrc, long long
   double sum = 0; int cnt = 0; long long mx = 0;
   for (int i = 0; i < grid; ++i) if (h[i] > 0) { sum += h[i]; ++cnt; if (h[i] > mx) mx = h[i]; }
   const double per = sum / cnt / (iters * 8.0);
-  const double macs = (CG == 2 ? 128.0 : 128.0) * N * 16;     // per SM
-  printf("%-44s grid %3d: %7.1f clk/MMA (max %7.1f)  %6.0f MAC/clk/SM  (%.0f%% of 4096)\n", name, grid, per, mx / (iters * 8.0), macs / per,
-         100.0 * macs / per / 4096.0);
+  const double macs = (CG == 2 ? 128.0 : 128.0) * N * (F8 ? 32 : 16);     // per SM
+  const double peak = F8 ? 8192.0 : 4096.0;                                 // dense MAC/clk/SM: e4m3 twice bf16
+  printf("%-44s grid %3d: %7.1f clk/MMA (max %7.1f)  %6.0f MAC/clk/SM  (%.0f%% of %.0f)\n", name, grid, per, mx / (iters * 8.0), macs / per,
+         100.0 * macs / per / peak, peak);
 }
 
 int main() {
@@ -197,6 +208,10 @@ int main() {
   run<1, 128, 0, 2048>("cg1 N128 noswz + 2 KB fill per MMA", 148, gsrc, d_out);
   run<1, 128, 1, 2048>("cg1 N128 sw128 + 2 KB fill per MMA", 148, gsrc, d_out);
   run<2, 128, 0, 1024>("cg2 M256 N128 noswz + 1 KB fill per MMA", 148, gsrc, d_out);
+  run<1, 128, 0, 0, true>("f8 K32 cg1 N128 noswz", 148, gsrc, d_out);
+  run<2, 128, 0, 0, true>("f8 K32 cg2 M256 N128 noswz", 148, gsrc, d_out);
+  run<2, 128, 2, 0, true>("f8 K32 cg2 M256 N128 noswz desc-in-loop", 148, gsrc, d_out);
+  run<2, 128, 0, 1024, true>("f8 K32 cg2 M256 N128 noswz + 1 KB fill/MMA", 148, gsrc, d_out);
   run<1, 128, 0, 0>("cg1 N128 noswz, 1 CTA", 1, gsrc, d_out);
   return 0;
 }
